@@ -9,6 +9,7 @@ plays its own 4,096 games (disjoint seeds), no data-path collective (SURVEY 8e).
   python bench.py --gpus 1 --steps 20 --warmup 3
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
   python bench.py --impl reference ...     # CPU arm: the oracle port on all host threads
+  python bench.py ... --dump-outputs DIR   # also write the last timed step's results as DIR/<name>.npy (float32)
 
 JSON keys follow the driver contract; `roofline` and `cpu_baseline` are described in DESIGN.md.
 """
@@ -22,6 +23,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path[:0] = [ROOT]
+sys.dont_write_bytecode = True  # the bench leaves the source tree as it found it (it may be read-only)
 
 B_STEP = 2 * 512 + 1 + 20 + 2  # algorithmic bytes per env step (SURVEY 8d): state in+out, action, mask, reward/done
 METRIC = "env_steps_per_sec"
@@ -146,6 +148,29 @@ def issue_roofline(key, env_steps_per_launch, seconds_per_launch, sm_count, sm_m
     return out
 
 
+DUMP_LIMIT = 64_000_000  # bytes of the files written by --dump-outputs in all, .npy headers included
+NPY_HEADER_MAX = 1024  # allowance per file for its .npy header (numpy writes 128 bytes for these shapes)
+
+
+def dump_outputs(out_dir, arrays, seed=0):
+    """Writes each array as out_dir/<name>.npy in float32 (exact for the u8 records and int32 step counts).  When the files
+    would exceed DUMP_LIMIT, the same seeded sample of rows is taken from every array and its indices are written as
+    rows.npy, so that two builds run with the same arguments write the same rows."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    host = {k: v.detach().cpu().numpy().astype(np.float32) for k, v in arrays.items()}
+    n = len(next(iter(host.values())))
+    row_bytes = sum(a[:1].nbytes for a in host.values())
+    if n * row_bytes + len(host) * NPY_HEADER_MAX > DUMP_LIMIT:  # sample rows; one more file, rows.npy (8 bytes a row)
+        keep = (DUMP_LIMIT - (len(host) + 1) * NPY_HEADER_MAX) // (row_bytes + 8)
+        rows = np.sort(np.random.default_rng(seed).choice(n, keep, replace=False))
+        host = {k: a[rows] for k, a in host.items()}
+        host["rows"] = rows.astype(np.float64)
+    for k, a in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    return sorted(host)
+
+
 def cpu_port(n_games, threads, seed0=10_000_000):
     """The oracle port (plain C restatement of the reference engine) on `threads` host threads."""
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
@@ -185,42 +210,41 @@ def run_reference(args):
         return
     threads = os.cpu_count() or 1
     n_games = 4096 * max(args.gpus, 1)  # the job's games per step: 4,096 per GPU, like the GPU arm at this N
-    # the port: every step plays all n_games
-    for _ in range(min(args.warmup, 1)):
+    # the port: every step plays all n_games; exactly args.warmup untimed steps, then exactly args.steps timed ones
+    for _ in range(args.warmup):
         cpu_port(n_games, threads)
     tot_steps, tot_t = 0, 0.0
-    for k in range(min(args.steps, 3)):
+    for k in range(args.steps):
         s, dt = cpu_port(n_games, threads, seed0=20_000_000 + k * n_games)
         tot_steps += s
         tot_t += dt
-    port = {"value": tot_steps / tot_t, "unit": "env_steps/s", "cores": threads, "kind": "port",
-            "sample": "%d games (default decks, random agents, to completion) per step, %d steps; dealing excluded from the clock" % (n_games, min(args.steps, 3))}
-    # the reference itself: a bounded sample of the same games per step (whole games; ~500 env steps/s per core)
+    port = {"value": tot_steps / tot_t, "unit": "env_steps/s", "cores": threads, "kind": "port", "timed_steps": args.steps,
+            "env_steps": int(tot_steps), "seconds": tot_t,
+            "sample": "%d games (default decks, random agents, to completion) per step, %d steps; dealing excluded from the clock" % (n_games, args.steps)}
+    # the reference itself: a bounded sample of the same games per step (whole games; ~500 env steps/s per core), exactly
+    # args.warmup untimed and args.steps timed steps like the port
     py, py_steps, py_t, sample_games = None, 0, 0.0, max(64, 2 * threads)
     try:
         sys.path.insert(0, os.path.join(ROOT, "oracle"))
         import ref_python_baseline
         if ref_python_baseline.reference_dir() is not None:
-            budget = time.perf_counter() + 150.0  # keep the whole arm within a few minutes whatever K is
             for k in range(args.warmup + args.steps):
                 r = ref_python_baseline.run(sample_games, seed0=30_000_000 + k * 100_000)
                 if k >= args.warmup:
                     py_steps += r["steps"]
                     py_t += r["seconds"]
-                if time.perf_counter() > budget and py_t > 0:
-                    break
-            if py_t > 0:
-                py = {"value": py_steps / py_t, "unit": "env_steps/s", "cores": threads, "kind": "reference",
-                      "sample": "%d of the job's %d games per step (default decks, random agents, to completion, %d env steps in %.1f s in all): the "
-                                "reference's unmodified Python engine (games/stormbound.py) under multiprocessing.Pool(%d)"
-                                % (sample_games, n_games, py_steps, py_t, threads)}
+            py = {"value": py_steps / py_t, "unit": "env_steps/s", "cores": threads, "kind": "reference", "timed_steps": args.steps,
+                  "env_steps": int(py_steps), "seconds": py_t,
+                  "sample": "%d of the job's %d games per step (default decks, random agents, to completion, %d env steps in %.1f s in all): the "
+                            "reference's unmodified Python engine (games/stormbound.py) under multiprocessing.Pool(%d)"
+                            % (sample_games, n_games, py_steps, py_t, threads)}
     except Exception as e:  # noqa: BLE001 -- fall back to the port rather than lose the arm
         py = None
         port["reference_unavailable"] = "%s: %s" % (type(e).__name__, e)
     arm = py or port
     line = {
-        "impl": "reference", "metric": METRIC, "value": arm["value"], "unit": "env_steps/s", "n_gpus": args.gpus, "steps": args.steps,
-        "warmup": args.warmup, "ms_per_step": (1e3 * py_t / max(args.steps, 1)) if py else (1e3 * tot_t / max(min(args.steps, 3), 1)),
+        "impl": "reference", "metric": METRIC, "value": arm["value"], "unit": "env_steps/s", "n_gpus": args.gpus, "steps": arm["timed_steps"],
+        "warmup": args.warmup, "ms_per_step": 1e3 * arm["seconds"] / arm["timed_steps"],
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "u8", "data": "synthetic",
         "config": bench_config(),
         "notes": "CPU arm = the reference's own Python engine on all host cores (kind reference) when its staged copy travelled with the "
@@ -242,7 +266,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-saturated", action="store_true")
     ap.add_argument("--no-evo", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the final game records and env-step counts of the last timed step "
+                                                          "(rank 0) as DIR/states.npy and DIR/steps.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup < 0:
+        ap.error("--warmup must not be negative")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed: not available with --impl reference")
     if args.impl == "reference":
         return run_reference(args)
     load_ncu_constants()
@@ -268,6 +300,7 @@ def main():
     states = eng.empty_states(n)
     flush = torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device=dev)  # > 126 MB L2
     steps_total = torch.zeros((), dtype=torch.int64, device=dev)
+    last_steps = []
 
     def one_pass(k, timed):
         seeds.copy_(base + (rank * 1_000_003 + k) * n)
@@ -280,6 +313,7 @@ def main():
         e2.record()
         if timed:
             steps_total.add_(st.sum())
+            last_steps[:] = [st]
         return e0, e1, e2
 
     for k in range(warmup):
@@ -303,6 +337,8 @@ def main():
     torch.cuda.synchronize()
     launches = eng.launches - launches0
     sampler.stop_flag = True
+    if args.dump_outputs and rank == 0:  # after the timed region: what the caller of reset + rollout_random received last
+        dump_outputs(args.dump_outputs, {"states": states, "steps": last_steps[0]})
     t_ms = sum(e0.elapsed_time(e2) for e0, _e1, e2 in events)
     t_roll_ms = sum(e1.elapsed_time(e2) for _e0, e1, e2 in events)
     tt = torch.tensor([t_ms, t_roll_ms], dtype=torch.float64, device=dev)

@@ -256,3 +256,33 @@ def test_eval_population_entry_matches_stepwise_calls(engine):
         res, _ = engine.rollout_heuristic(st, w, None if mode == "solo" else w, i1, None if mode == "solo" else i2)
         want = engine.accumulate_fitness(res, i1, torch.zeros((n_ind, 3), dtype=torch.int32, device=engine.device))
         assert torch.equal(counts, want) and int(counts.sum()) == n_games - 3
+
+
+def test_bench_dump_outputs_end_to_end(oracle, tmp_path):
+    """`bench.py --dump-outputs` on the GPU: states.npy / steps.npy are the final records and env-step counts of the LAST timed
+    step (not a warm-up pass), equal to the oracle's rollouts of the same seeds.  Rank 0's pass k (warm-up passes first,
+    max(--warmup, 3) of them) plays seeds k * games + i."""
+    import json
+    import os
+    import subprocess
+    import sys
+    from monsoon_b200.engine import DEFAULT_DECKS, DEFAULT_FACTIONS, deck_indices
+    if not torch.cuda.is_available():
+        pytest.skip("no CUDA device")
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    n, steps, warmup = 256, 2, 3
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--games", str(n), "--steps", str(steps), "--warmup", "0",
+                          "--no-saturated", "--no-evo", "--no-cpu-baseline", "--dump-outputs", str(tmp_path / "dump")],
+                         capture_output=True, text=True, timeout=600, cwd=root, env=dict(os.environ, RANK="0", WORLD_SIZE="1"))
+    assert out.returncode == 0, out.stderr[-2000:]
+    d = json.loads([l for l in out.stdout.splitlines() if l.strip()][-1])
+    assert d["steps"] == steps and d["warmup"] == warmup
+    assert sorted(os.listdir(tmp_path / "dump")) == ["states.npy", "steps.npy"]
+    states, counts = np.load(tmp_path / "dump" / "states.npy"), np.load(tmp_path / "dump" / "steps.npy")
+    assert states.dtype == np.float32 and states.shape == (n, 512) and counts.dtype == np.float32 and counts.shape == (n,)
+    d0, d1 = (deck_indices(x) for x in DEFAULT_DECKS)
+    last = warmup + steps - 1
+    for i in range(n):
+        st = oracle.new_game(last * n + i, d0, d1, *DEFAULT_FACTIONS)
+        actions, _dig, _masks = oracle.rollout_random(st, 400)
+        assert np.array_equal(states[i], st.astype(np.float32)) and counts[i] == len(actions), i

@@ -1,5 +1,6 @@
 """CPU: host-side logic of the drop-in layer (no kernels): pairing schedule, sharding, seeds, the
 reference-faithful evaluator, hall of fame, and the N>1 reduction path over gloo (world_size 2)."""
+import json
 import os
 import socket
 import subprocess
@@ -227,24 +228,39 @@ def test_checkpoint_round_trip_and_reference_class_paths(tmp_path):
     assert "evo" not in sys.modules or not hasattr(sys.modules["evo"], "__path__") or sys.modules["evo"].__path__ != []
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/evo"), reason="needs the reference checkout (build container only)")
 def test_reference_loads_our_checkpoint(tmp_path):
-    """The other direction, where the reference is present: its own Population.load_population reads our file."""
+    """The other direction: the reference's Population.load_population (evo/population.py) is a plain pickle.load of
+    evo.weights.WeightVector / evo.config.EvolutionaryConfig objects.  A fresh interpreter, with stand-in `evo` modules in place
+    of the reference's and without monsoon_b200, loads our file, and every object carries the attributes, with the types (and
+    for arrays the dtype and shape), of the same object in the checkpoint the reference itself wrote (golden/ref_population.pkl)."""
     from monsoon_b200.training import EvolutionaryConfig, dump_checkpoint
     from monsoon_b200.evo import WeightVector
     np.random.seed(4)
     vecs = [WeightVector(10) for _ in range(3)]
     path = tmp_path / "ours.pkl"
     dump_checkpoint({"generation": 2, "individuals": vecs, "fitness_scores": [0.9, 0.8, 0.7], "config": EvolutionaryConfig(mu=3, lambda_=3)}, str(path))
-    code = ("import sys, pickle, numpy as np; sys.path.insert(0, '/root/reference'); sys.path.insert(0, %r);"
-            "from evo.population import Population; from evo.config import EvolutionaryConfig; from evo.weights import WeightVector;"
-            "p = Population(EvolutionaryConfig()); p.load_population(%r);"
-            "assert p.generation == 2 and p.config.mu == 3 and type(p.individuals[0]) is WeightVector;"
-            "p.individuals[0].mutate(0.1, 0.01, 1e-5); print(repr(p.individuals[1].weights.tolist()))"
-            % (os.path.join(os.path.dirname(GOLDEN), "..", "oracle", "refshim"), str(path)))
-    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd="/root/reference")
+    evo = tmp_path / "standin" / "evo"
+    evo.mkdir(parents=True)
+    (evo / "__init__.py").write_text("")
+    (evo / "weights.py").write_text("class WeightVector:\n    pass\n")
+    (evo / "config.py").write_text("class EvolutionaryConfig:\n    pass\n")
+    code = ("import sys, json, pickle; sys.path.insert(0, %r)\n"
+            "from evo.weights import WeightVector; from evo.config import EvolutionaryConfig\n"
+            "def shape(p):\n"
+            "    d = pickle.load(open(p, 'rb'))\n"
+            "    assert type(d['config']) is EvolutionaryConfig and all(type(v) is WeightVector for v in d['individuals'])\n"
+            "    attrs = lambda o: sorted((k, type(v).__name__, str(getattr(v, 'dtype', '')), tuple(getattr(v, 'shape', ())))\n"
+            "                             for k, v in vars(o).items())\n"
+            "    return {'keys': sorted(d), 'vectors': sorted({tuple(attrs(v)) for v in d['individuals']}), 'config': attrs(d['config'])}\n"
+            "ours = pickle.load(open(%r, 'rb'))\n"
+            "assert 'monsoon_b200' not in sys.modules\n"
+            "print(json.dumps([shape(%r), shape(%r), ours['generation'], ours['config'].mu, ours['individuals'][1].weights.tolist()]))"
+            % (str(evo.parent), str(path), str(path), os.path.join(GOLDEN, "ref_population.pkl")))
+    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=str(tmp_path))
     assert out.returncode == 0, out.stderr[-2000:]
-    assert eval(out.stdout.strip().splitlines()[-1]) == vecs[1].weights.tolist()
+    ours, ref, generation, mu, weights = json.loads(out.stdout.strip().splitlines()[-1])
+    assert ours == ref
+    assert generation == 2 and mu == 3 and weights == vecs[1].weights.tolist()
 
 
 def test_training_log_rows_match_reference_format(tmp_path):
@@ -273,21 +289,26 @@ def test_config_mirror_matches_reference_defaults():
 def test_bench_reference_arm_prints_the_contract_line():
     """`bench.py --impl reference` (the CPU arm: the reference's own Python engine when its staged copy is at hand, else the
     oracle port, on all host cores; the port always printed beside it) runs without a GPU and prints ONE JSON line with the
-    keys the driver reads; ranks other than 0 print nothing."""
+    keys the driver reads; both legs time exactly --steps steps and report them; ranks other than 0 print nothing."""
     import json
     import subprocess
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     env = dict(os.environ, RANK="0", WORLD_SIZE="1")
-    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0"],
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--steps", "5", "--warmup", "1"],
                          capture_output=True, text=True, timeout=600, env=env, cwd=root)
     assert out.returncode == 0, out.stderr[-2000:]
     lines = [l for l in out.stdout.splitlines() if l.strip()]
     assert len(lines) == 1
     d = json.loads(lines[0])
     assert d["impl"] == "reference" and d["metric"] == "env_steps_per_sec" and d["unit"] == "env_steps/s"
-    assert d["value"] > 0 and d["higher_is_better"] is True and d["steps"] == 1
+    assert d["value"] > 0 and d["higher_is_better"] is True and d["steps"] == 5 and d["warmup"] == 1
     assert d["cpu_baseline"]["kind"] in ("reference", "port") and d["cpu_baseline"]["cores"] >= 1 and d["cpu_baseline"]["value"] == d["value"]
     assert d["cpu_baseline_port"]["kind"] == "port" and d["cpu_baseline_port"]["value"] > 0
+    for leg in (d["cpu_baseline"], d["cpu_baseline_port"]):
+        assert leg["timed_steps"] == 5 and leg["seconds"] > 0 and leg["value"] == leg["env_steps"] / leg["seconds"]
+    port = d["cpu_baseline_port"]
+    assert port["env_steps"] > 5 * 4096  # every timed step plays all 4,096 games to completion
+    assert d["ms_per_step"] == 1e3 * d["cpu_baseline"]["seconds"] / 5
     if d["cpu_baseline"]["kind"] == "reference":  # the Python engine is two to three orders of magnitude slower than its C restatement
         assert d["cpu_baseline_port"]["value"] > 50 * d["value"]
     assert d["e2e"] == {"value": d["value"], "unit": "env_steps/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
@@ -296,27 +317,46 @@ def test_bench_reference_arm_prints_the_contract_line():
     out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0"],
                          capture_output=True, text=True, timeout=600, env=env, cwd=root)
     assert out.returncode == 0 and out.stdout.strip() == ""
+    for bad in (["--steps", "0"], ["--steps", "1", "--dump-outputs", "unused"]):  # refused, not silently changed or ignored
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference"] + bad,
+                             capture_output=True, text=True, timeout=600, env=env, cwd=root)
+        assert out.returncode == 2 and out.stdout.strip() == "", bad
+    assert not os.path.exists(os.path.join(root, "unused"))
+
+
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs`: float32 copies of the arrays, exact for u8 records and int32 counts; above the size limit the
+    same seeded rows of every array, with their indices, and the same files from run to run."""
+    import torch
+    monkeypatch.setattr(sys, "path", list(sys.path))
+    monkeypatch.setattr(sys, "dont_write_bytecode", sys.dont_write_bytecode)
+    import bench
+    states = torch.arange(64 * 32, dtype=torch.int64).remainder(251).to(torch.uint8).view(64, 32)
+    steps = torch.arange(64, dtype=torch.int32) * 7
+    assert bench.dump_outputs(str(tmp_path / "all"), {"states": states, "steps": steps}) == ["states", "steps"]
+    got = np.load(tmp_path / "all" / "states.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, states.numpy())
+    assert np.array_equal(np.load(tmp_path / "all" / "steps.npy"), steps.numpy())
+    assert bench.DUMP_LIMIT == 64_000_000
+    monkeypatch.setattr(bench, "DUMP_LIMIT", 8192)
+    for d in ("a", "b"):
+        assert bench.dump_outputs(str(tmp_path / d), {"states": states, "steps": steps}) == ["rows", "states", "steps"]
+    rows = np.load(tmp_path / "a" / "rows.npy").astype(np.int64)
+    assert 0 < len(rows) < 64 and np.array_equal(rows, np.unique(rows))
+    assert sum(os.path.getsize(tmp_path / "a" / (k + ".npy")) for k in ("rows", "states", "steps")) <= 8192  # the files, headers too
+    for k in ("rows", "states", "steps"):
+        assert (tmp_path / "a" / (k + ".npy")).read_bytes() == (tmp_path / "b" / (k + ".npy")).read_bytes()
+    assert np.array_equal(np.load(tmp_path / "a" / "states.npy"), states.numpy()[rows])
+    assert np.array_equal(np.load(tmp_path / "a" / "steps.npy"), steps.numpy()[rows])
 
 
 def test_evolutionary_stormbound_mirror_surface():
     """games/evolutionary_stormbound.py:21-232: same public members, and -- like the reference (SURVEY Q17) -- no `.env`,
-    which is what makes the reference's adapter / evaluator fall into their AttributeError branches with this class."""
+    which is what makes the reference's adapter / evaluator fall into their AttributeError branches with this class.
+    `want` is the public callable member list read off the reference class itself (it has no `env` attribute)."""
     from monsoon_b200.games import EvolutionaryStormbound as Mirror
     want = {"to_play", "reset", "set_generation", "get_phase_info", "step", "legal_actions", "get_observation", "have_winner",
             "render", "close", "expert_agent", "action_to_string"}
-    ref_dir = "/root/reference"
-    if os.path.isdir(ref_dir):  # build container: read the member list off the reference class itself
-        import ref_harness as h
-        h.ref()
-        cwd = os.getcwd()
-        os.chdir(ref_dir)
-        try:
-            from games.evolutionary_stormbound import EvolutionaryStormbound as Ref
-        finally:
-            os.chdir(cwd)
-        ref_public = {n for n in vars(Ref) if not n.startswith("_") and callable(getattr(Ref, n))}
-        assert ref_public == want, ref_public ^ want
-        assert not hasattr(Ref, "env")
     have = {n for n in vars(Mirror) if not n.startswith("_") and callable(getattr(Mirror, n))}
     assert want <= have, want - have
     assert "env" not in vars(Mirror) and "env" not in Mirror.__init__.__code__.co_names
