@@ -132,6 +132,38 @@ int sb_rollout_heuristic(SbHandle *h, int n, uint8_t *states_d, const double *w_
                          const int32_t *idx_first_d, const int32_t *idx_second_d, int max_steps, int8_t *result_d,
                          int32_t *steps_d, void *stream);
 
+/* Batched auto-resetting environment: Game.reset / Game.step (games/stormbound.py:121-250) driven by an outside policy, and
+ * the agent-vs-expert loop of play_vs_expert.py:65-94, one env per 512-byte record of states_d u8[n,512].
+ * opponent: 0 none (self-play: the caller acts for both seats), 1 uniform-random legal agent (the stream of
+ * sb_rollout_random), 2 Stormbound.expert_action (the game's own stream, as sb_expert_action), 3 heuristic agent
+ * (sb_select_action) with weights w_opp_d f64[P,10], row idx_opp_d[g] (nullable = row g).  seat_d u8[n] (nullable = 0):
+ * the learner's seat, 0 FIRST / non-zero SECOND; ignored for opponent 0.
+ * sb_env_reset: sb_reset for seeds_d (byte-identical), then the opponent plays until the learner is to move.
+ * sb_env_step: (1) actions_d[g] outside the legal mask leaves env g untouched, result -4; (2) apply it; (3) the opponent plays
+ * until the learner is to move or the episode is over; (4) at the end of an episode the finished record goes to
+ * final_states_d and the env deals its next game in place from next_seed(Philox key of the finished record), with the same
+ * decks / factions (u8[2,n_deck] + u8[2] when decks_shared, else u8[n,2,n_deck] + u8[n,2]), and the opponent opens it when it
+ * is FIRST; (5) observation obs_d i32[n,27,5,4] with obs_err_d (observe()'s code: non-zero only for UP01-03) and legal mask
+ * masks_d u32[n,5] of the returned record.  An episode is over when a base is below 0, state.err is set, or the record's
+ * steps (both seats, since the deal) reach max_steps.  result_d i8[n]: 0 FIRST won, 1 SECOND won, -1 draw / timeout,
+ * -2 aborted by an engine status (as sb_rollout_heuristic), -3 the episode continues, -4 action rejected; length_d i32[n] =
+ * env steps of the episode that ended in this call, else 0.  Between calls every record is what chaining sb_step (plus
+ * sb_expert_action / sb_select_action for the opponent) gives.  next_seed(s): z = s + 0x9E3779B97F4A7C15,
+ * z = (z ^ z >> 30) * 0xBF58476D1CE4E5B9, z = (z ^ z >> 27) * 0x94D049BB133111EB, z ^= z >> 31, z & 0x7FFFFFFFFFFFFFFF.
+ * obs_d, masks_d, obs_err_d, final_states_d are nullable.  A bad opponent kind, kind 3 without a table, n_deck outside 1..16
+ * or max_steps outside 1..65535 returns -1 (sb_last_error) and launches nothing; n = 0 is a no-op.  One call = one kernel
+ * launch without handle scratch, atomics or host synchronisation: calls on different streams through one handle do not race,
+ * and a call can be captured in a CUDA graph.  The kernel is fixed by the opponent kind ("engine" of sb_set_option does not
+ * apply): one env per thread for 0-2, one env per warp for 3. */
+int sb_env_reset(SbHandle *h, int n, const uint64_t *seeds_d, const uint8_t *decks_d, int n_deck, int decks_shared,
+                 const uint8_t *factions_d, int opponent, const uint8_t *seat_d, const double *w_opp_d,
+                 const int32_t *idx_opp_d, int max_steps, uint8_t *states_d, int32_t *obs_d, uint32_t *masks_d,
+                 uint8_t *obs_err_d, void *stream);
+int sb_env_step(SbHandle *h, int n, uint8_t *states_d, const uint8_t *actions_d, const uint8_t *decks_d, int n_deck,
+                int decks_shared, const uint8_t *factions_d, int opponent, const uint8_t *seat_d, const double *w_opp_d,
+                const int32_t *idx_opp_d, int max_steps, int8_t *result_d, int32_t *length_d, uint8_t *final_states_d,
+                int32_t *obs_d, uint32_t *masks_d, uint8_t *obs_err_d, void *stream);
+
 /* FitnessEvaluator.evaluate_population inner reduction (evo/fitness.py:95,160-166): counts_d i32[P,3]
  * += {wins, draws, losses} of individual idx_first_d[g] over the n finished games. */
 int sb_accumulate_fitness(SbHandle *h, int n, const int8_t *result_d, const int32_t *idx_first_d, int32_t *counts_d,

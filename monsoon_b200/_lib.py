@@ -41,6 +41,8 @@ SIGNATURES = {
     "sb_expert_action": (_int, [_vp, _int, _vp, _vp, _vp]),
     "sb_rollout_random": (_int, [_vp, _int, _vp, _int, _vp, _vp, _vp]),
     "sb_rollout_heuristic": (_int, [_vp, _int, _vp, _vp, _vp, _vp, _vp, _int, _vp, _vp, _vp]),
+    "sb_env_reset": (_int, [_vp, _int, _vp, _vp, _int, _int, _vp, _int, _vp, _vp, _vp, _int, _vp, _vp, _vp, _vp, _vp]),
+    "sb_env_step": (_int, [_vp, _int, _vp, _vp, _vp, _int, _int, _vp, _int, _vp, _vp, _vp, _int, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "sb_accumulate_fitness": (_int, [_vp, _int, _vp, _vp, _vp, _vp]),
     "sb_count_aborted": (_int, [_vp, _int, _vp, _vp, _vp, _vp]),
     "sb_eval_schedule": (_int, [_vp, _int, _int, _int, _int, ctypes.c_uint64, ctypes.c_uint32, ctypes.c_int64, _int, _vp, _vp, _vp, _vp]),

@@ -13,6 +13,8 @@
 //                      warp arg-max by shuffles) -- evo/heuristic_agent.py:53-80
 //   k_rollout_heuristic  one warp per game, whole game in one launch, working-set image of the game in shared memory;
 //                      a seat without weights is played by the scripted opponent
+//   k_env_step         one env per thread: learner action, random / expert / no opponent, auto-reset, observation + mask
+//   k_env_step_heur    one env per warp: the same with a heuristic-agent opponent (decide(), as in k_rollout_heuristic)
 //   k_accumulate_fitness win/draw/loss counts per individual (evo/fitness.py:95,160-166)
 //   k_es_*             evolution-strategy operators on the resident population (sb_es.cuh; evo/weights.py, evo/population.py)
 // State is AoS [n][512 B]; every thread (or warp) moves its record with 128-bit loads/stores; the card
@@ -27,7 +29,7 @@
 #include "sb_es.cuh"
 #include "sbw_launch.h"
 
-#define SB_ABI_VERSION 1
+#define SB_ABI_VERSION 2
 #define TPB_GAME 64      // threads per CTA for thread-per-game kernels
 #define WARPS_PER_CTA 4  // games per CTA for warp-per-game kernels
 #ifndef HEUR_MIN_CTAS
@@ -44,24 +46,15 @@ SBD_FI void stage_cards(DCard* s_cards, const DCard* cards) {
 SBD_FI void init_g(G& g, const DCard* s_cards, const double* wt) { g.cards = s_cards; g.wt = wt; }
 
 // ---------------------------------------------------------------- thread-per-game kernels
-__global__ void __launch_bounds__(TPB_GAME) k_reset(int n, const unsigned long long* seeds, const u8* decks, int n_deck,
-                                                    int decks_shared, const u8* factions, u8* states, const DCard* cards,
-                                                    const double* wt) {
-  __shared__ DCard s_cards[SBC_COUNT];
-  stage_cards(s_cards, cards);
-  int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  G g;
-  init_g(g, s_cards, wt);
+// Stormbound.__init__ for one game: the working set of an all-zero record, dealt from `seed` with decks dk u8[2,n_deck]
+// and factions fc u8[2] (k_reset and the environment kernels)
+SBD_FI void new_game(G& g, unsigned long long seed, const u8* dk, int n_deck, const u8* fc) {
   __align__(16) SbState s;  // 128-bit moves
   uint4* z = reinterpret_cast<uint4*>(&s);
   for (int k = 0; k < SB_STATE_BYTES / 16; k++) z[k] = make_uint4(0, 0, 0, 0);
   unpack(g, s);
-  unsigned long long seed = seeds[i];
   g.seed_lo = (u32)seed; g.seed_hi = (u32)(seed >> 32);
   g.local_order = 0; g.current_order = 0; g.player_sign = 1; g.phase = PH_PLAY;
-  const u8* dk = decks + (decks_shared ? 0 : (size_t)i * 2 * n_deck);
-  const u8* fc = factions + (decks_shared ? 0 : (size_t)i * 2);
   for (int o = 0; o < 2; o++) {
     Ply& p = g.pl[o];
     p.max_mana = o == 0 ? 3 : 4; p.mana = p.max_mana; p.base = 20; p.front_line = o == 0 ? 4 : 0;
@@ -81,6 +74,18 @@ __global__ void __launch_bounds__(TPB_GAME) k_reset(int n, const unsigned long l
     }
     player_fill_hand(g, o);  // player.py:35
   }
+}
+__global__ void __launch_bounds__(TPB_GAME) k_reset(int n, const unsigned long long* seeds, const u8* decks, int n_deck,
+                                                    int decks_shared, const u8* factions, u8* states, const DCard* cards,
+                                                    const double* wt) {
+  __shared__ DCard s_cards[SBC_COUNT];
+  stage_cards(s_cards, cards);
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  G g;
+  init_g(g, s_cards, wt);
+  new_game(g, seeds[i], decks + (decks_shared ? 0 : (size_t)i * 2 * n_deck), n_deck, factions + (decks_shared ? 0 : (size_t)i * 2));
+  __align__(16) SbState s;  // 128-bit moves
   pack(g, s);
   store_state(states + (size_t)i * SB_STATE_BYTES, s);
 }
@@ -849,6 +854,171 @@ __global__ void __launch_bounds__(WPC * 32, MINB) k_rollout_heuristic_packed(int
   }
 }
 
+// ---------------------------------------------------------------- batched environment (sb_env_reset / sb_env_step)
+// One call moves every env from "the learner is to move" to "the learner is to move" again: check and apply the learner's
+// action, let the opponent play, close a finished episode and deal the next one in place, then emit observation and legal
+// mask.  Opponent kinds: 0 none (self-play), 1 uniform-random legal agent (the stream of k_rollout_random), 2 expert_action,
+// 3 heuristic agent (k_env_step_heur).  Episode end and result codes are those of k_rollout_heuristic.
+struct EnvArgs {
+  int n;
+  u8* states;
+  const unsigned long long* seeds;  // non-null: sb_env_reset (deal from these seeds), null: sb_env_step (apply actions)
+  const u8* actions;
+  const u8* decks; int n_deck; int decks_shared; const u8* factions;
+  int opponent; const u8* seat; const double* w_opp; const int* idx_opp; int max_steps;
+  i8* result; int* length; u8* final_states; int* obs; u32* masks; u8* obs_err;
+};
+#define ENV_CONTINUES (-3)
+#define ENV_REJECTED (-4)
+// seed of an env's next episode from the Philox key of the finished one (splitmix64 finaliser, 63 bits)
+SBD_FI unsigned long long env_next_seed(unsigned long long s) {
+  unsigned long long z = s + 0x9E3779B97F4A7C15ull;
+  z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+  z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+  z ^= z >> 31;
+  return z & 0x7FFFFFFFFFFFFFFFull;
+}
+SBD_FI unsigned long long env_key(const G& g) { return ((unsigned long long)g.seed_hi << 32) | g.seed_lo; }
+SBD_FI bool env_over(const G& g, int max_steps) { return g.pl[0].base < 0 || g.pl[1].base < 0 || g.err || (int)g.steps >= max_steps; }
+SBD_FI int env_result(const G& g) {
+  if (g.err) return -2;
+  const bool l0 = g.pl[0].base < 0, l1 = g.pl[1].base < 0;
+  return (l1 && !l0) ? 0 : (l0 && !l1) ? 1 : -1;
+}
+SBD_FI bool env_learner_moves(const G& g, const EnvArgs& a, int seat) { return a.opponent == 0 || (g.player_sign == 1 ? 0 : 1) == seat; }
+SBD_FI const u8* env_deck(const EnvArgs& a, int i) { return a.decks + (a.decks_shared ? 0 : (size_t)i * 2 * a.n_deck); }
+SBD_FI const u8* env_factions(const EnvArgs& a, int i) { return a.factions + (a.decks_shared ? 0 : (size_t)i * 2); }
+// a fresh game as sb_reset writes it, and the working set as the next sb_* call would unpack it from that record
+SBD_FI void env_deal(G& g, SbState& s, const EnvArgs& a, int i, unsigned long long seed) {
+  new_game(g, seed, env_deck(a, i), a.n_deck, env_factions(a, i));
+  pack(g, s);
+  unpack(g, s);
+}
+SBD_FI bool env_legal(const u32* m, int action) { return action < SB_N_ACTIONS && (m[action >> 5] >> (action & 31) & 1u); }
+SBD_FI void env_outputs(const G& g, const EnvArgs& a, int i, int res, int len, const u32* m) {
+  if (a.result) a.result[i] = (i8)res;
+  if (a.length) a.length[i] = len;
+  if (a.masks) for (int k = 0; k < SB_MASK_WORDS; k++) a.masks[(size_t)i * SB_MASK_WORDS + k] = m[k];
+  if (a.obs) {
+    const int e = observe(g, a.obs + (size_t)i * SB_OBS_INTS);
+    if (a.obs_err) a.obs_err[i] = (u8)e;
+  } else if (a.obs_err) {
+    int scratch[SB_OBS_INTS];
+    a.obs_err[i] = (u8)observe(g, scratch);
+  }
+}
+
+// opponents 0-2: one env per thread, the record in registers / local memory from load to store
+SBD_FI void env_opponent_thread(G& g, const EnvArgs& a, int seat) {
+  #pragma unroll 1
+  while (!env_learner_moves(g, a, seat) && !env_over(g, a.max_steps)) {
+    const int act = a.opponent == 1 ? pick_action(g) : expert_action(g);  // expert_action draws from the game's stream first
+    game_step(g, act);
+    end_of_step(g);
+  }
+}
+__global__ void __launch_bounds__(TPB_GAME) k_env_step(const EnvArgs a, const DCard* cards, const double* wt) {
+  __shared__ DCard s_cards[SBC_COUNT];
+  stage_cards(s_cards, cards);
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= a.n) return;
+  G g;
+  init_g(g, s_cards, wt);
+  __align__(16) SbState s;  // 128-bit moves
+  const int seat = a.seat && a.seat[i] ? 1 : 0;  // any non-zero seat byte is SECOND
+  int res = ENV_CONTINUES, len = 0;
+  u32 m[SB_MASK_WORDS];
+  if (a.seeds) {
+    env_deal(g, s, a, i, a.seeds[i]);
+    env_opponent_thread(g, a, seat);
+  } else {
+    load_state(s, a.states + (size_t)i * SB_STATE_BYTES);
+    unpack(g, s);
+    legal_mask(g, m);
+    if (!env_legal(m, a.actions[i])) res = ENV_REJECTED;
+    else {
+      game_step(g, a.actions[i]);
+      end_of_step(g);
+      env_opponent_thread(g, a, seat);
+      if (env_over(g, a.max_steps)) {
+        res = env_result(g); len = g.steps;
+        if (a.final_states) { pack(g, s); store_state(a.final_states + (size_t)i * SB_STATE_BYTES, s); }
+        env_deal(g, s, a, i, env_next_seed(env_key(g)));
+        env_opponent_thread(g, a, seat);
+      }
+    }
+  }
+  if (res != ENV_REJECTED) {
+    pack(g, s);
+    store_state(a.states + (size_t)i * SB_STATE_BYTES, s);
+    legal_mask(g, m);
+  }
+  env_outputs(g, a, i, res, len, m);
+}
+
+// opponent 3: one env per warp, like k_rollout_heuristic: the working-set image of the game in shared memory, decide() for the
+// opponent's decisions (a lane per candidate), lane 0 for the learner's action, the deal and the outputs
+SBD_FI void env_opponent_warp(G& g, G* base, const EnvArgs& a, const double* w, int seat) {
+  #pragma unroll 1
+  while (!env_learner_moves(*base, a, seat) && !env_over(*base, a.max_steps)) decide(g, base, w, nullptr, true);
+}
+__global__ void __launch_bounds__(WARPS_PER_CTA * 32) k_env_step_heur(const EnvArgs a, const DCard* cards, const double* wt) {
+  __shared__ DCard s_cards[SBC_COUNT];
+  extern __shared__ __align__(16) unsigned char s_dyn[];  // WARPS_PER_CTA working-set images (sizeof(G) each)
+  stage_cards(s_cards, cards);
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int i = blockIdx.x * WARPS_PER_CTA + warp;
+  if (i >= a.n) return;
+  G* base = reinterpret_cast<G*>(s_dyn) + warp;
+  G g;
+  init_g(g, s_cards, wt);
+  __align__(16) SbState s;
+  double w[SB_N_FEATURES];
+  const double* pw = a.w_opp + (size_t)(a.idx_opp ? a.idx_opp[i] : i) * SB_N_FEATURES;
+  for (int k = 0; k < SB_N_FEATURES; k++) w[k] = pw[k];
+  const int seat = a.seat && a.seat[i] ? 1 : 0;  // any non-zero seat byte is SECOND
+  int res = ENV_CONTINUES, len = 0;
+  u32 m[SB_MASK_WORDS];
+  if (lane == 0) {
+    if (a.seeds) env_deal(g, s, a, i, a.seeds[i]);
+    else {
+      load_state(s, a.states + (size_t)i * SB_STATE_BYTES);
+      unpack(g, s);
+      legal_mask(g, m);
+      if (!env_legal(m, a.actions[i])) res = ENV_REJECTED;
+      else { game_step(g, a.actions[i]); end_of_step(g); }
+    }
+    scan_badobs(g);
+    copy_g(*base, g);
+  }
+  res = __shfl_sync(0xFFFFFFFFu, res, 0);
+  __syncwarp();
+  if (res != ENV_REJECTED) {
+    env_opponent_warp(g, base, a, w, seat);
+    if (!a.seeds && env_over(*base, a.max_steps)) {  // warp-uniform: every lane reads the same image
+      __syncwarp();
+      if (lane == 0) {
+        copy_g(g, *base);
+        res = env_result(g); len = g.steps;
+        if (a.final_states) { pack(g, s); store_state(a.final_states + (size_t)i * SB_STATE_BYTES, s); }
+        env_deal(g, s, a, i, env_next_seed(env_key(g)));
+        scan_badobs(g);
+        copy_g(*base, g);
+      }
+      __syncwarp();
+      env_opponent_warp(g, base, a, w, seat);
+    }
+    __syncwarp();
+    if (lane == 0) {
+      copy_g(g, *base);
+      pack(g, s);
+      store_state(a.states + (size_t)i * SB_STATE_BYTES, s);
+      legal_mask(g, m);
+    }
+  }
+  if (lane == 0) env_outputs(g, a, i, res, len, m);
+}
+
 __global__ void k_accumulate_fitness(int n, const i8* result, const int* idx_first, int* counts) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
@@ -1366,6 +1536,42 @@ int sb_rollout_heuristic(SbHandle* h, int n, uint8_t* states_d, const double* w_
 #undef HEUR
   LAUNCH_CHECK();
   return 0;
+}
+// The environment entries launch exactly one kernel, use no handle scratch, no atomics and no host synchronisation.  The kernel
+// is fixed by the opponent kind (the "engine" option does not apply).
+static int env_launch(SbHandle* h, const EnvArgs& a, const char* what, void* stream) {
+  DEV_GUARD(h);
+  const char* bad = a.opponent < 0 || a.opponent > 3 ? "opponent must be 0..3"
+                    : a.opponent == 3 && !a.w_opp ? "opponent 3 needs a weight table"
+                    : a.n_deck < 1 || a.n_deck > SB_DECK_MAX ? "n_deck must be 1..16"
+                    : a.max_steps < 1 || a.max_steps > 65535 ? "max_steps must be 1..65535"
+                    : a.n > 0 && (!a.states || !a.decks || !a.factions || !(a.seeds || a.actions)) ? "states, decks, factions and seeds / actions are required"
+                    : nullptr;
+  if (bad) { snprintf(h->err, sizeof h->err, "%s: %s", what, bad); return -1; }
+  if (a.n <= 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (a.opponent == 3)
+    k_env_step_heur<<<grid_for(a.n, WARPS_PER_CTA), WARPS_PER_CTA * 32, WARPS_PER_CTA * sizeof(G), st>>>(a, h->d_cards, h->d_wt);
+  else
+    k_env_step<<<grid_for(a.n, TPB_GAME), TPB_GAME, 0, st>>>(a, h->d_cards, h->d_wt);
+  LAUNCH_CHECK();
+  return 0;
+}
+int sb_env_reset(SbHandle* h, int n, const uint64_t* seeds_d, const uint8_t* decks_d, int n_deck, int decks_shared,
+                 const uint8_t* factions_d, int opponent, const uint8_t* seat_d, const double* w_opp_d,
+                 const int32_t* idx_opp_d, int max_steps, uint8_t* states_d, int32_t* obs_d, uint32_t* masks_d,
+                 uint8_t* obs_err_d, void* stream) {
+  EnvArgs a = {n, states_d, (const unsigned long long*)seeds_d, nullptr, decks_d, n_deck, decks_shared, factions_d, opponent, seat_d,
+               w_opp_d, idx_opp_d, max_steps, nullptr, nullptr, nullptr, obs_d, masks_d, obs_err_d};
+  return env_launch(h, a, "sb_env_reset", stream);
+}
+int sb_env_step(SbHandle* h, int n, uint8_t* states_d, const uint8_t* actions_d, const uint8_t* decks_d, int n_deck,
+                int decks_shared, const uint8_t* factions_d, int opponent, const uint8_t* seat_d, const double* w_opp_d,
+                const int32_t* idx_opp_d, int max_steps, int8_t* result_d, int32_t* length_d, uint8_t* final_states_d,
+                int32_t* obs_d, uint32_t* masks_d, uint8_t* obs_err_d, void* stream) {
+  EnvArgs a = {n, states_d, nullptr, actions_d, decks_d, n_deck, decks_shared, factions_d, opponent, seat_d, w_opp_d, idx_opp_d,
+               max_steps, (i8*)result_d, length_d, final_states_d, obs_d, masks_d, obs_err_d};
+  return env_launch(h, a, "sb_env_step", stream);
 }
 int sb_accumulate_fitness(SbHandle* h, int n, const int8_t* result_d, const int32_t* idx_first_d, int32_t* counts_d, void* stream) {
   DEV_GUARD(h);

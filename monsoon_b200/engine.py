@@ -228,6 +228,81 @@ class Engine:
                                                   self._p(steps), self._stream()), "sb_rollout_heuristic")
         return result, steps
 
+    # ---- batched auto-resetting environment (sb_env_reset / sb_env_step)
+    def _env_args(self, n, decks, factions, opponent, seat, w_opp, idx_opp):
+        if decks is None:
+            decks, factions = self._default_deck_tensors()
+        decks = self._dev(decks, torch.uint8)
+        shared = 1 if decks.dim() == 2 else 0
+        if factions is None:
+            factions = torch.zeros((2,) if shared else (n, 2), dtype=torch.uint8, device=self.device)
+        assert decks.shape[-2] == 2 and (shared or decks.shape[0] == n), "decks are u8[2,k] (shared) or u8[n,2,k]"
+        factions = self._dev(factions, torch.uint8)
+        assert factions.shape == ((2,) if shared else (n, 2)), "factions are u8[2] with shared decks, else u8[n,2]"
+        if seat is not None:
+            self._dev(seat, torch.uint8)
+            assert seat.numel() == n
+        if w_opp is not None:  # the kernel indexes the table unchecked
+            self._dev(w_opp, torch.float64)
+            assert w_opp.dim() == 2 and w_opp.shape[1] == 10, "weight tables are f64[P, 10] (SB_N_FEATURES)"
+            if idx_opp is None:
+                assert w_opp.shape[0] >= n
+            else:
+                self._dev(idx_opp, torch.int32)
+                assert idx_opp.numel() == n
+        return decks, decks.shape[-1], shared, factions
+
+    def _default_deck_tensors(self):
+        if self._default_decks is None:
+            self._default_decks = (torch.tensor([deck_indices(d) for d in DEFAULT_DECKS], dtype=torch.uint8, device=self.device),
+                                   torch.tensor(DEFAULT_FACTIONS, dtype=torch.uint8, device=self.device))
+        return self._default_decks
+
+    def _env_outputs(self, n, out, names):
+        out = dict(out or {})
+        shapes = {"states": ((n, STATE_BYTES), torch.uint8), "obs": ((n, 27, 5, 4), torch.int32), "masks": ((n, MASK_WORDS), torch.int32),
+                  "obs_err": ((n,), torch.uint8), "result": ((n,), torch.int8), "length": ((n,), torch.int32),
+                  "final_states": ((n, STATE_BYTES), torch.uint8)}
+        for k in names:
+            shape, dtype = shapes[k]
+            if k not in out:
+                out[k] = torch.empty(shape, dtype=dtype, device=self.device)
+            elif out[k] is not None:
+                self._dev(out[k], dtype)
+                assert tuple(out[k].shape) == shape, (k, tuple(out[k].shape), shape)
+        return out
+
+    def env_reset(self, seeds, opponent=0, seat=None, w_opp=None, idx_opp=None, max_steps=400, decks=None, factions=None, out=None):
+        """sb_env_reset: deal games from seeds i64[n] and let the opponent (0 none, 1 random, 2 expert, 3 heuristic with
+        w_opp f64[P,10] / idx_opp i32[n]) play until the learner (seat u8[n], 0 FIRST / 1 SECOND) is to move.
+        out: dict of preallocated buffers (states, obs, masks, obs_err; None skips a nullable output).  Returns that dict."""
+        seeds = self._dev(seeds, torch.int64)
+        n = seeds.numel()
+        decks, n_deck, shared, factions = self._env_args(n, decks, factions, opponent, seat, w_opp, idx_opp)
+        o = self._env_outputs(n, out, ("states", "obs", "masks", "obs_err"))
+        self._check(self.lib.sb_env_reset(self.h, n, self._p(seeds), self._p(decks), n_deck, shared, self._p(factions), int(opponent),
+                                          self._p(seat), self._p(w_opp), self._p(idx_opp), int(max_steps), self._p(o["states"]),
+                                          self._p(o["obs"]), self._p(o["masks"]), self._p(o["obs_err"]), self._stream()), "sb_env_reset")
+        return o
+
+    def env_step(self, states, actions, opponent=0, seat=None, w_opp=None, idx_opp=None, max_steps=400, decks=None, factions=None,
+                 out=None):
+        """sb_env_step on states u8[n,512] in place with actions u8[n]: check, apply, opponent, auto-reset, observe.
+        out: dict of preallocated buffers (result, length, final_states, obs, masks, obs_err; None skips a nullable output).
+        Returns that dict."""
+        states = self._dev(states, torch.uint8)
+        assert states.dim() == 2 and states.shape[1] == STATE_BYTES, "states are u8[n, 512]"
+        n = states.shape[0]
+        actions = self._dev(actions, torch.uint8)
+        assert actions.numel() == n
+        decks, n_deck, shared, factions = self._env_args(n, decks, factions, opponent, seat, w_opp, idx_opp)
+        o = self._env_outputs(n, out, ("result", "length", "final_states", "obs", "masks", "obs_err"))
+        self._check(self.lib.sb_env_step(self.h, n, self._p(states), self._p(actions), self._p(decks), n_deck, shared, self._p(factions),
+                                         int(opponent), self._p(seat), self._p(w_opp), self._p(idx_opp), int(max_steps), self._p(o["result"]),
+                                         self._p(o["length"]), self._p(o["final_states"]), self._p(o["obs"]), self._p(o["masks"]),
+                                         self._p(o["obs_err"]), self._stream()), "sb_env_step")
+        return o
+
     def accumulate_fitness(self, result, idx_first, counts):
         n = result.shape[0]
         self._check(self.lib.sb_accumulate_fitness(self.h, n, self._p(result), self._p(idx_first), self._p(counts),
