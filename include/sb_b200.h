@@ -14,6 +14,7 @@
  */
 #ifndef SB_B200_H
 #define SB_B200_H
+#include <stddef.h>
 #include <stdint.h>
 #include "sb_state.h"
 #ifdef __cplusplus
@@ -163,6 +164,43 @@ int sb_env_step(SbHandle *h, int n, uint8_t *states_d, const uint8_t *actions_d,
                 int decks_shared, const uint8_t *factions_d, int opponent, const uint8_t *seat_d, const double *w_opp_d,
                 const int32_t *idx_opp_d, int max_steps, int8_t *result_d, int32_t *length_d, uint8_t *final_states_d,
                 int32_t *obs_d, uint32_t *masks_d, uint8_t *obs_err_d, void *stream);
+
+/* Batched Monte-Carlo tree search (PUCT) with a caller-supplied evaluator: n independent trees, tree g rooted at record
+ * roots_d[g] (u8[n,512]), at most max_nodes nodes each, node 0 the root.  The evaluator (prior f32[n,156] over action ids,
+ * value f32[n] from the point of view of the seat to move at the leaf) stays with the caller; the loop is
+ *   sb_search_begin -> evaluate -> (sb_search_simulate -> evaluate) x S -> sb_search_end.
+ * Transitions: the child of (s, a) is the record sb_step(s, a) produces (game_step + end_of_step on the parent record, draws
+ * from the game's own stream), so the tree sees both hands and the future draws (perfect-information search).
+ * Terminal (as sb_env_step): a base below 0, err set, or steps >= max_steps; value +1 FIRST won, -1 SECOND won, 0 draw,
+ * timeout or engine status.  Selection at a non-terminal node s: the legal a maximising q + u, q = sgn(s) W(child) / n_a
+ * (fpu when n_a = 0), u = ((c_puct P(s,a)) sqrt(N(s))) / (1 + n_a), sgn = +1 when FIRST is to move; correctly rounded
+ * FP64 in this order, ties to the lowest action id; descent continues through existing non-terminal children.  A missing
+ * child is expanded into the next free node; a terminal node ends the walk without a new node.  Backup: N += 1 and W += v
+ * (FIRST's view: the caller's value times sgn(leaf), or the game value at a terminal leaf) from the leaf to the root.
+ * Leaf outputs (all nullable): leaf_states_d u8[n,512] the leaf record, obs_d i32[n,27,5,4] / obs_err_d u8[n] (sb_observe),
+ * masks_d u32[n,5] (sb_legal_mask), to_move_d u8[n] (0 FIRST, 1 SECOND), leaf_kind_d u8[n]: 0 evaluate the leaf, 1 terminal
+ * (the game value is used, the caller's prior / value are ignored), 2 the tree is full and nothing is pending (the root is
+ * emitted).  A tree that has used all max_nodes nodes stops: that call backs up and reports 2, later calls leave it alone.
+ * sb_search_begin: root -> node 0, emitted as the first pending leaf.  sb_search_simulate: store prior_d / value_d for the
+ * pending leaf and back it up, then select, expand and emit the next leaf.  sb_search_end: back up the last pending leaf,
+ * then visits_d i32[n,156] (N of the root's children, 0 where none), q_d f64[n,156] (sgn(root) W / N of the root's
+ * children, NaN where unvisited), root_value_d f64[n] (sgn(root) W / N of the root).
+ * The workspace ws_d is caller-owned and opaque, 16-byte aligned, at least sb_search_workspace_bytes(n, max_nodes) bytes
+ * (host only, no GPU; 0 for n < 0 or max_nodes outside 1..2^24); every call of one search passes the same n, max_nodes and
+ * workspace.  Bad arguments return -1 (sb_last_error) and launch nothing: n < 0, max_nodes outside 1..2^24, a NULL,
+ * misaligned or too small workspace, max_steps outside 1..65535, c_puct negative or not finite, fpu not finite, NULL
+ * roots / prior / value / visits / q / root_value where they are used; n = 0 is a no-op.  One call = one kernel launch, one
+ * tree per thread, without handle scratch, atomics or host synchronisation: searches on different streams through one handle
+ * do not race, and a whole search with a capture-safe evaluator can be captured in a CUDA graph. */
+size_t sb_search_workspace_bytes(int n, int max_nodes);
+int sb_search_begin(SbHandle *h, int n, int max_nodes, void *ws_d, size_t ws_bytes, const uint8_t *roots_d, int max_steps,
+                    uint8_t *leaf_states_d, int32_t *obs_d, uint32_t *masks_d, uint8_t *obs_err_d, uint8_t *to_move_d,
+                    uint8_t *leaf_kind_d, void *stream);
+int sb_search_simulate(SbHandle *h, int n, int max_nodes, void *ws_d, size_t ws_bytes, const float *prior_d,
+                       const float *value_d, double c_puct, double fpu, uint8_t *leaf_states_d, int32_t *obs_d,
+                       uint32_t *masks_d, uint8_t *obs_err_d, uint8_t *to_move_d, uint8_t *leaf_kind_d, void *stream);
+int sb_search_end(SbHandle *h, int n, int max_nodes, void *ws_d, size_t ws_bytes, const float *prior_d, const float *value_d,
+                  int32_t *visits_d, double *q_d, double *root_value_d, void *stream);
 
 /* FitnessEvaluator.evaluate_population inner reduction (evo/fitness.py:95,160-166): counts_d i32[P,3]
  * += {wins, draws, losses} of individual idx_first_d[g] over the n finished games. */

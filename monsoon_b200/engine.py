@@ -303,6 +303,65 @@ class Engine:
                                          self._p(o["obs_err"]), self._stream()), "sb_env_step")
         return o
 
+    # ---- batched tree search (sb_search_begin / sb_search_simulate / sb_search_end)
+    def search_workspace_bytes(self, n, max_nodes):
+        return search_workspace_bytes(n, max_nodes)
+
+    def _search_outputs(self, n, out, names):
+        out = dict(out or {})
+        shapes = {"states": ((n, STATE_BYTES), torch.uint8), "obs": ((n, 27, 5, 4), torch.int32), "masks": ((n, MASK_WORDS), torch.int32),
+                  "obs_err": ((n,), torch.uint8), "to_move": ((n,), torch.uint8), "kind": ((n,), torch.uint8),
+                  "visits": ((n, N_ACTIONS), torch.int32), "q": ((n, N_ACTIONS), torch.float64), "root_value": ((n,), torch.float64)}
+        for k in names:
+            shape, dtype = shapes[k]
+            if k not in out:
+                out[k] = torch.empty(shape, dtype=dtype, device=self.device)
+            elif out[k] is not None:
+                self._dev(out[k], dtype)
+                assert tuple(out[k].shape) == shape, (k, tuple(out[k].shape), shape)
+        return out
+
+    def _search_eval(self, n, prior, value):
+        self._dev(prior, torch.float32)
+        self._dev(value, torch.float32)
+        assert tuple(prior.shape) == (n, N_ACTIONS) and tuple(value.shape) == (n,), "prior is f32[n,156], value f32[n]"
+
+    def search_begin(self, ws, roots, max_nodes, max_steps=400, out=None):
+        """sb_search_begin: root records u8[n,512] -> node 0 of n trees in the workspace ws (u8 tensor of at least
+        search_workspace_bytes(n, max_nodes) bytes).  out: dict of preallocated leaf buffers (states, obs, masks, obs_err,
+        to_move, kind; None skips a nullable output).  Returns that dict: the roots as the first leaves to evaluate."""
+        self._dev(ws, torch.uint8)
+        roots = self._dev(roots, torch.uint8)
+        assert roots.dim() == 2 and roots.shape[1] == STATE_BYTES, "roots are u8[n, 512]"
+        n = roots.shape[0]
+        o = self._search_outputs(n, out, ("states", "obs", "masks", "obs_err", "to_move", "kind"))
+        self._check(self.lib.sb_search_begin(self.h, n, int(max_nodes), self._p(ws), ws.numel(), self._p(roots), int(max_steps),
+                                             self._p(o["states"]), self._p(o["obs"]), self._p(o["masks"]), self._p(o["obs_err"]),
+                                             self._p(o["to_move"]), self._p(o["kind"]), self._stream()), "sb_search_begin")
+        return o
+
+    def search_simulate(self, ws, n, max_nodes, prior, value, c_puct=1.25, fpu=0.0, out=None):
+        """sb_search_simulate: back up the pending leaves with prior f32[n,156] / value f32[n] (the seat to move's view), then
+        select, expand and emit the next leaves into out (as search_begin).  Returns that dict."""
+        self._dev(ws, torch.uint8)
+        self._search_eval(n, prior, value)
+        o = self._search_outputs(n, out, ("states", "obs", "masks", "obs_err", "to_move", "kind"))
+        self._check(self.lib.sb_search_simulate(self.h, n, int(max_nodes), self._p(ws), ws.numel(), self._p(prior), self._p(value),
+                                                float(c_puct), float(fpu), self._p(o["states"]), self._p(o["obs"]), self._p(o["masks"]),
+                                                self._p(o["obs_err"]), self._p(o["to_move"]), self._p(o["kind"]), self._stream()),
+                    "sb_search_simulate")
+        return o
+
+    def search_end(self, ws, n, max_nodes, prior, value, out=None):
+        """sb_search_end: back up the last pending leaves, then read out the roots into out: visits i32[n,156], q f64[n,156]
+        (NaN where unvisited) and root_value f64[n], both for the seat to move at the root.  Returns that dict."""
+        self._dev(ws, torch.uint8)
+        self._search_eval(n, prior, value)
+        o = self._search_outputs(n, out, ("visits", "q", "root_value"))
+        self._check(self.lib.sb_search_end(self.h, n, int(max_nodes), self._p(ws), ws.numel(), self._p(prior), self._p(value),
+                                           self._p(o["visits"]), self._p(o["q"]), self._p(o["root_value"]), self._stream()), "sb_search_end")
+        return o
+
     def accumulate_fitness(self, result, idx_first, counts):
         n = result.shape[0]
         self._check(self.lib.sb_accumulate_fitness(self.h, n, self._p(result), self._p(idx_first), self._p(counts),
@@ -377,6 +436,14 @@ class Engine:
                                                     states.ctypes.data if want_states else None, steps.ctypes.data,
                                                     chain.ctypes.data if want_chain else None), "sb_rollout_random_host")
         return states, steps, chain
+
+
+def search_workspace_bytes(n, max_nodes):
+    """sb_search_workspace_bytes: bytes of the search workspace of n trees of max_nodes nodes (host only, no GPU needed)."""
+    b = int(_lib.load().sb_search_workspace_bytes(int(n), int(max_nodes)))
+    if n < 0 or max_nodes < 1 or (n > 0 and b == 0):
+        raise ValueError("no search workspace for n=%d, max_nodes=%d (n >= 0, max_nodes 1..2^24)" % (n, max_nodes))
+    return b
 
 
 _engines = {}

@@ -1,0 +1,116 @@
+"""BatchedMCTS: n independent Monte-Carlo tree searches (PUCT) on the GPU with a caller-supplied evaluator.
+
+The tree lives in a workspace on the device (sb_search_begin / sb_search_simulate / sb_search_end, include/sb_b200.h); one
+simulation is one launch that backs up the last leaf, selects a new leaf, expands it with the engine's own step and emits
+what the evaluator needs.  The evaluator stays in Python, usually a torch network:
+
+    mcts = BatchedMCTS(env.n, num_simulations=64)
+    visits, q, root_value = mcts.run(env.states, evaluate)   # evaluate(leaf, k) -> (prior f32[n,156], value f32[n])
+    obs, masks, reward, done, info = env.step(select_actions(visits))
+
+The search sees both hands and the future draws of the game's own random stream (the child of (s, a) is exactly the record
+sb_step(s, a) gives), i.e. it is a perfect-information search, like the reference agent's forks.
+"""
+import math
+
+import torch
+
+from .engine import N_ACTIONS, get_engine
+
+_PLAYER_SIGN, _ERR = 16, 18     # byte offsets in SbState (include/sb_state.h)
+_BASE_I16 = (16, 68)            # pl[0].base and pl[1].base as int16 indices (byte offsets 32 and 136)
+LEAF_KEYS = ("states", "obs", "masks", "obs_err", "to_move", "kind")
+_bits = {}
+
+
+def legal_actions(masks):
+    """bool[n,156] from legal masks i32[n,5] (u32 words, bit a of the mask = action id a)."""
+    dev = masks.device
+    if dev not in _bits:
+        _bits[dev] = torch.arange(32, dtype=torch.int32, device=dev)
+    return ((masks.unsqueeze(-1) >> _bits[dev]) & 1).reshape(masks.shape[0], -1)[:, :N_ACTIONS].bool()
+
+
+def masked_softmax(logits, masks):
+    """softmax of logits [n,156] over the legal set of masks i32[n,5]: f32, 0 at illegal action ids."""
+    x = logits.float().masked_fill(~legal_actions(masks), float("-inf"))
+    return torch.softmax(x, dim=-1).nan_to_num_(0.0)
+
+
+def rollout_evaluator(engine=None, max_steps=400):
+    """evaluate(leaf, k) with a uniform prior over the legal set (1/popcount in f32) and the value of one uniform-random
+    rollout (sb_rollout_random, at most max_steps steps) run in place on leaf["states"]: +1 / -1 when the seat to move at the
+    leaf wins / loses by the bases, 0 for a draw, an engine status or a rollout that hit max_steps."""
+    engine = engine if engine is not None else get_engine()
+    bufs = {}
+
+    def evaluate(leaf, k):
+        states = leaf["states"]
+        n = states.shape[0]
+        if bufs.get("n") != n:
+            bufs.update(n=n, prior=torch.empty((n, N_ACTIONS), dtype=torch.float32, device=states.device),
+                        value=torch.empty(n, dtype=torch.float32, device=states.device))
+        prior, value = bufs["prior"], bufs["value"]
+        legal = legal_actions(leaf["masks"])
+        inv = torch.reciprocal(legal.sum(1, keepdim=True, dtype=torch.int32).to(torch.float32))
+        torch.where(legal, inv, torch.zeros((), dtype=torch.float32, device=states.device), out=prior)
+        engine.rollout_random(states, max_steps)
+        bases = states.view(torch.int16)[:, list(_BASE_I16)]
+        lost = bases < 0
+        first = (lost[:, 1] & ~lost[:, 0]).to(torch.float32) - (lost[:, 0] & ~lost[:, 1]).to(torch.float32)
+        first.masked_fill_(states[:, _ERR] != 0, 0.0)
+        torch.mul(first, 1.0 - 2.0 * leaf["to_move"].to(torch.float32), out=value)
+        return prior, value
+
+    return evaluate
+
+
+def select_actions(visits, temperature=0.0, generator=None):
+    """One action id per row of visits i32[n,156] (int64[n]): the arg-max (ties to the lowest id) at temperature 0, else a
+    sample proportional to visits^(1/temperature).  A row without visits gives 255, which is never a legal action id."""
+    has = visits.sum(1) > 0
+    if temperature == 0:
+        a = torch.argmax(visits, dim=1)
+    else:
+        v = visits.to(torch.float64)
+        w = (v / v.amax(1, keepdim=True).clamp_min(1.0)) ** (1.0 / float(temperature))
+        w = torch.where(has.unsqueeze(1), w, torch.ones_like(w))
+        a = torch.multinomial(w, 1, generator=generator).squeeze(1)
+    return torch.where(has, a, torch.full_like(a, 255))
+
+
+class BatchedMCTS:
+    """n trees of num_simulations + 1 nodes in one workspace, with every output buffer allocated once.
+
+    run(roots, evaluate) -> (visits i32[n,156], q f64[n,156] NaN where unvisited, root_value f64[n]), q and root_value for
+    the seat to move at the root.  evaluate(leaf, k) receives the leaf buffers (dict of states u8[n,512], obs i32[n,27,5,4],
+    masks i32[n,5], obs_err u8[n], to_move u8[n], kind u8[n]: 0 evaluate, 1 terminal, 2 full) and the simulation index k
+    (0 = the roots; add exploration noise to the prior there) and returns (prior f32[n,156], value f32[n]) on the device,
+    the value from the point of view of to_move.  A run is exactly num_simulations + 2 library launches; with an evaluator
+    that only uses torch it synchronises nothing with the host and can be captured in a torch.cuda.CUDAGraph.  The returned
+    tensors are buffers of this object, overwritten by the next run.
+    """
+
+    def __init__(self, n, num_simulations, c_puct=1.25, fpu=0.0, max_steps=400, engine=None, device=None):
+        if int(num_simulations) < 0:
+            raise ValueError("num_simulations must be >= 0")
+        if not (math.isfinite(c_puct) and c_puct >= 0) or not math.isfinite(fpu):
+            raise ValueError("c_puct must be finite and >= 0, fpu finite")
+        self.engine = engine if engine is not None else get_engine(device)
+        self.n, self.num_simulations = int(n), int(num_simulations)
+        self.c_puct, self.fpu, self.max_steps = float(c_puct), float(fpu), int(max_steps)
+        self.max_nodes = self.num_simulations + 1
+        self.ws = torch.empty(self.engine.search_workspace_bytes(self.n, self.max_nodes), dtype=torch.uint8, device=self.engine.device)
+        self.leaf = self.engine._search_outputs(self.n, None, LEAF_KEYS)
+        self.out = self.engine._search_outputs(self.n, None, ("visits", "q", "root_value"))
+
+    def run(self, roots, evaluate):
+        e, n, m = self.engine, self.n, self.max_nodes
+        assert roots.shape[0] == n, "roots are u8[n, 512] with n = %d" % n
+        e.search_begin(self.ws, roots, m, self.max_steps, out=self.leaf)
+        prior, value = evaluate(self.leaf, 0)
+        for k in range(1, self.num_simulations + 1):
+            e.search_simulate(self.ws, n, m, prior, value, self.c_puct, self.fpu, out=self.leaf)
+            prior, value = evaluate(self.leaf, k)
+        e.search_end(self.ws, n, m, prior, value, out=self.out)
+        return self.out["visits"], self.out["q"], self.out["root_value"]
