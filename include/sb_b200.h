@@ -202,6 +202,22 @@ int sb_search_simulate(SbHandle *h, int n, int max_nodes, void *ws_d, size_t ws_
 int sb_search_end(SbHandle *h, int n, int max_nodes, void *ws_d, size_t ws_bytes, const float *prior_d, const float *value_d,
                   int32_t *visits_d, double *q_d, double *root_value_d, void *stream);
 
+/* Determinization for sampled (PIMC) search: out_d[g] = states_d[g] with everything observer o cannot see resampled and
+ * everything o sees kept byte for byte (sb_observe / sb_legal_mask / sb_features of o's view are unchanged).
+ * observer_d u8[n] is nullable: NULL = each record's own local_order (the seat sb_observe and sb_legal_mask show); a
+ * non-zero byte means SECOND.  keys_d u64[n] is the new Philox key of each record.  With r = 1 - o:
+ *   movable slots of pl[r]: hand 0..n_hand-1, then deck 0..n_deck-1 (clamped to 4 / 16), skipping every record whose
+ *   flags carry SB_CF_OBJ (ext[91..107] addresses those by slot); Fisher-Yates from the end over the (card, cost, flags)
+ *   triples at those slots, for i = m-1 .. 1: j = umulhi(w0, i + 1), w0 = word 0 of
+ *   philox(counter=(t, 0, 0xDE7E, 0), key=(keys_d[g] low, high)), t = 0, 1, .. the swap index; deck_wn stays with its
+ *   slot; seed_lo / seed_hi <- keys_d[g].  Every other byte is unchanged (turn, draw, steps, err, done included).
+ * The opponent's card multiset (hand + deck) is taken as known: both decks are fixed per game.  out_d may equal
+ * states_d (in place); partial overlap is undefined.  Bad arguments return -1 (sb_last_error) and launch nothing: n < 0,
+ * NULL states / keys / out with n > 0; n = 0 is a no-op.  One call = one kernel launch (one record per warp), without
+ * handle scratch, atomics or host synchronisation, so it can be captured in a CUDA graph. */
+int sb_determinize(SbHandle *h, int n, const uint8_t *states_d, const uint8_t *observer_d, const uint64_t *keys_d,
+                   uint8_t *out_d, void *stream);
+
 /* FitnessEvaluator.evaluate_population inner reduction (evo/fitness.py:95,160-166): counts_d i32[P,3]
  * += {wins, draws, losses} of individual idx_first_d[g] over the n finished games. */
 int sb_accumulate_fitness(SbHandle *h, int n, const int8_t *result_d, const int32_t *idx_first_d, int32_t *counts_d,

@@ -16,6 +16,7 @@
 //   k_env_step         one env per thread: learner action, random / expert / no opponent, auto-reset, observation + mask
 //   k_env_step_heur    one env per warp: the same with a heuristic-agent opponent (decide(), as in k_rollout_heuristic)
 //   k_search_*         batched PUCT tree search, one tree per thread, one launch per simulation (sb_search.cuh)
+//   k_determinize      one record per warp: resample what the observer cannot see (sb_determinize.cuh)
 //   k_accumulate_fitness win/draw/loss counts per individual (evo/fitness.py:95,160-166)
 //   k_es_*             evolution-strategy operators on the resident population (sb_es.cuh; evo/weights.py, evo/population.py)
 // State is AoS [n][512 B]; every thread (or warp) moves its record with 128-bit loads/stores; the card
@@ -30,7 +31,7 @@
 #include "sb_es.cuh"
 #include "sbw_launch.h"
 
-#define SB_ABI_VERSION 3
+#define SB_ABI_VERSION 4
 #define TPB_GAME 64      // threads per CTA for thread-per-game kernels
 #define WARPS_PER_CTA 4  // games per CTA for warp-per-game kernels
 #ifndef HEUR_MIN_CTAS
@@ -1023,6 +1024,9 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32) k_env_step_heur(const EnvA
 // ---------------------------------------------------------------- batched tree search (sb_search_*)
 #include "sb_search.cuh"
 
+// ---------------------------------------------------------------- determinization for sampled search (sb_determinize)
+#include "sb_determinize.cuh"
+
 __global__ void k_accumulate_fitness(int n, const i8* result, const int* idx_first, int* counts) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
@@ -1637,6 +1641,18 @@ int sb_search_end(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes
                     : n > 0 && (!visits_d || !q_d || !root_value_d) ? "visits, q and root_value are required"
                     : nullptr;
   return search_launch(h, a, ws_bytes, bad, 2, stream);
+}
+// One launch, no handle scratch, atomics or host synchronisation (capturable in a CUDA graph).
+int sb_determinize(SbHandle* h, int n, const uint8_t* states_d, const uint8_t* observer_d, const uint64_t* keys_d, uint8_t* out_d,
+                   void* stream) {
+  DEV_GUARD(h);
+  const char* bad = n < 0 ? "n must be >= 0" : n > 0 && (!states_d || !keys_d || !out_d) ? "states, keys and out are required" : nullptr;
+  if (bad) { snprintf(h->err, sizeof h->err, "sb_determinize: %s", bad); return -1; }
+  if (n == 0) return 0;
+  k_determinize<<<grid_for(n, DET_WARPS), DET_WARPS * 32, 0, (cudaStream_t)stream>>>(n, states_d, observer_d,
+                                                                                     (const unsigned long long*)keys_d, out_d);
+  LAUNCH_CHECK();
+  return 0;
 }
 int sb_accumulate_fitness(SbHandle* h, int n, const int8_t* result_d, const int32_t* idx_first_d, int32_t* counts_d, void* stream) {
   DEV_GUARD(h);

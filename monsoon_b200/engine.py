@@ -362,6 +362,26 @@ class Engine:
                                            self._p(o["visits"]), self._p(o["q"]), self._p(o["root_value"]), self._stream()), "sb_search_end")
         return o
 
+    # ---- determinization for sampled search (sb_determinize)
+    def determinize(self, states, keys, observer=None, out=None):
+        """sb_determinize: states u8[n,512] with what the observer cannot see resampled (the other seat's hand / deck
+        assignment of its cards, and the Philox key <- keys i64[n]); observer u8[n] or None (each record's local_order,
+        non-zero = SECOND).  out: u8[n,512] (a new tensor when None; may be states itself).  Returns out."""
+        states = self._dev(states, torch.uint8)
+        assert states.dim() == 2 and states.shape[1] == STATE_BYTES, "states are u8[n, 512]"
+        n = states.shape[0]
+        keys = self._dev(keys.view(torch.int64) if keys.dtype == torch.uint64 else keys, torch.int64)
+        assert tuple(keys.shape) == (n,), "keys are i64[n]"
+        if observer is not None:
+            observer = self._dev(observer, torch.uint8)
+            assert tuple(observer.shape) == (n,), "observer is u8[n]"
+        out = out if out is not None else self.empty_states(n)
+        self._dev(out, torch.uint8)
+        assert tuple(out.shape) == (n, STATE_BYTES), "out is u8[n, 512]"
+        self._check(self.lib.sb_determinize(self.h, n, self._p(states), self._p(observer), self._p(keys), self._p(out),
+                                            self._stream()), "sb_determinize")
+        return out
+
     def accumulate_fitness(self, result, idx_first, counts):
         n = result.shape[0]
         self._check(self.lib.sb_accumulate_fitness(self.h, n, self._p(result), self._p(idx_first), self._p(counts),

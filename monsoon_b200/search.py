@@ -8,14 +8,21 @@ what the evaluator needs.  The evaluator stays in Python, usually a torch networ
     visits, q, root_value = mcts.run(env.states, evaluate)   # evaluate(leaf, k) -> (prior f32[n,156], value f32[n])
     obs, masks, reward, done, info = env.step(select_actions(visits))
 
-The search sees both hands and the future draws of the game's own random stream (the child of (s, a) is exactly the record
-sb_step(s, a) gives), i.e. it is a perfect-information search, like the reference agent's forks.
+BatchedMCTS sees both hands and the future draws of the game's own random stream (the child of (s, a) is exactly the record
+sb_step(s, a) gives), i.e. it is a perfect-information search, like the reference agent's forks.  DeterminizedMCTS is the fair
+agent (Perfect-Information Monte Carlo): it searches K determinizations of each root (sb_determinize: the opponent's hand /
+deck assignment and the random stream resampled, everything the player to move sees kept) and sums the root visits:
+
+    mcts = DeterminizedMCTS(env.n, num_determinizations=8, num_simulations=8)
+    visits, q, root_value = mcts.run(env.states, rollout_evaluator())
 """
 import math
 
+import numpy as np
 import torch
 
-from .engine import N_ACTIONS, get_engine
+from .engine import N_ACTIONS, STATE_BYTES, get_engine
+from .vec_env import next_seed, next_seed_array
 
 _PLAYER_SIGN, _ERR = 16, 18     # byte offsets in SbState (include/sb_state.h)
 _BASE_I16 = (16, 68)            # pl[0].base and pl[1].base as int16 indices (byte offsets 32 and 136)
@@ -67,7 +74,9 @@ def rollout_evaluator(engine=None, max_steps=400):
 
 def select_actions(visits, temperature=0.0, generator=None):
     """One action id per row of visits i32[n,156] (int64[n]): the arg-max (ties to the lowest id) at temperature 0, else a
-    sample proportional to visits^(1/temperature).  A row without visits gives 255, which is never a legal action id."""
+    sample proportional to visits^(1/temperature).  A row without visits gives 255, which is never a legal action id.
+    visits may come from BatchedMCTS (perfect information: the search saw the opponent's cards and future draws) or from
+    DeterminizedMCTS (only what the player to move sees)."""
     has = visits.sum(1) > 0
     if temperature == 0:
         a = torch.argmax(visits, dim=1)
@@ -113,4 +122,60 @@ class BatchedMCTS:
             e.search_simulate(self.ws, n, m, prior, value, self.c_puct, self.fpu, out=self.leaf)
             prior, value = evaluate(self.leaf, k)
         e.search_end(self.ws, n, m, prior, value, out=self.out)
+        return self.out["visits"], self.out["q"], self.out["root_value"]
+
+
+class DeterminizedMCTS:
+    """Perfect-Information Monte Carlo over BatchedMCTS: n roots, K determinizations each, num_simulations per tree.
+
+    Tree t = i * K + k searches root i under determinization k: the roots are repeated into a preallocated u8[n*K,512]
+    buffer and determinized in place for each root's own local_order (the seat to move, whose hand sb_observe shows), so
+    every tree sees the root player's cards as they are and a resampled assignment of the opponent's cards to hand and
+    deck slots, with a resampled random stream.  One inner BatchedMCTS(n*K, num_simulations) runs over them and
+    evaluate(leaf, k) sees n*K leaves in that layout (rollout_evaluator works unchanged).
+
+    run(roots, evaluate, keys=None) -> (visits i32[n,156] summed over the K trees, q f64[n,156] the visit-weighted mean of
+    the trees' q, NaN where the summed visits are 0, root_value f64[n] the mean of the trees' root values), for the seat to
+    move at the root.  The root player is the observer, so the root's legal set is the same in all K trees.
+    keys: device i64[n*K], the Philox keys of the determinizations.  When None they come from `seed` and a per-object
+    call counter on the host (next_seed mix) and are copied to the device: that run is reproducible but not capture-safe.
+    With caller keys (and a capture-safe evaluator) a run synchronises nothing with the host and can be captured in a
+    torch.cuda.CUDAGraph.  A run is exactly num_simulations + 3 library launches.  The returned tensors are buffers of this
+    object, overwritten by the next run.
+    """
+
+    def __init__(self, n, num_determinizations, num_simulations, c_puct=1.25, fpu=0.0, max_steps=400, seed=0, engine=None,
+                 device=None):
+        if int(num_determinizations) < 1:
+            raise ValueError("num_determinizations must be >= 1")
+        self.n, self.k = int(n), int(num_determinizations)
+        self.inner = BatchedMCTS(self.n * self.k, num_simulations, c_puct, fpu, max_steps, engine, device)
+        self.engine = e = self.inner.engine
+        self.seed, self.calls = int(seed), 0
+        self.states = torch.empty((self.n * self.k, STATE_BYTES), dtype=torch.uint8, device=e.device)
+        self.out = e._search_outputs(self.n, None, ("visits", "q", "root_value"))
+
+    def default_keys(self):
+        """the keys of the next run without caller keys: next_seed(base + t) for tree t, base = next_seed(next_seed(seed) +
+        call index)"""
+        base = next_seed(next_seed(self.seed) + self.calls)
+        self.calls += 1
+        return next_seed_array(np.arange(self.n * self.k, dtype=np.uint64) + np.uint64(base))
+
+    def run(self, roots, evaluate, keys=None):
+        e, n, k = self.engine, self.n, self.k
+        assert roots.shape == (n, STATE_BYTES), "roots are u8[n, 512] with n = %d" % n
+        if keys is None:
+            keys = torch.from_numpy(self.default_keys()).to(e.device)
+        assert keys.shape == (n * k,), "keys are i64[n * K] with n * K = %d" % (n * k)
+        self.states.view(n, k, STATE_BYTES).copy_(roots.unsqueeze(1).expand(n, k, STATE_BYTES))
+        e.determinize(self.states, keys, out=self.states)
+        visits, q, root_value = self.inner.run(self.states, evaluate)
+        vis = visits.view(n, k, N_ACTIONS)
+        total = vis.sum(1)
+        wsum = (torch.nan_to_num(q.view(n, k, N_ACTIONS), nan=0.0) * vis).sum(1)
+        self.out["visits"].copy_(total)
+        torch.div(wsum, total, out=self.out["q"])
+        self.out["q"].masked_fill_(total == 0, float("nan"))
+        torch.mean(root_value.view(n, k), 1, out=self.out["root_value"])
         return self.out["visits"], self.out["q"], self.out["root_value"]
