@@ -180,24 +180,37 @@ def test_evaluate_vs_expert_matches_oracle(engine, oracle):
 
 
 def test_dense_variants_give_identical_states(engine):
-    """The 32-register (2,048 resident threads per SM) builds of k_step are normally chosen for batches that fill the
-    chip; forced here on a small batch they must produce the same records as the default build."""
+    """The 32-register (2,048 resident threads per SM) build k_step<true> is normally chosen for batches that fill the
+    chip; forced here on a small batch, with 8, 16 and 32 games per warp, it must give the records, rewards, done flags,
+    errors and next masks of the default build k_step<false>.  The thread-per-game engine is forced: at this batch size the
+    policy picks the warp engine, which has no dense build."""
     dev = engine.device
-    seeds = torch.arange(300, dtype=torch.int64, device=dev) + 4242
-    outs = []
+    n = 300
+    seeds = torch.arange(n, dtype=torch.int64, device=dev) + 4242
+    outs = {}
     try:
+        engine.set_option("engine", 0)
         for dense in (0, 1):
-            engine.set_option("dense", dense)
-            st = engine.reset(seeds)
-            engine.rollout_random(st, 15)
-            for _ in range(6):
-                masks = engine.legal_mask(st).cpu().numpy().view(np.uint32)
-                acts = np.array([next(a for a in range(156) if m[a >> 5] >> (a & 31) & 1) for m in masks], dtype=np.uint8)
-                engine.step(st, torch.from_numpy(acts).to(dev))
-            outs.append(st.cpu().numpy())
+            for gpw in (8, 16, 32):
+                engine.set_option("dense", dense)
+                engine.set_option("games_per_warp", gpw)
+                st = engine.reset(seeds)
+                for lo, depth in zip(range(0, n, 75), (15, 45, 65, 85)):  # late records: some games end during the steps
+                    engine.rollout_random(st[lo:lo + 75], depth)
+                trace = []
+                for _ in range(8):
+                    masks = engine.legal_mask(st).cpu().numpy().view(np.uint32)
+                    acts = np.array([next(a for a in range(156) if m[a >> 5] >> (a & 31) & 1) for m in masks], dtype=np.uint8)
+                    nm = torch.empty((n, 5), dtype=torch.int32, device=dev)
+                    trace += [t.cpu().numpy() for t in engine.step(st, torch.from_numpy(acts).to(dev), next_masks=nm)] + [nm.cpu().numpy()]
+                outs[dense, gpw] = trace + [st.cpu().numpy()]
     finally:
-        engine.set_option("dense", -1)
-    assert np.array_equal(outs[0], outs[1])
+        for k, v in (("engine", -1), ("dense", -1), ("games_per_warp", 0)):
+            engine.set_option(k, v)
+    want = outs[0, 8]
+    assert any(r.any() for r in want[0:-1:4]), "no step gave a reward: the comparison of rewards would be vacuous"
+    for key, got in outs.items():
+        assert all(np.array_equal(u, v) for u, v in zip(got, want)), key
 
 
 def test_evolutionary_stormbound(engine):

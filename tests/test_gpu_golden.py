@@ -37,7 +37,7 @@ def test_10k_default_games_lane_refill(engine):
     ok = z["err"] == 0
     seeds = torch.from_numpy(z["seeds"].astype(np.int64)).to(engine.device)
     try:
-        for bs, grid, dense in ((128, 8, 0), (1024, 2, 0), (1024, 3, 1)):  # dense = the 32-register, two-CTAs-per-SM variant
+        for bs, grid, dense in ((128, 8, 0), (256, 5, 0), (512, 4, 0), (1024, 2, 0), (1024, 3, 1)):  # dense = the 32-register, two-CTAs-per-SM variant
             engine.set_option("refill", 1)
             engine.set_option("block_sync", bs)
             engine.set_option("refill_grid", grid)
