@@ -202,7 +202,49 @@ int sb_search_simulate(SbHandle *h, int n, int max_nodes, void *ws_d, size_t ws_
 int sb_search_end(SbHandle *h, int n, int max_nodes, void *ws_d, size_t ws_bytes, const float *prior_d, const float *value_d,
                   int32_t *visits_d, double *q_d, double *root_value_d, void *stream);
 
-/* Determinization for sampled (PIMC) search: out_d[g] = states_d[g] with everything observer o cannot see resampled and
+/* Information-set Monte-Carlo tree search (single-observer ISMCTS) with a caller-supplied evaluator: n trees, tree g built
+ * over the information set of the player to move at its root, at most max_nodes nodes, node 0 the root.  The loop is
+ *   sb_ismcts_begin(world 0) -> evaluate -> (sb_ismcts_simulate(world k) -> evaluate) x S -> sb_ismcts_end.
+ * Worlds come from the caller: det_d u8[n,512] is this call's world of each root, normally sb_determinize(roots, keys_k)
+ * with fresh keys_k per call (simulation k walks world k; world 0 is the one passed to begin).  The kernels do not
+ * determinize; the caller promises that every world of tree g is a determinization of the same root for that root's own
+ * local_order, so the root's legal set is the same in every world.
+ * Nodes carry no record: parent, first child, next sibling, the move code of the edge into the node, the seat to move,
+ * N, W (FIRST's view) and the f32[156] prior the caller gave when the node was evaluated (zero for a node created terminal).
+ * Move codes (u32, kind << 24 | card << 16 | x) key an edge by what the move is, from the mover's hand in the current
+ * world, ci the hand slot: PLACE a < 64 -> (0, hand[ci].card, a & 15); SPELL 64..147 -> (1, card, (a - 64) % 21);
+ * CYCLE 148..151 -> (2, card, 0); 152..154 -> (3, hand[ci].card, hand[0].card); PASS -> 4 << 24.  When two legal ids
+ * give one code (copies of a card), the lowest id represents it and the others are never chosen.
+ * Walk (sb_ismcts_simulate, after the backup): unpack the world's record at the root; at each node (1) if the world's
+ * state is over (as sb_env_step: a base below 0, err set, or steps >= max_steps) the walk ends: a terminal leaf, kind 1,
+ * with this world's game value (a node can be terminal in one world and not in another); (2) else select among the
+ * world's legal representative ids with sb_search_simulate's PUCT formula, FP64 order and ties (n_a, W of the child with
+ * that id's code, P the node's stored prior at the world's action id); (3) step as sb_step does (game_step + end_of_step +
+ * pack + unpack) and descend into the child with the code, or expand a new node for it, emitted with kind 0, or 1 when
+ * its state is over.  Leaf outputs (all nullable) as sb_search_*: the WORLD's record at the leaf (so the evaluator never
+ * sees the true root's hidden cards or key), observation, legal mask, seat to move, kind.  Backup as sb_search_*: N += 1,
+ * W += v from the leaf to the root.  A tree that has used all max_nodes nodes stops: kind 2, the world's root record is
+ * emitted, later calls leave it alone.  sb_ismcts_end: back up the last pending leaf, then visits_d i32[n,156], q_d
+ * f64[n,156] and root_value_d f64[n] as sb_search_end, by the root's action ids through the codes stored at begin; an id
+ * that does not represent its code (or is illegal) reads 0 / NaN.
+ * Workspace: caller-owned, opaque, 16-byte aligned, at least sb_ismcts_workspace_bytes(n, max_nodes) = n * 656 * (1 +
+ * max_nodes) bytes (host only; 0 for n < 0 or max_nodes outside 1..2^24); every call of one search passes the same n,
+ * max_nodes and workspace.  Node indices read from the workspace are bounds-checked, so a workspace not written by
+ * sb_ismcts_begin cannot send a thread outside its own tree.  Bad arguments return -1 (sb_last_error) and launch nothing,
+ * as sb_search_*, plus a NULL det_d; n = 0 is a no-op.  One call = one kernel launch, one tree per thread, without handle
+ * scratch, atomics or host synchronisation (capturable in a CUDA graph with a capture-safe evaluator). */
+size_t sb_ismcts_workspace_bytes(int n, int max_nodes);
+int sb_ismcts_begin(SbHandle *h, int n, int max_nodes, void *ws_d, size_t ws_bytes, const uint8_t *det_d, int max_steps,
+                    uint8_t *leaf_states_d, int32_t *obs_d, uint32_t *masks_d, uint8_t *obs_err_d, uint8_t *to_move_d,
+                    uint8_t *leaf_kind_d, void *stream);
+int sb_ismcts_simulate(SbHandle *h, int n, int max_nodes, void *ws_d, size_t ws_bytes, const uint8_t *det_d,
+                       const float *prior_d, const float *value_d, double c_puct, double fpu, uint8_t *leaf_states_d,
+                       int32_t *obs_d, uint32_t *masks_d, uint8_t *obs_err_d, uint8_t *to_move_d, uint8_t *leaf_kind_d,
+                       void *stream);
+int sb_ismcts_end(SbHandle *h, int n, int max_nodes, void *ws_d, size_t ws_bytes, const float *prior_d, const float *value_d,
+                  int32_t *visits_d, double *q_d, double *root_value_d, void *stream);
+
+/* Determinization for sampled (PIMC) search:out_d[g] = states_d[g] with everything observer o cannot see resampled and
  * everything o sees kept byte for byte (sb_observe / sb_legal_mask / sb_features of o's view are unchanged).
  * observer_d u8[n] is nullable: NULL = each record's own local_order (the seat sb_observe and sb_legal_mask show); a
  * non-zero byte means SECOND.  keys_d u64[n] is the new Philox key of each record.  With r = 1 - o:

@@ -16,6 +16,7 @@
 //   k_env_step         one env per thread: learner action, random / expert / no opponent, auto-reset, observation + mask
 //   k_env_step_heur    one env per warp: the same with a heuristic-agent opponent (decide(), as in k_rollout_heuristic)
 //   k_search_*         batched PUCT tree search, one tree per thread, one launch per simulation (sb_search.cuh)
+//   k_ismcts_*         information-set tree search over caller-supplied worlds, one tree per thread (sb_ismcts.cuh)
 //   k_determinize      one record per warp: resample what the observer cannot see (sb_determinize.cuh)
 //   k_accumulate_fitness win/draw/loss counts per individual (evo/fitness.py:95,160-166)
 //   k_es_*             evolution-strategy operators on the resident population (sb_es.cuh; evo/weights.py, evo/population.py)
@@ -31,7 +32,7 @@
 #include "sb_es.cuh"
 #include "sbw_launch.h"
 
-#define SB_ABI_VERSION 4
+#define SB_ABI_VERSION 5
 #define TPB_GAME 64      // threads per CTA for thread-per-game kernels
 #define WARPS_PER_CTA 4  // games per CTA for warp-per-game kernels
 #ifndef HEUR_MIN_CTAS
@@ -1024,6 +1025,9 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32) k_env_step_heur(const EnvA
 // ---------------------------------------------------------------- batched tree search (sb_search_*)
 #include "sb_search.cuh"
 
+// ---------------------------------------------------------------- information-set tree search (sb_ismcts_*)
+#include "sb_ismcts.cuh"
+
 // ---------------------------------------------------------------- determinization for sampled search (sb_determinize)
 #include "sb_determinize.cuh"
 
@@ -1641,6 +1645,64 @@ int sb_search_end(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes
                     : n > 0 && (!visits_d || !q_d || !root_value_d) ? "visits, q and root_value are required"
                     : nullptr;
   return search_launch(h, a, ws_bytes, bad, 2, stream);
+}
+// The information-set search entries launch exactly one kernel, use no handle scratch, no atomics and no host synchronisation.
+size_t sb_ismcts_workspace_bytes(int n, int max_nodes) {
+  if (n < 0 || max_nodes < 1 || max_nodes > SEARCH_MAX_NODES) return 0;
+  const size_t tree = sizeof(ITree) + (size_t)max_nodes * sizeof(INode);
+  return (size_t)n > SIZE_MAX / tree ? 0 : (size_t)n * tree;
+}
+static int ismcts_launch(SbHandle* h, const SearchArgs& a, size_t ws_bytes, const char* bad, int which, void* stream) {
+  DEV_GUARD(h);
+  const size_t need = sb_ismcts_workspace_bytes(a.n, a.max_nodes);
+  if (!bad) bad = a.n < 0 ? "n must be >= 0"
+                  : a.max_nodes < 1 || a.max_nodes > SEARCH_MAX_NODES ? "max_nodes must be 1..2^24"
+                  : a.n > 0 && need == 0 ? "workspace size overflows size_t"
+                  : a.n > 0 && !a.ws ? "workspace is NULL"
+                  : ((uintptr_t)a.ws & 15) ? "workspace must be 16-byte aligned"
+                  : ws_bytes < need ? "workspace too small (sb_ismcts_workspace_bytes)"
+                  : nullptr;
+  if (bad) { snprintf(h->err, sizeof h->err, "%s: %s", which == 0 ? "sb_ismcts_begin" : which == 1 ? "sb_ismcts_simulate" : "sb_ismcts_end", bad); return -1; }
+  if (a.n == 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int grid = grid_for(a.n, TPB_GAME);
+  if (which == 0) k_ismcts_begin<<<grid, TPB_GAME, 0, st>>>(a, h->d_cards, h->d_wt);
+  else if (which == 1) k_ismcts_simulate<<<grid, TPB_GAME, 0, st>>>(a, h->d_cards, h->d_wt);
+  else k_ismcts_end<<<grid, TPB_GAME, 0, st>>>(a);
+  LAUNCH_CHECK();
+  return 0;
+}
+static size_t ismcts_tree_bytes(int max_nodes) { return sizeof(ITree) + (size_t)(max_nodes > 0 ? max_nodes : 0) * sizeof(INode); }
+int sb_ismcts_begin(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const uint8_t* det_d, int max_steps,
+                    uint8_t* leaf_states_d, int32_t* obs_d, uint32_t* masks_d, uint8_t* obs_err_d, uint8_t* to_move_d,
+                    uint8_t* leaf_kind_d, void* stream) {
+  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, ismcts_tree_bytes(max_nodes), det_d, max_steps, nullptr, nullptr, 0.0, 0.0,
+                  leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d, nullptr, nullptr, nullptr};
+  const char* bad = max_steps < 1 || max_steps > 65535 ? "max_steps must be 1..65535"
+                    : n > 0 && !det_d ? "worlds (det) are required"
+                    : nullptr;
+  return ismcts_launch(h, a, ws_bytes, bad, 0, stream);
+}
+int sb_ismcts_simulate(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const uint8_t* det_d, const float* prior_d,
+                       const float* value_d, double c_puct, double fpu, uint8_t* leaf_states_d, int32_t* obs_d, uint32_t* masks_d,
+                       uint8_t* obs_err_d, uint8_t* to_move_d, uint8_t* leaf_kind_d, void* stream) {
+  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, ismcts_tree_bytes(max_nodes), det_d, 0, prior_d, value_d, c_puct, fpu,
+                  leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d, nullptr, nullptr, nullptr};
+  const char* bad = !(c_puct >= 0.0 && c_puct <= 1.7976931348623157e308) ? "c_puct must be finite and >= 0"
+                    : !(fpu >= -1.7976931348623157e308 && fpu <= 1.7976931348623157e308) ? "fpu must be finite"
+                    : n > 0 && !det_d ? "worlds (det) are required"
+                    : n > 0 && (!prior_d || !value_d) ? "prior and value are required"
+                    : nullptr;
+  return ismcts_launch(h, a, ws_bytes, bad, 1, stream);
+}
+int sb_ismcts_end(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const float* prior_d, const float* value_d,
+                  int32_t* visits_d, double* q_d, double* root_value_d, void* stream) {
+  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, ismcts_tree_bytes(max_nodes), nullptr, 0, prior_d, value_d, 0.0, 0.0,
+                  nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, visits_d, q_d, root_value_d};
+  const char* bad = n > 0 && (!prior_d || !value_d) ? "prior and value are required"
+                    : n > 0 && (!visits_d || !q_d || !root_value_d) ? "visits, q and root_value are required"
+                    : nullptr;
+  return ismcts_launch(h, a, ws_bytes, bad, 2, stream);
 }
 // One launch, no handle scratch, atomics or host synchronisation (capturable in a CUDA graph).
 int sb_determinize(SbHandle* h, int n, const uint8_t* states_d, const uint8_t* observer_d, const uint64_t* keys_d, uint8_t* out_d,

@@ -362,6 +362,52 @@ class Engine:
                                            self._p(o["visits"]), self._p(o["q"]), self._p(o["root_value"]), self._stream()), "sb_search_end")
         return o
 
+    # ---- information-set tree search (sb_ismcts_begin / sb_ismcts_simulate / sb_ismcts_end)
+    def ismcts_workspace_bytes(self, n, max_nodes):
+        return ismcts_workspace_bytes(n, max_nodes)
+
+    def _worlds(self, det):
+        det = self._dev(det, torch.uint8)
+        assert det.dim() == 2 and det.shape[1] == STATE_BYTES, "worlds are u8[n, 512]"
+        return det
+
+    def ismcts_begin(self, ws, det, max_nodes, max_steps=400, out=None):
+        """sb_ismcts_begin: node 0 of n information-set trees in ws (u8 tensor of at least ismcts_workspace_bytes(n, max_nodes)
+        bytes) from det u8[n,512], the first world of each root (a determinization of it for its own local_order).  out: dict
+        of preallocated leaf buffers (as search_begin).  Returns that dict: the worlds' roots as the first leaves."""
+        self._dev(ws, torch.uint8)
+        det = self._worlds(det)
+        n = det.shape[0]
+        o = self._search_outputs(n, out, ("states", "obs", "masks", "obs_err", "to_move", "kind"))
+        self._check(self.lib.sb_ismcts_begin(self.h, n, int(max_nodes), self._p(ws), ws.numel(), self._p(det), int(max_steps),
+                                             self._p(o["states"]), self._p(o["obs"]), self._p(o["masks"]), self._p(o["obs_err"]),
+                                             self._p(o["to_move"]), self._p(o["kind"]), self._stream()), "sb_ismcts_begin")
+        return o
+
+    def ismcts_simulate(self, ws, det, max_nodes, prior, value, c_puct=1.25, fpu=0.0, out=None):
+        """sb_ismcts_simulate: back up the pending leaves with prior f32[n,156] / value f32[n] (the seat to move's view), then
+        walk each tree through this call's world det u8[n,512] and emit the next leaves into out (as search_begin)."""
+        self._dev(ws, torch.uint8)
+        det = self._worlds(det)
+        n = det.shape[0]
+        self._search_eval(n, prior, value)
+        o = self._search_outputs(n, out, ("states", "obs", "masks", "obs_err", "to_move", "kind"))
+        self._check(self.lib.sb_ismcts_simulate(self.h, n, int(max_nodes), self._p(ws), ws.numel(), self._p(det), self._p(prior),
+                                                self._p(value), float(c_puct), float(fpu), self._p(o["states"]), self._p(o["obs"]),
+                                                self._p(o["masks"]), self._p(o["obs_err"]), self._p(o["to_move"]), self._p(o["kind"]),
+                                                self._stream()), "sb_ismcts_simulate")
+        return o
+
+    def ismcts_end(self, ws, n, max_nodes, prior, value, out=None):
+        """sb_ismcts_end: back up the last pending leaves, then read out the roots by their action ids into out: visits
+        i32[n,156], q f64[n,156] (NaN where unvisited or not the representative of its move code) and root_value f64[n]."""
+        self._dev(ws, torch.uint8)
+        self._search_eval(n, prior, value)
+        o = self._search_outputs(n, out, ("visits", "q", "root_value"))
+        self._check(self.lib.sb_ismcts_end(self.h, n, int(max_nodes), self._p(ws), ws.numel(), self._p(prior), self._p(value),
+                                           self._p(o["visits"]), self._p(o["q"]), self._p(o["root_value"]), self._stream()), "sb_ismcts_end")
+        return o
+
     # ---- determinization for sampled search (sb_determinize)
     def determinize(self, states, keys, observer=None, out=None):
         """sb_determinize: states u8[n,512] with what the observer cannot see resampled (the other seat's hand / deck
@@ -463,6 +509,14 @@ def search_workspace_bytes(n, max_nodes):
     b = int(_lib.load().sb_search_workspace_bytes(int(n), int(max_nodes)))
     if n < 0 or max_nodes < 1 or (n > 0 and b == 0):
         raise ValueError("no search workspace for n=%d, max_nodes=%d (n >= 0, max_nodes 1..2^24)" % (n, max_nodes))
+    return b
+
+
+def ismcts_workspace_bytes(n, max_nodes):
+    """sb_ismcts_workspace_bytes: bytes of the information-set search workspace of n trees of max_nodes nodes (host only)."""
+    b = int(_lib.load().sb_ismcts_workspace_bytes(int(n), int(max_nodes)))
+    if n < 0 or max_nodes < 1 or (n > 0 and b == 0):
+        raise ValueError("no ISMCTS workspace for n=%d, max_nodes=%d (n >= 0, max_nodes 1..2^24)" % (n, max_nodes))
     return b
 
 

@@ -15,6 +15,13 @@ deck assignment and the random stream resampled, everything the player to move s
 
     mcts = DeterminizedMCTS(env.n, num_determinizations=8, num_simulations=8)
     visits, q, root_value = mcts.run(env.states, rollout_evaluator())
+
+InformationSetMCTS is the information-set search (single-observer ISMCTS, sb_ismcts_*): one tree per root over what the
+player to move sees, every simulation walking it through a fresh determinization, so the simulations are not split into K
+separate trees that each believe their own world:
+
+    mcts = InformationSetMCTS(env.n, num_simulations=64)
+    visits, q, root_value = mcts.run(env.states, rollout_evaluator())
 """
 import math
 
@@ -76,7 +83,7 @@ def select_actions(visits, temperature=0.0, generator=None):
     """One action id per row of visits i32[n,156] (int64[n]): the arg-max (ties to the lowest id) at temperature 0, else a
     sample proportional to visits^(1/temperature).  A row without visits gives 255, which is never a legal action id.
     visits may come from BatchedMCTS (perfect information: the search saw the opponent's cards and future draws) or from
-    DeterminizedMCTS (only what the player to move sees)."""
+    DeterminizedMCTS / InformationSetMCTS (only what the player to move sees)."""
     has = visits.sum(1) > 0
     if temperature == 0:
         a = torch.argmax(visits, dim=1)
@@ -178,4 +185,61 @@ class DeterminizedMCTS:
         torch.div(wsum, total, out=self.out["q"])
         self.out["q"].masked_fill_(total == 0, float("nan"))
         torch.mean(root_value.view(n, k), 1, out=self.out["root_value"])
+        return self.out["visits"], self.out["q"], self.out["root_value"]
+
+
+class InformationSetMCTS:
+    """Information-set MCTS: n roots, one tree each over the root player's information set, num_simulations per tree.
+
+    Every call of the search gets a fresh world per root: sb_determinize(roots, keys_k) for the root's own local_order (the
+    seat to move) into one preallocated u8[n,512] buffer, then sb_ismcts_begin (k = 0) or sb_ismcts_simulate (k = 1..S)
+    walks the tree through it.  Edges are keyed by move codes (card and target, not hand slot), so the tree is shared by
+    every world.  evaluate(leaf, k) receives the leaf buffers as in BatchedMCTS; leaf["states"] holds the world's record at
+    the leaf, never the root's hidden cards or key, so rollout_evaluator works unchanged.
+
+    run(roots, evaluate, keys=None) -> (visits i32[n,156], q f64[n,156] NaN where unvisited, root_value f64[n]), for the seat
+    to move at the root, by the root's action ids (an id that plays the same card as a lower legal id reads 0 / NaN).
+    keys: device i64[(S+1)*n], simulation-major (keys[k*n:(k+1)*n] are the worlds of call k).  When None they come from
+    `seed` and a per-object call counter on the host (next_seed mix) and are copied to the device: reproducible but not
+    capture-safe.  With caller keys (and a capture-safe evaluator) a run synchronises nothing with the host and can be
+    captured in a torch.cuda.CUDAGraph.  A run is exactly 2 * num_simulations + 3 library launches (S + 1 sb_determinize,
+    begin, S simulate, end).  The returned tensors are buffers of this object, overwritten by the next run.
+    """
+
+    def __init__(self, n, num_simulations, c_puct=1.25, fpu=0.0, max_steps=400, seed=0, engine=None, device=None):
+        if int(num_simulations) < 0:
+            raise ValueError("num_simulations must be >= 0")
+        if not (math.isfinite(c_puct) and c_puct >= 0) or not math.isfinite(fpu):
+            raise ValueError("c_puct must be finite and >= 0, fpu finite")
+        self.engine = e = engine if engine is not None else get_engine(device)
+        self.n, self.num_simulations = int(n), int(num_simulations)
+        self.c_puct, self.fpu, self.max_steps = float(c_puct), float(fpu), int(max_steps)
+        self.max_nodes = self.num_simulations + 1
+        self.seed, self.calls = int(seed), 0
+        self.ws = torch.empty(e.ismcts_workspace_bytes(self.n, self.max_nodes), dtype=torch.uint8, device=e.device)
+        self.world = torch.empty((self.n, STATE_BYTES), dtype=torch.uint8, device=e.device)
+        self.leaf = e._search_outputs(self.n, None, LEAF_KEYS)
+        self.out = e._search_outputs(self.n, None, ("visits", "q", "root_value"))
+
+    def default_keys(self):
+        """the keys of the next run without caller keys: next_seed(base + t) for t < (S+1)*n, base = next_seed(next_seed(seed)
+        + call index)"""
+        base = next_seed(next_seed(self.seed) + self.calls)
+        self.calls += 1
+        return next_seed_array(np.arange(self.max_nodes * self.n, dtype=np.uint64) + np.uint64(base))
+
+    def run(self, roots, evaluate, keys=None):
+        e, n, m = self.engine, self.n, self.max_nodes
+        assert roots.shape == (n, STATE_BYTES), "roots are u8[n, 512] with n = %d" % n
+        if keys is None:
+            keys = torch.from_numpy(self.default_keys()).to(e.device)
+        assert keys.shape == (m * n,), "keys are i64[(S + 1) * n] with (S + 1) * n = %d" % (m * n)
+        e.determinize(roots, keys[:n], out=self.world)
+        e.ismcts_begin(self.ws, self.world, m, self.max_steps, out=self.leaf)
+        prior, value = evaluate(self.leaf, 0)
+        for k in range(1, self.num_simulations + 1):
+            e.determinize(roots, keys[k * n:(k + 1) * n], out=self.world)
+            e.ismcts_simulate(self.ws, self.world, m, prior, value, self.c_puct, self.fpu, out=self.leaf)
+            prior, value = evaluate(self.leaf, k)
+        e.ismcts_end(self.ws, n, m, prior, value, out=self.out)
         return self.out["visits"], self.out["q"], self.out["root_value"]
