@@ -244,6 +244,45 @@ int sb_ismcts_simulate(SbHandle *h, int n, int max_nodes, void *ws_d, size_t ws_
 int sb_ismcts_end(SbHandle *h, int n, int max_nodes, void *ws_d, size_t ws_bytes, const float *prior_d, const float *value_d,
                   int32_t *visits_d, double *q_d, double *root_value_d, void *stream);
 
+/* Gumbel search (Gumbel MuZero, Danihelka et al. 2022; mctx's gumbel_muzero_policy) for both tree searches, ABI 5's additive
+ * entry points.  A search is the PUCT begin, then S calls of the Gumbel simulate with sim = 1..S, then the Gumbel end:
+ *   sb_search_begin -> evaluate -> (sb_search_simulate_gumbel(sim = k) -> evaluate) x S -> sb_search_end_gumbel
+ *   sb_ismcts_begin(world 0) -> evaluate -> (sb_ismcts_simulate_gumbel(world k, sim = k) -> evaluate) x S -> sb_ismcts_end_gumbel
+ * Workspaces, backup, expansion, terminal rule, leaf outputs and full trees are those of sb_search_* / sb_ismcts_*; mixing
+ * PUCT and Gumbel calls in one search is unsupported.  gumbel_d f32[n,156] is the caller's Gumbel noise (normally
+ * -log(-log u)), the same for every call of one search; only entries at legal ids are read.  Selection (correctly rounded
+ * FP64, log / exp the library's own, DESIGN.md 8.9), at a non-terminal node s with legal set A (8.6: its legal ids; 8.8: the
+ * world's legal representatives, children by move code), n_a / W_a of a's child, q_a = sgn(s) W_a / n_a:
+ *   vhat = sgn (W(s) - sum_children W) / (N(s) - sum_children N) (0 if that denominator is < 1);
+ *   vmix = (vhat + sumN * (sum_{n_a>0} p~_a q_a / sum_{n_a>0} p~_a)) / (1 + sumN), p~ = max(prior, 2^-126), sumN = sum_A n_a;
+ *   completed q = q_a (n_a > 0) else vmix, rescaled to [0, 1] over A (range floor 1e-8);
+ *   sigma_a = (c_visit + max_A n) * c_scale * rescaled q_a;  logit_a = log(prior_a) (-1e9 where prior_a <= 0);
+ *   interior nodes: argmax_A of softmax_A(logit + sigma)_a - n_a / (1 + sumN);
+ *   the root at call sim = k: argmax of max(-1e9, g_a + logit_a + sigma_a) over the ids whose n_a equals seq(m, S)[k-1]
+ *   (all of A when none does), m = min(max_considered, |A|), seq mctx's sequential-halving visit schedule.
+ * Ties go to the lowest id and a NaN never wins, so a non-empty A always gives a legal id.  The end backs up the last pending
+ * leaf and writes visits_d, q_d and root_value_d exactly as sb_search_end / sb_ismcts_end, plus action_d i32[n] (argmax of
+ * g + logit + sigma over the ids with the most root visits; 255 when no root id has a visit, e.g. a terminal root) and
+ * policy_d f32[n,156] (the softmax of logit + sigma over A with the final counts, 0 outside A; 8.8's A at the end is the ids
+ * with a root code, so an id that repeats a lower id's card reads 0).  Bad arguments return -1 and launch nothing: those of
+ * the PUCT sibling, sim outside 1..num_simulations, num_simulations outside 1..2^24, max_considered outside 1..156, c_visit
+ * or c_scale negative or not finite, a NULL gumbel (and, at the end, action or policy) with n > 0; n = 0 is a no-op.  One
+ * call = one kernel launch, without handle scratch, atomics or host synchronisation (capturable in a CUDA graph). */
+int sb_search_simulate_gumbel(SbHandle *h, int n, int max_nodes, void *ws_d, size_t ws_bytes, const float *prior_d,
+                              const float *value_d, const float *gumbel_d, int sim, int num_simulations, int max_considered,
+                              double c_visit, double c_scale, uint8_t *leaf_states_d, int32_t *obs_d, uint32_t *masks_d,
+                              uint8_t *obs_err_d, uint8_t *to_move_d, uint8_t *leaf_kind_d, void *stream);
+int sb_search_end_gumbel(SbHandle *h, int n, int max_nodes, void *ws_d, size_t ws_bytes, const float *prior_d,
+                         const float *value_d, const float *gumbel_d, double c_visit, double c_scale, int32_t *action_d,
+                         float *policy_d, int32_t *visits_d, double *q_d, double *root_value_d, void *stream);
+int sb_ismcts_simulate_gumbel(SbHandle *h, int n, int max_nodes, void *ws_d, size_t ws_bytes, const uint8_t *det_d,
+                              const float *prior_d, const float *value_d, const float *gumbel_d, int sim, int num_simulations,
+                              int max_considered, double c_visit, double c_scale, uint8_t *leaf_states_d, int32_t *obs_d,
+                              uint32_t *masks_d, uint8_t *obs_err_d, uint8_t *to_move_d, uint8_t *leaf_kind_d, void *stream);
+int sb_ismcts_end_gumbel(SbHandle *h, int n, int max_nodes, void *ws_d, size_t ws_bytes, const float *prior_d,
+                         const float *value_d, const float *gumbel_d, double c_visit, double c_scale, int32_t *action_d,
+                         float *policy_d, int32_t *visits_d, double *q_d, double *root_value_d, void *stream);
+
 /* Determinization for sampled (PIMC) search:out_d[g] = states_d[g] with everything observer o cannot see resampled and
  * everything o sees kept byte for byte (sb_observe / sb_legal_mask / sb_features of o's view are unchanged).
  * observer_d u8[n] is nullable: NULL = each record's own local_order (the seat sb_observe and sb_legal_mask show); a

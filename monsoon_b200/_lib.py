@@ -54,6 +54,14 @@ SIGNATURES = {
     "sb_ismcts_simulate": (_int, [_vp, _int, _int, _vp, ctypes.c_size_t, _vp, _vp, _vp, ctypes.c_double, ctypes.c_double, _vp, _vp, _vp,
                                   _vp, _vp, _vp, _vp]),
     "sb_ismcts_end": (_int, [_vp, _int, _int, _vp, ctypes.c_size_t, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "sb_search_simulate_gumbel": (_int, [_vp, _int, _int, _vp, ctypes.c_size_t, _vp, _vp, _vp, _int, _int, _int, ctypes.c_double,
+                                         ctypes.c_double, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "sb_search_end_gumbel": (_int, [_vp, _int, _int, _vp, ctypes.c_size_t, _vp, _vp, _vp, ctypes.c_double, ctypes.c_double, _vp, _vp,
+                                    _vp, _vp, _vp, _vp]),
+    "sb_ismcts_simulate_gumbel": (_int, [_vp, _int, _int, _vp, ctypes.c_size_t, _vp, _vp, _vp, _vp, _int, _int, _int, ctypes.c_double,
+                                         ctypes.c_double, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "sb_ismcts_end_gumbel": (_int, [_vp, _int, _int, _vp, ctypes.c_size_t, _vp, _vp, _vp, ctypes.c_double, ctypes.c_double, _vp, _vp,
+                                    _vp, _vp, _vp, _vp]),
     "sb_accumulate_fitness": (_int, [_vp, _int, _vp, _vp, _vp, _vp]),
     "sb_count_aborted": (_int, [_vp, _int, _vp, _vp, _vp, _vp]),
     "sb_eval_schedule": (_int, [_vp, _int, _int, _int, _int, ctypes.c_uint64, ctypes.c_uint32, ctypes.c_int64, _int, _vp, _vp, _vp, _vp]),

@@ -216,26 +216,11 @@ __global__ void __launch_bounds__(TPB_GAME) k_ismcts_begin(const SearchArgs a, c
   ism_emit(a, i, g, s, m, t.kind);
 }
 
-__global__ void __launch_bounds__(TPB_GAME) k_ismcts_simulate(const SearchArgs a, const DCard* cards, const double* wt) {
-  __shared__ DCard s_cards[SBC_COUNT];
-  stage_cards(s_cards, cards);
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= a.n) return;
-  G g;
-  init_g(g, s_cards, wt);
-  ITree& t = ism_tree(a, i);
-  INode* nodes = ism_nodes(a, i);
-  ism_backup(a, i, t, nodes);
-  __align__(16) SbState s;
-  load_state(s, a.roots + (size_t)i * SB_STATE_BYTES);  // this call's world at the root
-  unpack(g, s);
-  u32 m[SB_MASK_WORDS];
-  legal_mask(g, m);
-  if (t.kind == SEARCH_FULL || t.used < 1 || t.used >= a.max_nodes) {  // the tree stops: the world's root is emitted
-    t.kind = SEARCH_FULL;
-    ism_emit(a, i, g, s, m, SEARCH_FULL);
-    return;
-  }
+// one simulation's walk after the backup, in this call's world (record s, working set g, legal mask m at the root):
+// select(j, lim, c) chooses the action at node j among the world's legal representatives and sets c to the child with its
+// code (-1 = none).  Every node index is checked against lim and the descent is bounded by max_nodes.
+template <class Select>
+SBD_FI void ism_walk(const SearchArgs& a, int i, G& g, ITree& t, INode* nodes, SbState& s, u32* m, Select select) {
   const int lim = t.used;
   int j = 0;
   #pragma unroll 1
@@ -248,7 +233,7 @@ __global__ void __launch_bounds__(TPB_GAME) k_ismcts_simulate(const SearchArgs a
       return;
     }
     int c;
-    const int act = ism_select(a, nodes, lim, nodes[j], g.pl[g.local_order], m, c);
+    const int act = select(j, lim, c);
     if (act < 0) break;
     const u32 code = ism_code(g.pl[g.local_order], act);
     game_step(g, act);  // as sb_step: the working set the next sb_* call would unpack from the child's record
@@ -285,24 +270,43 @@ __global__ void __launch_bounds__(TPB_GAME) k_ismcts_simulate(const SearchArgs a
   ism_emit(a, i, g, s, m, SEARCH_FULL);
 }
 
-// back up the last pending leaf (the tree then holds nothing pending) and read out the root's edges by the root's action ids
-__global__ void __launch_bounds__(TPB_GAME) k_ismcts_end(const SearchArgs a) {
+__global__ void __launch_bounds__(TPB_GAME) k_ismcts_simulate(const SearchArgs a, const DCard* cards, const double* wt) {
+  __shared__ DCard s_cards[SBC_COUNT];
+  stage_cards(s_cards, cards);
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= a.n) return;
+  G g;
+  init_g(g, s_cards, wt);
   ITree& t = ism_tree(a, i);
   INode* nodes = ism_nodes(a, i);
   ism_backup(a, i, t, nodes);
-  t.kind = SEARCH_FULL;
-  const int lim = ism_lim(t, a.max_nodes);
-  const double nan = __longlong_as_double(0x7FF8000000000000ll);
-  if (lim < 1) {
-    #pragma unroll 1
-    for (int act = 0; act < SB_N_ACTIONS; act++) { a.visits[(size_t)i * SB_N_ACTIONS + act] = 0; a.q[(size_t)i * SB_N_ACTIONS + act] = nan; }
-    a.root_value[i] = nan;
+  __align__(16) SbState s;
+  load_state(s, a.roots + (size_t)i * SB_STATE_BYTES);  // this call's world at the root
+  unpack(g, s);
+  u32 m[SB_MASK_WORDS];
+  legal_mask(g, m);
+  if (t.kind == SEARCH_FULL || t.used < 1 || t.used >= a.max_nodes) {  // the tree stops: the world's root is emitted
+    t.kind = SEARCH_FULL;
+    ism_emit(a, i, g, s, m, SEARCH_FULL);
     return;
   }
+  ism_walk(a, i, g, t, nodes, s, m, [&](int j, int lim, int& c) { return ism_select(a, nodes, lim, nodes[j], g.pl[g.local_order], m, c); });
+}
+
+// the child of node nd whose code is `code` (first in the sibling walk), -1 if none
+SBD_FI int ism_find(const INode* nodes, int lim, const INode& nd, u32 code) {
+  int c = nd.child;
+  #pragma unroll 1
+  for (int k = 0; k < lim && ism_in(c, lim); k++, c = nodes[c].sibling)
+    if (nodes[c].code == code) return c;
+  return -1;
+}
+
+// visits, q and root_value of tree i by the root's action ids (sb_ismcts_end), lim >= 1
+SBD_FI void ism_read_out(const SearchArgs& a, int i, const ITree& t, const INode* nodes, int lim) {
   const INode& root = nodes[0];
   const double sgn = s_sign(root.seat);
+  const double nan = __longlong_as_double(0x7FF8000000000000ll);
   #pragma unroll 1
   for (int act = 0; act < SB_N_ACTIONS; act++) {
     const u32 code = t.root_code[act];
@@ -318,4 +322,27 @@ __global__ void __launch_bounds__(TPB_GAME) k_ismcts_end(const SearchArgs a) {
     a.q[(size_t)i * SB_N_ACTIONS + act] = na ? __ddiv_rn(__dmul_rn(sgn, w), (double)na) : nan;
   }
   a.root_value[i] = __ddiv_rn(__dmul_rn(sgn, root.W), (double)root.N);
+}
+// the read-out of a tree whose header holds no usable node count
+SBD_FI void ism_read_out_empty(const SearchArgs& a, int i) {
+  const double nan = __longlong_as_double(0x7FF8000000000000ll);
+  #pragma unroll 1
+  for (int act = 0; act < SB_N_ACTIONS; act++) { a.visits[(size_t)i * SB_N_ACTIONS + act] = 0; a.q[(size_t)i * SB_N_ACTIONS + act] = nan; }
+  a.root_value[i] = nan;
+}
+
+// back up the last pending leaf (the tree then holds nothing pending) and read out the root's edges by the root's action ids
+__global__ void __launch_bounds__(TPB_GAME) k_ismcts_end(const SearchArgs a) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= a.n) return;
+  ITree& t = ism_tree(a, i);
+  INode* nodes = ism_nodes(a, i);
+  ism_backup(a, i, t, nodes);
+  t.kind = SEARCH_FULL;
+  const int lim = ism_lim(t, a.max_nodes);
+  if (lim < 1) {
+    ism_read_out_empty(a, i);
+    return;
+  }
+  ism_read_out(a, i, t, nodes, lim);
 }

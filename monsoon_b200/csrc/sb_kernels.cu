@@ -17,6 +17,7 @@
 //   k_env_step_heur    one env per warp: the same with a heuristic-agent opponent (decide(), as in k_rollout_heuristic)
 //   k_search_*         batched PUCT tree search, one tree per thread, one launch per simulation (sb_search.cuh)
 //   k_ismcts_*         information-set tree search over caller-supplied worlds, one tree per thread (sb_ismcts.cuh)
+//   k_*_gumbel         Gumbel selection and read-out for both tree searches (sb_gumbel.cuh)
 //   k_determinize      one record per warp: resample what the observer cannot see (sb_determinize.cuh)
 //   k_accumulate_fitness win/draw/loss counts per individual (evo/fitness.py:95,160-166)
 //   k_es_*             evolution-strategy operators on the resident population (sb_es.cuh; evo/weights.py, evo/population.py)
@@ -1028,6 +1029,9 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32) k_env_step_heur(const EnvA
 // ---------------------------------------------------------------- information-set tree search (sb_ismcts_*)
 #include "sb_ismcts.cuh"
 
+// ---------------------------------------------------------------- Gumbel search for both trees (sb_*_gumbel)
+#include "sb_gumbel.cuh"
+
 // ---------------------------------------------------------------- determinization for sampled search (sb_determinize)
 #include "sb_determinize.cuh"
 
@@ -1652,16 +1656,19 @@ size_t sb_ismcts_workspace_bytes(int n, int max_nodes) {
   const size_t tree = sizeof(ITree) + (size_t)max_nodes * sizeof(INode);
   return (size_t)n > SIZE_MAX / tree ? 0 : (size_t)n * tree;
 }
+static const char* ismcts_bad(const SearchArgs& a, size_t ws_bytes) {
+  const size_t need = sb_ismcts_workspace_bytes(a.n, a.max_nodes);
+  return a.n < 0 ? "n must be >= 0"
+         : a.max_nodes < 1 || a.max_nodes > SEARCH_MAX_NODES ? "max_nodes must be 1..2^24"
+         : a.n > 0 && need == 0 ? "workspace size overflows size_t"
+         : a.n > 0 && !a.ws ? "workspace is NULL"
+         : ((uintptr_t)a.ws & 15) ? "workspace must be 16-byte aligned"
+         : ws_bytes < need ? "workspace too small (sb_ismcts_workspace_bytes)"
+         : nullptr;
+}
 static int ismcts_launch(SbHandle* h, const SearchArgs& a, size_t ws_bytes, const char* bad, int which, void* stream) {
   DEV_GUARD(h);
-  const size_t need = sb_ismcts_workspace_bytes(a.n, a.max_nodes);
-  if (!bad) bad = a.n < 0 ? "n must be >= 0"
-                  : a.max_nodes < 1 || a.max_nodes > SEARCH_MAX_NODES ? "max_nodes must be 1..2^24"
-                  : a.n > 0 && need == 0 ? "workspace size overflows size_t"
-                  : a.n > 0 && !a.ws ? "workspace is NULL"
-                  : ((uintptr_t)a.ws & 15) ? "workspace must be 16-byte aligned"
-                  : ws_bytes < need ? "workspace too small (sb_ismcts_workspace_bytes)"
-                  : nullptr;
+  if (!bad) bad = ismcts_bad(a, ws_bytes);
   if (bad) { snprintf(h->err, sizeof h->err, "%s: %s", which == 0 ? "sb_ismcts_begin" : which == 1 ? "sb_ismcts_simulate" : "sb_ismcts_end", bad); return -1; }
   if (a.n == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
@@ -1703,6 +1710,87 @@ int sb_ismcts_end(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes
                     : n > 0 && (!visits_d || !q_d || !root_value_d) ? "visits, q and root_value are required"
                     : nullptr;
   return ismcts_launch(h, a, ws_bytes, bad, 2, stream);
+}
+// The Gumbel entries: the checks of their PUCT siblings plus the Gumbel arguments; one launch each, no handle scratch, no
+// atomics and no host synchronisation.
+static const char* gumbel_bad(int n, const GumbelArgs& gb, bool end) {
+  const double big = 1.7976931348623157e308;
+  return !(gb.c_visit >= 0.0 && gb.c_visit <= big) ? "c_visit must be finite and >= 0"
+         : !(gb.c_scale >= 0.0 && gb.c_scale <= big) ? "c_scale must be finite and >= 0"
+         : n > 0 && !gb.gumbel ? "gumbel is required"
+         : end && n > 0 && (!gb.action || !gb.policy) ? "action and policy are required"
+         : end ? nullptr
+         : gb.num_simulations < 1 || gb.num_simulations > GUMBEL_MAX_SIMULATIONS ? "num_simulations must be 1..2^24"
+         : gb.sim < 1 || gb.sim > gb.num_simulations ? "sim must be 1..num_simulations"
+         : gb.max_considered < 1 || gb.max_considered > SB_N_ACTIONS ? "max_considered must be 1..156"
+         : nullptr;
+}
+int sb_search_simulate_gumbel(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const float* prior_d,
+                              const float* value_d, const float* gumbel_d, int sim, int num_simulations, int max_considered,
+                              double c_visit, double c_scale, uint8_t* leaf_states_d, int32_t* obs_d, uint32_t* masks_d,
+                              uint8_t* obs_err_d, uint8_t* to_move_d, uint8_t* leaf_kind_d, void* stream) {
+  DEV_GUARD(h);
+  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, sizeof(STree) + (size_t)(max_nodes > 0 ? max_nodes : 0) * sizeof(SNode), nullptr,
+                  0, prior_d, value_d, 0.0, 0.0, leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d,
+                  nullptr, nullptr, nullptr};
+  const GumbelArgs gb = {gumbel_d, sim, num_simulations, max_considered, c_visit, c_scale, nullptr, nullptr};
+  const char* bad = gumbel_bad(n, gb, false);
+  if (!bad) bad = n > 0 && (!prior_d || !value_d) ? "prior and value are required" : search_bad(a, ws_bytes);
+  if (bad) { snprintf(h->err, sizeof h->err, "sb_search_simulate_gumbel: %s", bad); return -1; }
+  if (n == 0) return 0;
+  k_search_simulate_gumbel<<<grid_for(n, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a, gb, h->d_cards, h->d_wt);
+  LAUNCH_CHECK();
+  return 0;
+}
+int sb_search_end_gumbel(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const float* prior_d, const float* value_d,
+                         const float* gumbel_d, double c_visit, double c_scale, int32_t* action_d, float* policy_d,
+                         int32_t* visits_d, double* q_d, double* root_value_d, void* stream) {
+  DEV_GUARD(h);
+  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, sizeof(STree) + (size_t)(max_nodes > 0 ? max_nodes : 0) * sizeof(SNode), nullptr,
+                  0, prior_d, value_d, 0.0, 0.0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, visits_d, q_d, root_value_d};
+  const GumbelArgs gb = {gumbel_d, 0, 0, 0, c_visit, c_scale, action_d, policy_d};
+  const char* bad = gumbel_bad(n, gb, true);
+  if (!bad) bad = n > 0 && (!prior_d || !value_d) ? "prior and value are required"
+                  : n > 0 && (!visits_d || !q_d || !root_value_d) ? "visits, q and root_value are required"
+                  : search_bad(a, ws_bytes);
+  if (bad) { snprintf(h->err, sizeof h->err, "sb_search_end_gumbel: %s", bad); return -1; }
+  if (n == 0) return 0;
+  k_search_end_gumbel<<<grid_for(n, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a, gb);
+  LAUNCH_CHECK();
+  return 0;
+}
+int sb_ismcts_simulate_gumbel(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const uint8_t* det_d,
+                              const float* prior_d, const float* value_d, const float* gumbel_d, int sim, int num_simulations,
+                              int max_considered, double c_visit, double c_scale, uint8_t* leaf_states_d, int32_t* obs_d,
+                              uint32_t* masks_d, uint8_t* obs_err_d, uint8_t* to_move_d, uint8_t* leaf_kind_d, void* stream) {
+  DEV_GUARD(h);
+  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, ismcts_tree_bytes(max_nodes), det_d, 0, prior_d, value_d, 0.0, 0.0,
+                  leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d, nullptr, nullptr, nullptr};
+  const GumbelArgs gb = {gumbel_d, sim, num_simulations, max_considered, c_visit, c_scale, nullptr, nullptr};
+  const char* bad = gumbel_bad(n, gb, false);
+  if (!bad) bad = n > 0 && !det_d ? "worlds (det) are required" : n > 0 && (!prior_d || !value_d) ? "prior and value are required" : ismcts_bad(a, ws_bytes);
+  if (bad) { snprintf(h->err, sizeof h->err, "sb_ismcts_simulate_gumbel: %s", bad); return -1; }
+  if (n == 0) return 0;
+  k_ismcts_simulate_gumbel<<<grid_for(n, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a, gb, h->d_cards, h->d_wt);
+  LAUNCH_CHECK();
+  return 0;
+}
+int sb_ismcts_end_gumbel(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const float* prior_d, const float* value_d,
+                         const float* gumbel_d, double c_visit, double c_scale, int32_t* action_d, float* policy_d,
+                         int32_t* visits_d, double* q_d, double* root_value_d, void* stream) {
+  DEV_GUARD(h);
+  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, ismcts_tree_bytes(max_nodes), nullptr, 0, prior_d, value_d, 0.0, 0.0,
+                  nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, visits_d, q_d, root_value_d};
+  const GumbelArgs gb = {gumbel_d, 0, 0, 0, c_visit, c_scale, action_d, policy_d};
+  const char* bad = gumbel_bad(n, gb, true);
+  if (!bad) bad = n > 0 && (!prior_d || !value_d) ? "prior and value are required"
+                  : n > 0 && (!visits_d || !q_d || !root_value_d) ? "visits, q and root_value are required"
+                  : ismcts_bad(a, ws_bytes);
+  if (bad) { snprintf(h->err, sizeof h->err, "sb_ismcts_end_gumbel: %s", bad); return -1; }
+  if (n == 0) return 0;
+  k_ismcts_end_gumbel<<<grid_for(n, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a, gb);
+  LAUNCH_CHECK();
+  return 0;
 }
 // One launch, no handle scratch, atomics or host synchronisation (capturable in a CUDA graph).
 int sb_determinize(SbHandle* h, int n, const uint8_t* states_d, const uint8_t* observer_d, const uint64_t* keys_d, uint8_t* out_d,

@@ -208,14 +208,46 @@ __global__ void __launch_bounds__(TPB_GAME) k_search_simulate(const SearchArgs a
   s_emit_node(a, i, g, nodes[j], SEARCH_TERMINAL);
 }
 
-// back up the last pending leaf (the tree then holds nothing pending) and read out the root's edges
-__global__ void __launch_bounds__(TPB_GAME) k_search_end(const SearchArgs a) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= a.n) return;
-  STree& t = s_tree(a, i);
-  SNode* nodes = s_nodes(a, i);
-  s_backup(a, i, t, nodes);
-  t.kind = SEARCH_FULL;
+// one simulation's walk after the backup, as k_search_simulate's but checked (the Gumbel kernel): select(j, c) chooses the
+// action at the non-terminal node j and sets c to its child (0 = none), already checked against the node count; the
+// descent stops after max_nodes levels, and a selection without an action (act < 0) stops the tree, as sb_ismcts does.
+template <class Select>
+SBD_FI void s_walk(const SearchArgs& a, int i, G& g, STree& t, SNode* nodes, Select select) {
+  int j = 0;
+  #pragma unroll 1
+  for (int d = 0; !nodes[j].terminal; d++) {
+    int c;
+    const int act = d < a.max_nodes ? select(j, c) : -1;
+    if (act < 0) {  // only a workspace not written by sb_search_begin gets here: the tree stops
+      t.kind = SEARCH_FULL;
+      s_emit_node(a, i, g, nodes[0], SEARCH_FULL);
+      return;
+    }
+    if (!c) {  // expand: the child is the record sb_step(parent, act) produces
+      __align__(16) SbState s;
+      load_state(s, &nodes[j].rec);
+      unpack(g, s);
+      game_step(g, act);
+      end_of_step(g);
+      pack(g, s);
+      unpack(g, s);  // the working set as the next sb_* call would unpack it from the child's record
+      const int k = t.used++;
+      s_write_node(nodes[k], g, s, j, act, t.max_steps);
+      nodes[j].child[act] = k;
+      t.leaf = k;
+      t.kind = nodes[k].terminal ? SEARCH_TERMINAL : SEARCH_EVAL;
+      s_emit(a, i, g, nodes[k], t.kind);
+      return;
+    }
+    j = c;
+  }
+  t.leaf = j;  // an existing terminal node (or a terminal root): its game value is backed up again
+  t.kind = SEARCH_TERMINAL;
+  s_emit_node(a, i, g, nodes[j], SEARCH_TERMINAL);
+}
+
+// visits, q and root_value of tree i (sb_search_end)
+SBD_FI void s_read_out(const SearchArgs& a, int i, const SNode* nodes) {
   const SNode& root = nodes[0];
   const double sgn = s_sign(root.seat);
   #pragma unroll 1
@@ -226,4 +258,15 @@ __global__ void __launch_bounds__(TPB_GAME) k_search_end(const SearchArgs a) {
     a.q[(size_t)i * SB_N_ACTIONS + act] = na ? __ddiv_rn(__dmul_rn(sgn, nodes[c].W), (double)na) : __longlong_as_double(0x7FF8000000000000ll);
   }
   a.root_value[i] = __ddiv_rn(__dmul_rn(sgn, root.W), (double)root.N);
+}
+
+// back up the last pending leaf (the tree then holds nothing pending) and read out the root's edges
+__global__ void __launch_bounds__(TPB_GAME) k_search_end(const SearchArgs a) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= a.n) return;
+  STree& t = s_tree(a, i);
+  SNode* nodes = s_nodes(a, i);
+  s_backup(a, i, t, nodes);
+  t.kind = SEARCH_FULL;
+  s_read_out(a, i, nodes);
 }

@@ -311,7 +311,8 @@ class Engine:
         out = dict(out or {})
         shapes = {"states": ((n, STATE_BYTES), torch.uint8), "obs": ((n, 27, 5, 4), torch.int32), "masks": ((n, MASK_WORDS), torch.int32),
                   "obs_err": ((n,), torch.uint8), "to_move": ((n,), torch.uint8), "kind": ((n,), torch.uint8),
-                  "visits": ((n, N_ACTIONS), torch.int32), "q": ((n, N_ACTIONS), torch.float64), "root_value": ((n,), torch.float64)}
+                  "visits": ((n, N_ACTIONS), torch.int32), "q": ((n, N_ACTIONS), torch.float64), "root_value": ((n,), torch.float64),
+                  "action": ((n,), torch.int32), "policy": ((n, N_ACTIONS), torch.float32)}
         for k in names:
             shape, dtype = shapes[k]
             if k not in out:
@@ -406,6 +407,68 @@ class Engine:
         o = self._search_outputs(n, out, ("visits", "q", "root_value"))
         self._check(self.lib.sb_ismcts_end(self.h, n, int(max_nodes), self._p(ws), ws.numel(), self._p(prior), self._p(value),
                                            self._p(o["visits"]), self._p(o["q"]), self._p(o["root_value"]), self._stream()), "sb_ismcts_end")
+        return o
+
+    # ---- Gumbel search over both trees (sb_search_simulate_gumbel / sb_search_end_gumbel, sb_ismcts_*_gumbel)
+    def _gumbel(self, n, gumbel):
+        self._dev(gumbel, torch.float32)
+        assert tuple(gumbel.shape) == (n, N_ACTIONS), "gumbel is f32[n,156]"
+
+    def search_simulate_gumbel(self, ws, n, max_nodes, prior, value, gumbel, sim, num_simulations, max_considered=16,
+                               c_visit=50.0, c_scale=0.1, out=None):
+        """sb_search_simulate_gumbel: as search_simulate, selecting with the Gumbel rule (DESIGN.md 8.9): call sim = 1..S of
+        a search of num_simulations = S calls, gumbel f32[n,156] the search's Gumbel noise (the same for every call)."""
+        self._dev(ws, torch.uint8)
+        self._search_eval(n, prior, value)
+        self._gumbel(n, gumbel)
+        o = self._search_outputs(n, out, ("states", "obs", "masks", "obs_err", "to_move", "kind"))
+        self._check(self.lib.sb_search_simulate_gumbel(self.h, n, int(max_nodes), self._p(ws), ws.numel(), self._p(prior), self._p(value),
+                                                       self._p(gumbel), int(sim), int(num_simulations), int(max_considered), float(c_visit),
+                                                       float(c_scale), self._p(o["states"]), self._p(o["obs"]), self._p(o["masks"]),
+                                                       self._p(o["obs_err"]), self._p(o["to_move"]), self._p(o["kind"]), self._stream()),
+                    "sb_search_simulate_gumbel")
+        return o
+
+    def search_end_gumbel(self, ws, n, max_nodes, prior, value, gumbel, c_visit=50.0, c_scale=0.1, out=None):
+        """sb_search_end_gumbel: search_end's read-out plus action i32[n] (255 without root visits) and the improved policy
+        f32[n,156] (0 outside the legal set).  Returns the dict (action, policy, visits, q, root_value)."""
+        self._dev(ws, torch.uint8)
+        self._search_eval(n, prior, value)
+        self._gumbel(n, gumbel)
+        o = self._search_outputs(n, out, ("action", "policy", "visits", "q", "root_value"))
+        self._check(self.lib.sb_search_end_gumbel(self.h, n, int(max_nodes), self._p(ws), ws.numel(), self._p(prior), self._p(value),
+                                                  self._p(gumbel), float(c_visit), float(c_scale), self._p(o["action"]), self._p(o["policy"]),
+                                                  self._p(o["visits"]), self._p(o["q"]), self._p(o["root_value"]), self._stream()),
+                    "sb_search_end_gumbel")
+        return o
+
+    def ismcts_simulate_gumbel(self, ws, det, max_nodes, prior, value, gumbel, sim, num_simulations, max_considered=16,
+                               c_visit=50.0, c_scale=0.1, out=None):
+        """sb_ismcts_simulate_gumbel: as ismcts_simulate (this call's world det u8[n,512]), selecting with the Gumbel rule."""
+        self._dev(ws, torch.uint8)
+        det = self._worlds(det)
+        n = det.shape[0]
+        self._search_eval(n, prior, value)
+        self._gumbel(n, gumbel)
+        o = self._search_outputs(n, out, ("states", "obs", "masks", "obs_err", "to_move", "kind"))
+        self._check(self.lib.sb_ismcts_simulate_gumbel(self.h, n, int(max_nodes), self._p(ws), ws.numel(), self._p(det), self._p(prior),
+                                                       self._p(value), self._p(gumbel), int(sim), int(num_simulations), int(max_considered),
+                                                       float(c_visit), float(c_scale), self._p(o["states"]), self._p(o["obs"]),
+                                                       self._p(o["masks"]), self._p(o["obs_err"]), self._p(o["to_move"]), self._p(o["kind"]),
+                                                       self._stream()), "sb_ismcts_simulate_gumbel")
+        return o
+
+    def ismcts_end_gumbel(self, ws, n, max_nodes, prior, value, gumbel, c_visit=50.0, c_scale=0.1, out=None):
+        """sb_ismcts_end_gumbel: ismcts_end's read-out plus action i32[n] and the improved policy f32[n,156], by the root's
+        action ids (an id that repeats a lower id's card reads 0)."""
+        self._dev(ws, torch.uint8)
+        self._search_eval(n, prior, value)
+        self._gumbel(n, gumbel)
+        o = self._search_outputs(n, out, ("action", "policy", "visits", "q", "root_value"))
+        self._check(self.lib.sb_ismcts_end_gumbel(self.h, n, int(max_nodes), self._p(ws), ws.numel(), self._p(prior), self._p(value),
+                                                  self._p(gumbel), float(c_visit), float(c_scale), self._p(o["action"]), self._p(o["policy"]),
+                                                  self._p(o["visits"]), self._p(o["q"]), self._p(o["root_value"]), self._stream()),
+                    "sb_ismcts_end_gumbel")
         return o
 
     # ---- determinization for sampled search (sb_determinize)

@@ -22,6 +22,14 @@ separate trees that each believe their own world:
 
     mcts = InformationSetMCTS(env.n, num_simulations=64)
     visits, q, root_value = mcts.run(env.states, rollout_evaluator())
+
+GumbelMCTS and InformationSetGumbelMCTS run the same two trees with Gumbel MuZero's selection (sb_*_simulate_gumbel,
+DESIGN.md 8.9): Gumbel-top-k with sequential halving at the root instead of exploration noise, and an improved policy
+softmax(logits + sigma(completed q)) to train on, next to the action to play:
+
+    mcts = GumbelMCTS(env.n, num_simulations=16)
+    action, policy, visits, q, root_value = mcts.run(env.states, evaluate)
+    obs, masks, reward, done, info = env.step(action)
 """
 import math
 
@@ -243,3 +251,126 @@ class InformationSetMCTS:
             prior, value = evaluate(self.leaf, k)
         e.ismcts_end(self.ws, n, m, prior, value, out=self.out)
         return self.out["visits"], self.out["q"], self.out["root_value"]
+
+
+def gumbel_noise(n, seed):
+    """f32[n,156] of -log(-log u), u uniform on (0, 1) in steps of 2^-53, from numpy's default_rng(seed) (host)"""
+    u = np.random.default_rng(seed).integers(1, 1 << 53, size=(n, N_ACTIONS), dtype=np.int64).astype(np.float64) / float(1 << 53)
+    return (-np.log(-np.log(u))).astype(np.float32)
+
+
+def _gumbel_args(num_simulations, max_considered, c_visit, c_scale):
+    if not 1 <= int(num_simulations) <= 1 << 24:
+        raise ValueError("num_simulations must be 1..2^24")
+    if not 1 <= int(max_considered) <= N_ACTIONS:
+        raise ValueError("max_considered must be 1..156")
+    if not (math.isfinite(c_visit) and c_visit >= 0 and math.isfinite(c_scale) and c_scale >= 0):
+        raise ValueError("c_visit and c_scale must be finite and >= 0")
+
+
+class GumbelMCTS:
+    """Gumbel MuZero search over BatchedMCTS's perfect-information trees: n trees of num_simulations + 1 nodes.
+
+    run(roots, evaluate, gumbel=None) -> (action i32[n], policy f32[n,156], visits i32[n,156], q f64[n,156], root_value
+    f64[n]).  action is the id to play (the root id with the most visits and the best g + logit + sigma among those; 255
+    when the root has no visit, e.g. a finished game) and feeds StormboundVecEnv.step directly; policy is the improved
+    policy softmax(logit + sigma(completed q)) over the legal set, the training target; visits, q and root_value are
+    BatchedMCTS's.  evaluate(leaf, k) is BatchedMCTS's contract (rollout_evaluator works unchanged); the root needs no noise.
+    gumbel: device f32[n,156], the Gumbel noise of the search.  When None it is -log(-log u) drawn on the host from `seed`
+    and a per-object call counter (next_seed mix) and copied to the device: reproducible but not capture-safe.  With caller
+    noise (and a capture-safe evaluator) a run synchronises nothing with the host and can be captured in a
+    torch.cuda.CUDAGraph.  A run is exactly num_simulations + 2 library launches.  The returned tensors are buffers of this
+    object, overwritten by the next run.
+    """
+
+    def __init__(self, n, num_simulations, max_considered=16, c_visit=50.0, c_scale=0.1, max_steps=400, seed=0, engine=None,
+                 device=None):
+        _gumbel_args(num_simulations, max_considered, c_visit, c_scale)
+        self.engine = e = engine if engine is not None else get_engine(device)
+        self.n, self.num_simulations, self.max_considered = int(n), int(num_simulations), int(max_considered)
+        self.c_visit, self.c_scale, self.max_steps = float(c_visit), float(c_scale), int(max_steps)
+        self.max_nodes = self.num_simulations + 1
+        self.seed, self.calls = int(seed), 0
+        self.ws = torch.empty(e.search_workspace_bytes(self.n, self.max_nodes), dtype=torch.uint8, device=e.device)
+        self.gumbel = torch.empty((self.n, N_ACTIONS), dtype=torch.float32, device=e.device)
+        self.leaf = e._search_outputs(self.n, None, LEAF_KEYS)
+        self.out = e._search_outputs(self.n, None, ("action", "policy", "visits", "q", "root_value"))
+
+    def default_gumbel(self):
+        """the noise of the next run without caller noise: gumbel_noise(n, next_seed(next_seed(seed) + call index))"""
+        base = next_seed(next_seed(self.seed) + self.calls)
+        self.calls += 1
+        return gumbel_noise(self.n, base)
+
+    def _noise(self, gumbel):
+        if gumbel is None:
+            self.gumbel.copy_(torch.from_numpy(self.default_gumbel()))
+            return self.gumbel
+        assert tuple(gumbel.shape) == (self.n, N_ACTIONS), "gumbel is f32[n, 156] with n = %d" % self.n
+        return gumbel
+
+    def _result(self):
+        o = self.out
+        return o["action"], o["policy"], o["visits"], o["q"], o["root_value"]
+
+    def run(self, roots, evaluate, gumbel=None):
+        e, n, m, S = self.engine, self.n, self.max_nodes, self.num_simulations
+        assert roots.shape[0] == n, "roots are u8[n, 512] with n = %d" % n
+        g = self._noise(gumbel)
+        e.search_begin(self.ws, roots, m, self.max_steps, out=self.leaf)
+        prior, value = evaluate(self.leaf, 0)
+        for k in range(1, S + 1):
+            e.search_simulate_gumbel(self.ws, n, m, prior, value, g, k, S, self.max_considered, self.c_visit, self.c_scale, out=self.leaf)
+            prior, value = evaluate(self.leaf, k)
+        e.search_end_gumbel(self.ws, n, m, prior, value, g, self.c_visit, self.c_scale, out=self.out)
+        return self._result()
+
+
+class InformationSetGumbelMCTS(GumbelMCTS):
+    """Gumbel MuZero search over InformationSetMCTS's information-set trees: one tree per root over what the player to move
+    sees, every call walking it through a fresh determinization.
+
+    run(roots, evaluate, keys=None, gumbel=None) -> (action, policy, visits, q, root_value) as GumbelMCTS, by the root's
+    action ids (an id that plays the same card as a lower legal id reads 0 visits, NaN q and 0 policy).  keys are
+    InformationSetMCTS's (device i64[(S+1)*n], simulation-major; None: from `seed` and a call counter on the host), gumbel
+    GumbelMCTS's.  With caller keys and noise (and a capture-safe evaluator) a run can be captured in a torch.cuda.CUDAGraph.
+    A run is exactly 2 * num_simulations + 3 library launches (S + 1 sb_determinize, begin, S simulate, end).
+    """
+
+    def __init__(self, n, num_simulations, max_considered=16, c_visit=50.0, c_scale=0.1, max_steps=400, seed=0, engine=None,
+                 device=None):
+        _gumbel_args(num_simulations, max_considered, c_visit, c_scale)
+        self.engine = e = engine if engine is not None else get_engine(device)
+        self.n, self.num_simulations, self.max_considered = int(n), int(num_simulations), int(max_considered)
+        self.c_visit, self.c_scale, self.max_steps = float(c_visit), float(c_scale), int(max_steps)
+        self.max_nodes = self.num_simulations + 1
+        self.seed, self.calls, self.key_calls = int(seed), 0, 0
+        self.ws = torch.empty(e.ismcts_workspace_bytes(self.n, self.max_nodes), dtype=torch.uint8, device=e.device)
+        self.world = torch.empty((self.n, STATE_BYTES), dtype=torch.uint8, device=e.device)
+        self.gumbel = torch.empty((self.n, N_ACTIONS), dtype=torch.float32, device=e.device)
+        self.leaf = e._search_outputs(self.n, None, LEAF_KEYS)
+        self.out = e._search_outputs(self.n, None, ("action", "policy", "visits", "q", "root_value"))
+
+    def default_keys(self):
+        """InformationSetMCTS.default_keys, with a call counter of its own"""
+        base = next_seed(next_seed(self.seed) + self.key_calls)
+        self.key_calls += 1
+        return next_seed_array(np.arange(self.max_nodes * self.n, dtype=np.uint64) + np.uint64(base))
+
+    def run(self, roots, evaluate, keys=None, gumbel=None):
+        e, n, m, S = self.engine, self.n, self.max_nodes, self.num_simulations
+        assert roots.shape == (n, STATE_BYTES), "roots are u8[n, 512] with n = %d" % n
+        if keys is None:
+            keys = torch.from_numpy(self.default_keys()).to(e.device)
+        assert keys.shape == (m * n,), "keys are i64[(S + 1) * n] with (S + 1) * n = %d" % (m * n)
+        g = self._noise(gumbel)
+        e.determinize(roots, keys[:n], out=self.world)
+        e.ismcts_begin(self.ws, self.world, m, self.max_steps, out=self.leaf)
+        prior, value = evaluate(self.leaf, 0)
+        for k in range(1, S + 1):
+            e.determinize(roots, keys[k * n:(k + 1) * n], out=self.world)
+            e.ismcts_simulate_gumbel(self.ws, self.world, m, prior, value, g, k, S, self.max_considered, self.c_visit, self.c_scale,
+                                     out=self.leaf)
+            prior, value = evaluate(self.leaf, k)
+        e.ismcts_end_gumbel(self.ws, n, m, prior, value, g, self.c_visit, self.c_scale, out=self.out)
+        return self._result()
