@@ -309,7 +309,9 @@ int sb_accumulate_fitness(SbHandle *h, int n, const int8_t *result_d, const int3
  * games_per_pair consecutive games.  mode 0 = the reference's round robin: ordered pairs (i, j), i < n_ind, j < n_total,
  * j != i (rows n_ind.. are the hall of fame); mode 1 = every individual as FIRST against each of the n_total - n_ind fixed
  * opponents; mode 2 = (i, i), for a SECOND seat played by expert_action.  seeds are the partition-invariant hash of
- * (base_seed, generation, i, j, replicate) (the reference seeds every game from OS entropy, SURVEY Q16). */
+ * (base_seed, generation, i, j, replicate) (the reference seeds every game from OS entropy, SURVEY Q16).  A bad schedule
+ * returns -1 (sb_last_error) and launches nothing: mode outside 0..2, n_ind < 1, games_per_pair < 1, n_total < n_ind, a round
+ * robin of fewer than 2 rows, or versus without an opponent row (n_total == n_ind).  n <= 0 is a no-op. */
 int sb_eval_schedule(SbHandle *h, int mode, int n_ind, int n_total, int games_per_pair, uint64_t base_seed, uint32_t generation,
                      int64_t game_lo, int n, int32_t *idx_first_d, int32_t *idx_second_d, uint64_t *seeds_d, void *stream);
 
@@ -317,7 +319,8 @@ int sb_eval_schedule(SbHandle *h, int mode, int n_ind, int n_total, int games_pe
  * entirely on the device: sb_eval_schedule -> sb_reset (decks_d u8[2,n_deck] shared by all games, factions_d u8[2]) ->
  * sb_rollout_heuristic over weights_d f64[n_total,10] -> sb_accumulate_fitness into counts_d i32[n_ind,3] (+=) and
  * sb_count_aborted into aborted_d i32[2] (+=, nullable), chunk_games at a time (<= 0: 262,144) in a workspace owned by the
- * handle.  Asynchronous on `stream`; nothing is copied to the host. */
+ * handle.  Asynchronous on `stream`; nothing is copied to the host.  A bad schedule returns -1 as sb_eval_schedule does,
+ * before the first launch. */
 int sb_eval_population(SbHandle *h, int mode, int n_ind, int n_total, int games_per_pair, uint64_t base_seed, uint32_t generation,
                        int64_t game_lo, int64_t game_hi, const double *weights_d, const uint8_t *decks_d, int n_deck,
                        const uint8_t *factions_d, int max_steps, int chunk_games, int32_t *counts_d, int32_t *aborted_d, void *stream);

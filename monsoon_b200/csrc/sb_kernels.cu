@@ -1829,7 +1829,7 @@ int sb_eval_schedule(SbHandle* h, int mode, int n_ind, int n_total, int games_pe
   if (mode < 0 || mode > 2 || n_ind <= 0 || games_per_pair <= 0 || n_total < n_ind || (mode == 0 && n_total < 2) || (mode == 1 && n_total == n_ind)) {
     snprintf(h->err, sizeof(h->err), "sb_eval_schedule: bad schedule (mode %d, %d individuals, %d rows, %d games per pairing)", mode, n_ind,
              n_total, games_per_pair);
-    return 1;
+    return -1;
   }
   k_eval_schedule<<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(mode, n_ind, n_total, games_per_pair, (unsigned long long)base_seed, generation,
                                                                     (long long)game_lo, n, idx_first_d, idx_second_d, (unsigned long long*)seeds_d);

@@ -517,14 +517,19 @@ class Engine:
         return i1, i2, seeds
 
     def eval_population(self, mode, n_ind, weights, games_per_pair, base_seed, generation, game_lo, game_hi, max_steps=400,
-                        counts=None, aborted=None, chunk_games=0):
-        """sb_eval_population over the default decks: counts i32[n_ind,3] += {wins, draws, losses}, aborted i32[2] += ...; asynchronous."""
+                        counts=None, aborted=None, chunk_games=0, decks=None, factions=None):
+        """sb_eval_population: counts i32[n_ind,3] += {wins, draws, losses}, aborted i32[2] += ...; asynchronous.  Every game is
+        dealt the same deck pair: decks u8[2, n_deck] with factions u8[2], or the default decks when decks is None."""
         weights = self._dev(weights, torch.float64)
         assert weights.dim() == 2 and weights.shape[1] == 10 and weights.shape[0] >= n_ind, "weight tables are f64[P, 10] (SB_N_FEATURES)"
-        if self._default_decks is None:
-            self._default_decks = (torch.tensor([deck_indices(d) for d in DEFAULT_DECKS], dtype=torch.uint8, device=self.device),
-                                   torch.tensor(DEFAULT_FACTIONS, dtype=torch.uint8, device=self.device))
-        decks, factions = self._default_decks
+        if decks is None:
+            assert factions is None, "factions go with decks"
+            if self._default_decks is None:
+                self._default_decks = (torch.tensor([deck_indices(d) for d in DEFAULT_DECKS], dtype=torch.uint8, device=self.device),
+                                       torch.tensor(DEFAULT_FACTIONS, dtype=torch.uint8, device=self.device))
+            decks, factions = self._default_decks
+        decks, factions = self._dev(decks, torch.uint8), self._dev(factions, torch.uint8)
+        assert decks.dim() == 2 and decks.shape[0] == 2 and tuple(factions.shape) == (2,), "one deck pair u8[2, n_deck], factions u8[2]"
         counts = counts if counts is not None else torch.zeros((n_ind, 3), dtype=torch.int32, device=self.device)
         aborted = aborted if aborted is not None else torch.zeros(2, dtype=torch.int32, device=self.device)
         self._dev(counts, torch.int32)

@@ -104,8 +104,10 @@ def test_fitness_evaluator_with_deck_schedule(engine, oracle):
                     st = oracle.new_game(seed, d[0], d[1], fac[0], fac[1])
                     r, _ = oracle.play_heuristic(st, pop[i].weights, pop[j].weights, 400)
                     flagged += r == -2
-                    want[i] += 1.0 if r == 0 else 0.5 if r == -1 else 0.0
+                    want[i] += 1.0 if r == 0 else 0.5 if r < 0 else 0.0  # an aborted game (-2) is a draw, like a timeout
         assert np.allclose(fit, want / (2 * 2)), (generation, fit, want, flagged)
+        # none of these games aborts, so the draw scoring of -2 is not exercised here (tests/test_gpu_fitness.py does)
+        assert flagged == 0 and ev.last_aborted == (0, 0), (generation, flagged, ev.last_aborted)
 
 
 def test_deck_generation_matches_oracle_at_scale(engine, oracle):
