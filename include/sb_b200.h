@@ -283,6 +283,40 @@ int sb_ismcts_end_gumbel(SbHandle *h, int n, int max_nodes, void *ws_d, size_t w
                          const float *value_d, const float *gumbel_d, double c_visit, double c_scale, int32_t *action_d,
                          float *policy_d, int32_t *visits_d, double *q_d, double *root_value_d, void *stream);
 
+/* Tree reuse between moves for both PUCT searches, ABI 5's additive entry points (DESIGN.md 8.10).  An advance is the
+ * matching begin (sb_search_begin on roots_d / sb_ismcts_begin on world 0 det_d, same leaf outputs and kinds), except that
+ * it may carry each tree's subtree below the new root over from a finished search:
+ *   sb_search_advance(ws_src -> ws_dst, roots) -> evaluate -> (sb_search_simulate -> evaluate) x S -> sb_search_end
+ *   sb_ismcts_advance(ws_src -> ws_dst, world 0, played) -> evaluate -> (sb_ismcts_simulate(world k) -> evaluate) x S -> ...
+ * ws_src and ws_dst are two non-overlapping workspaces of this n and max_nodes (ws_bytes is checked for both); ws_src is
+ * consumed: its contents afterwards are unspecified, except that each of its trees then holds no node, so advancing from
+ * it again (e.g. replaying a captured advance) starts every tree fresh.  ws_dst receives, for each tree g, either exactly what the begin
+ * writes for this call's root (kept_d[g] = 0) or the kept subtree of ws_src's tree g (kept_d[g] = its node count >= 1):
+ * the matched node j and its descendants in creation order (increasing node index), the first `keep` of them, j as node 0
+ * with parent -1.  Kept nodes keep N, W, prior, mask, record or code, seat and terminal data; a child link to a node not
+ * kept becomes none (8.6: 0 in child[], 8.8: left out of the sibling list, whose order is otherwise kept).  The new root is
+ * the pending leaf (kind 0, or 1 when terminal); the next simulate or end backs it up as usual, so the caller's prior
+ * replaces the stored one and N / W gain that evaluation.  The ancestors' N / W still count the visits of dropped nodes.
+ * A tree is reused only when ws_src's header says finished (by _end, or stopped full: nothing pending) with this call's
+ * max_steps, and the rule finds j:
+ *   sb_search_advance: j = the lowest-index node whose 512-byte record equals roots_d[g] byte for byte;
+ *   sb_ismcts_advance: j = the child of the source root with the code ws_src's header stores for root action id played_d[g]
+ *     (0..155, not ISM_NONE), when det_d[g] is not over and its seat to move is both j's and the source root's (one
+ *     observer: a PASS or a turn handed over starts fresh).  The caller promises that the new root
+ *     is the record sb_step(old root, played) gives; -1 (or any id outside 0..155) starts the tree fresh.
+ * Otherwise the tree starts fresh.  Gumbel simulate / end calls on an advanced workspace are unsupported.  Bad arguments
+ * return -1 (sb_last_error) and launch nothing: those of the begin, keep outside 1..max_nodes, a NULL or misaligned ws_src,
+ * ws_src == ws_dst or overlapping, a NULL played_d (sb_ismcts_advance); kept_d and the leaf outputs are nullable; n = 0 is a
+ * no-op.  One call = one kernel launch (one warp per tree for the copy), without handle scratch, atomics or host
+ * synchronisation (capturable in a CUDA graph).  Node indices read from ws_src are bounds-checked against its node count. */
+int sb_search_advance(SbHandle *h, int n, int max_nodes, void *ws_src_d, void *ws_dst_d, size_t ws_bytes,
+                      const uint8_t *roots_d, int max_steps, int keep, int32_t *kept_d, uint8_t *leaf_states_d, int32_t *obs_d,
+                      uint32_t *masks_d, uint8_t *obs_err_d, uint8_t *to_move_d, uint8_t *leaf_kind_d, void *stream);
+int sb_ismcts_advance(SbHandle *h, int n, int max_nodes, void *ws_src_d, void *ws_dst_d, size_t ws_bytes,
+                      const uint8_t *det_d, const int32_t *played_d, int max_steps, int keep, int32_t *kept_d,
+                      uint8_t *leaf_states_d, int32_t *obs_d, uint32_t *masks_d, uint8_t *obs_err_d, uint8_t *to_move_d,
+                      uint8_t *leaf_kind_d, void *stream);
+
 /* Determinization for sampled (PIMC) search:out_d[g] = states_d[g] with everything observer o cannot see resampled and
  * everything o sees kept byte for byte (sb_observe / sb_legal_mask / sb_features of o's view are unchanged).
  * observer_d u8[n] is nullable: NULL = each record's own local_order (the seat sb_observe and sb_legal_mask show); a

@@ -182,6 +182,36 @@ SBD_FI int ism_select(const SearchArgs& a, const INode* nodes, int lim, const IN
   return best;
 }
 
+// the header of tree i (root codes from the world's record s, unpacked to g) and the leaf outputs of its root:
+// sb_ismcts_begin's tree (kept = 0: node 0 is written fresh), or one whose first `kept` nodes sb_ismcts_advance carried
+// over (node 0 is already the root, and the world is not over).  m receives the root's legal mask; it is the kernel's own
+// array so that the kernel's frame keeps the layout it had before this function was factored out of k_ismcts_begin.
+SBD_FI void ism_start(const SearchArgs& a, int i, const G& g, const SbState& s, u32* m, int kept) {
+  ITree& t = ism_tree(a, i);
+  INode& root = ism_nodes(a, i)[0];
+  legal_mask(g, m);
+  const Ply& p = g.pl[g.local_order];
+  #pragma unroll 1
+  for (int act = 0; act < SB_N_ACTIONS; act++) t.root_code[act] = ism_bit(m, act) && ism_rep(p, m, act) ? ism_code(p, act) : ISM_NONE;
+  if (!kept) {
+    root.W = 0.0;
+    root.parent = -1;
+    root.child = -1;
+    root.sibling = -1;
+    root.code = ISM_NONE;
+    root.N = 0;
+    root.seat = g.player_sign == 1 ? 0 : 1;
+  }
+  const bool over = env_over(g, a.max_steps);
+  if (!kept && over) ism_zero_prior(root);
+  t.used = kept ? kept : 1;
+  t.leaf = 0;
+  t.kind = over ? SEARCH_TERMINAL : SEARCH_EVAL;
+  t.max_steps = a.max_steps;
+  t.tval = over ? ism_value(g) : 0;
+  ism_emit(a, i, g, s, m, t.kind);
+}
+
 __global__ void __launch_bounds__(TPB_GAME) k_ismcts_begin(const SearchArgs a, const DCard* cards, const double* wt) {
   __shared__ DCard s_cards[SBC_COUNT];
   stage_cards(s_cards, cards);
@@ -192,28 +222,8 @@ __global__ void __launch_bounds__(TPB_GAME) k_ismcts_begin(const SearchArgs a, c
   __align__(16) SbState s;
   load_state(s, a.roots + (size_t)i * SB_STATE_BYTES);
   unpack(g, s);
-  ITree& t = ism_tree(a, i);
-  INode& root = ism_nodes(a, i)[0];
   u32 m[SB_MASK_WORDS];
-  legal_mask(g, m);
-  const Ply& p = g.pl[g.local_order];
-  #pragma unroll 1
-  for (int act = 0; act < SB_N_ACTIONS; act++) t.root_code[act] = ism_bit(m, act) && ism_rep(p, m, act) ? ism_code(p, act) : ISM_NONE;
-  root.W = 0.0;
-  root.parent = -1;
-  root.child = -1;
-  root.sibling = -1;
-  root.code = ISM_NONE;
-  root.N = 0;
-  root.seat = g.player_sign == 1 ? 0 : 1;
-  const bool over = env_over(g, a.max_steps);
-  if (over) ism_zero_prior(root);
-  t.used = 1;
-  t.leaf = 0;
-  t.kind = over ? SEARCH_TERMINAL : SEARCH_EVAL;
-  t.max_steps = a.max_steps;
-  t.tval = over ? ism_value(g) : 0;
-  ism_emit(a, i, g, s, m, t.kind);
+  ism_start(a, i, g, s, m, 0);
 }
 
 // one simulation's walk after the backup, in this call's world (record s, working set g, legal mask m at the root):

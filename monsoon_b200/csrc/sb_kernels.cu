@@ -18,6 +18,7 @@
 //   k_search_*         batched PUCT tree search, one tree per thread, one launch per simulation (sb_search.cuh)
 //   k_ismcts_*         information-set tree search over caller-supplied worlds, one tree per thread (sb_ismcts.cuh)
 //   k_*_gumbel         Gumbel selection and read-out for both tree searches (sb_gumbel.cuh)
+//   k_*_advance        tree reuse between moves for both PUCT searches, one warp per tree for the copy (sb_reuse.cuh)
 //   k_determinize      one record per warp: resample what the observer cannot see (sb_determinize.cuh)
 //   k_accumulate_fitness win/draw/loss counts per individual (evo/fitness.py:95,160-166)
 //   k_es_*             evolution-strategy operators on the resident population (sb_es.cuh; evo/weights.py, evo/population.py)
@@ -1032,6 +1033,9 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32) k_env_step_heur(const EnvA
 // ---------------------------------------------------------------- Gumbel search for both trees (sb_*_gumbel)
 #include "sb_gumbel.cuh"
 
+// ---------------------------------------------------------------- tree reuse between moves (sb_*_advance)
+#include "sb_reuse.cuh"
+
 // ---------------------------------------------------------------- determinization for sampled search (sb_determinize)
 #include "sb_determinize.cuh"
 
@@ -1789,6 +1793,54 @@ int sb_ismcts_end_gumbel(SbHandle* h, int n, int max_nodes, void* ws_d, size_t w
   if (bad) { snprintf(h->err, sizeof h->err, "sb_ismcts_end_gumbel: %s", bad); return -1; }
   if (n == 0) return 0;
   k_ismcts_end_gumbel<<<grid_for(n, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a, gb);
+  LAUNCH_CHECK();
+  return 0;
+}
+// The advance entries: the checks of the matching begin plus the second workspace and keep; one launch each, no handle
+// scratch, atomics or host synchronisation.
+static const char* reuse_bad(const SearchArgs& a, const ReuseArgs& r) {  // after search_bad / ismcts_bad
+  const size_t span = (size_t)(a.n > 0 ? a.n : 0) * a.tree_bytes;
+  const uintptr_t s = (uintptr_t)r.src, d = (uintptr_t)a.ws;
+  return r.keep < 1 || r.keep > a.max_nodes ? "keep must be 1..max_nodes"
+         : a.n > 0 && !r.src ? "source workspace is NULL"
+         : ((uintptr_t)r.src & 15) ? "source workspace must be 16-byte aligned"
+         : a.n > 0 && r.src == a.ws ? "ws_src and ws_dst must be two workspaces"
+         : a.n > 0 && s < d + span && d < s + span ? "ws_src and ws_dst overlap"
+         : nullptr;
+}
+int sb_search_advance(SbHandle* h, int n, int max_nodes, void* ws_src_d, void* ws_dst_d, size_t ws_bytes, const uint8_t* roots_d,
+                      int max_steps, int keep, int32_t* kept_d, uint8_t* leaf_states_d, int32_t* obs_d, uint32_t* masks_d,
+                      uint8_t* obs_err_d, uint8_t* to_move_d, uint8_t* leaf_kind_d, void* stream) {
+  DEV_GUARD(h);
+  SearchArgs a = {n, max_nodes, (unsigned char*)ws_dst_d, sizeof(STree) + (size_t)(max_nodes > 0 ? max_nodes : 0) * sizeof(SNode), roots_d,
+                  max_steps, nullptr, nullptr, 0.0, 0.0, leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d,
+                  nullptr, nullptr, nullptr};
+  const ReuseArgs r = {(unsigned char*)ws_src_d, keep, kept_d, nullptr};
+  const char* bad = max_steps < 1 || max_steps > 65535 ? "max_steps must be 1..65535"
+                    : n > 0 && !roots_d ? "roots are required"
+                    : search_bad(a, ws_bytes);
+  if (!bad) bad = reuse_bad(a, r);
+  if (bad) { snprintf(h->err, sizeof h->err, "sb_search_advance: %s", bad); return -1; }
+  if (n == 0) return 0;
+  k_search_advance<<<grid_for(n, TPB_GAME), RS_THREADS, 0, (cudaStream_t)stream>>>(a, r, h->d_cards, h->d_wt);
+  LAUNCH_CHECK();
+  return 0;
+}
+int sb_ismcts_advance(SbHandle* h, int n, int max_nodes, void* ws_src_d, void* ws_dst_d, size_t ws_bytes, const uint8_t* det_d,
+                      const int32_t* played_d, int max_steps, int keep, int32_t* kept_d, uint8_t* leaf_states_d, int32_t* obs_d,
+                      uint32_t* masks_d, uint8_t* obs_err_d, uint8_t* to_move_d, uint8_t* leaf_kind_d, void* stream) {
+  DEV_GUARD(h);
+  SearchArgs a = {n, max_nodes, (unsigned char*)ws_dst_d, ismcts_tree_bytes(max_nodes), det_d, max_steps, nullptr, nullptr, 0.0, 0.0,
+                  leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d, nullptr, nullptr, nullptr};
+  const ReuseArgs r = {(unsigned char*)ws_src_d, keep, kept_d, played_d};
+  const char* bad = max_steps < 1 || max_steps > 65535 ? "max_steps must be 1..65535"
+                    : n > 0 && !det_d ? "worlds (det) are required"
+                    : n > 0 && !played_d ? "played is required"
+                    : ismcts_bad(a, ws_bytes);
+  if (!bad) bad = reuse_bad(a, r);
+  if (bad) { snprintf(h->err, sizeof h->err, "sb_ismcts_advance: %s", bad); return -1; }
+  if (n == 0) return 0;
+  k_ismcts_advance<<<grid_for(n, TPB_GAME), RS_THREADS, 0, (cudaStream_t)stream>>>(a, r, h->d_cards, h->d_wt);
   LAUNCH_CHECK();
   return 0;
 }

@@ -145,6 +145,19 @@ SBD_FI int s_select(const SearchArgs& a, const SNode* nodes, const SNode& nd) {
   return best;
 }
 
+// the header of tree i and the leaf outputs of its root, whose record s unpacks to g: sb_search_begin's tree (kept = 0:
+// node 0 is written from s), or one whose first `kept` nodes sb_search_advance carried over (node 0 already holds s)
+SBD_FI void s_start(const SearchArgs& a, int i, const G& g, const SbState& s, int kept) {
+  STree& t = s_tree(a, i);
+  SNode* nodes = s_nodes(a, i);
+  if (!kept) s_write_node(nodes[0], g, s, -1, SB_ACTION_PASS, a.max_steps);
+  t.used = kept ? kept : 1;
+  t.leaf = 0;
+  t.kind = nodes[0].terminal ? SEARCH_TERMINAL : SEARCH_EVAL;
+  t.max_steps = a.max_steps;
+  s_emit(a, i, g, nodes[0], t.kind);
+}
+
 __global__ void __launch_bounds__(TPB_GAME) k_search_begin(const SearchArgs a, const DCard* cards, const double* wt) {
   __shared__ DCard s_cards[SBC_COUNT];
   stage_cards(s_cards, cards);
@@ -155,14 +168,7 @@ __global__ void __launch_bounds__(TPB_GAME) k_search_begin(const SearchArgs a, c
   __align__(16) SbState s;
   load_state(s, a.roots + (size_t)i * SB_STATE_BYTES);
   unpack(g, s);
-  STree& t = s_tree(a, i);
-  SNode* nodes = s_nodes(a, i);
-  s_write_node(nodes[0], g, s, -1, SB_ACTION_PASS, a.max_steps);
-  t.used = 1;
-  t.leaf = 0;
-  t.kind = nodes[0].terminal ? SEARCH_TERMINAL : SEARCH_EVAL;
-  t.max_steps = a.max_steps;
-  s_emit(a, i, g, nodes[0], t.kind);
+  s_start(a, i, g, s, 0);
 }
 
 __global__ void __launch_bounds__(TPB_GAME) k_search_simulate(const SearchArgs a, const DCard* cards, const double* wt) {

@@ -312,7 +312,7 @@ class Engine:
         shapes = {"states": ((n, STATE_BYTES), torch.uint8), "obs": ((n, 27, 5, 4), torch.int32), "masks": ((n, MASK_WORDS), torch.int32),
                   "obs_err": ((n,), torch.uint8), "to_move": ((n,), torch.uint8), "kind": ((n,), torch.uint8),
                   "visits": ((n, N_ACTIONS), torch.int32), "q": ((n, N_ACTIONS), torch.float64), "root_value": ((n,), torch.float64),
-                  "action": ((n,), torch.int32), "policy": ((n, N_ACTIONS), torch.float32)}
+                  "action": ((n,), torch.int32), "policy": ((n, N_ACTIONS), torch.float32), "kept": ((n,), torch.int32)}
         for k in names:
             shape, dtype = shapes[k]
             if k not in out:
@@ -469,6 +469,44 @@ class Engine:
                                                   self._p(gumbel), float(c_visit), float(c_scale), self._p(o["action"]), self._p(o["policy"]),
                                                   self._p(o["visits"]), self._p(o["q"]), self._p(o["root_value"]), self._stream()),
                     "sb_ismcts_end_gumbel")
+        return o
+
+    # ---- tree reuse between moves for both PUCT searches (sb_search_advance / sb_ismcts_advance)
+    def _two_workspaces(self, ws_src, ws_dst):
+        self._dev(ws_src, torch.uint8)
+        self._dev(ws_dst, torch.uint8)
+        assert ws_src.numel() == ws_dst.numel(), "ws_src and ws_dst are two workspaces of one size"
+        return ws_dst.numel()
+
+    def search_advance(self, ws_src, ws_dst, roots, max_nodes, keep, max_steps=400, out=None):
+        """sb_search_advance: search_begin on roots u8[n,512] into ws_dst, carrying over from the finished search in ws_src
+        (consumed) each tree's subtree below the lowest node whose record is the new root, at most `keep` nodes in creation
+        order.  Returns the leaf dict of search_begin plus kept i32[n] (nodes kept, 0 for a fresh root)."""
+        nb = self._two_workspaces(ws_src, ws_dst)
+        roots = self._dev(roots, torch.uint8)
+        assert roots.dim() == 2 and roots.shape[1] == STATE_BYTES, "roots are u8[n, 512]"
+        n = roots.shape[0]
+        o = self._search_outputs(n, out, ("states", "obs", "masks", "obs_err", "to_move", "kind", "kept"))
+        self._check(self.lib.sb_search_advance(self.h, n, int(max_nodes), self._p(ws_src), self._p(ws_dst), nb, self._p(roots),
+                                               int(max_steps), int(keep), self._p(o["kept"]), self._p(o["states"]), self._p(o["obs"]),
+                                               self._p(o["masks"]), self._p(o["obs_err"]), self._p(o["to_move"]), self._p(o["kind"]),
+                                               self._stream()), "sb_search_advance")
+        return o
+
+    def ismcts_advance(self, ws_src, ws_dst, det, played, max_nodes, keep, max_steps=400, out=None):
+        """sb_ismcts_advance: ismcts_begin on world 0 det u8[n,512] into ws_dst, carrying over from the finished search in
+        ws_src (consumed) each tree's subtree below the root child of the action id played i32[n] (-1: none) when det's seat
+        to move is that child's, at most `keep` nodes.  Returns the leaf dict of ismcts_begin plus kept i32[n]."""
+        nb = self._two_workspaces(ws_src, ws_dst)
+        det = self._worlds(det)
+        n = det.shape[0]
+        self._dev(played, torch.int32)
+        assert tuple(played.shape) == (n,), "played is i32[n]"
+        o = self._search_outputs(n, out, ("states", "obs", "masks", "obs_err", "to_move", "kind", "kept"))
+        self._check(self.lib.sb_ismcts_advance(self.h, n, int(max_nodes), self._p(ws_src), self._p(ws_dst), nb, self._p(det),
+                                               self._p(played), int(max_steps), int(keep), self._p(o["kept"]), self._p(o["states"]),
+                                               self._p(o["obs"]), self._p(o["masks"]), self._p(o["obs_err"]), self._p(o["to_move"]),
+                                               self._p(o["kind"]), self._stream()), "sb_ismcts_advance")
         return o
 
     # ---- determinization for sampled search (sb_determinize)

@@ -23,6 +23,15 @@ separate trees that each believe their own world:
     mcts = InformationSetMCTS(env.n, num_simulations=64)
     visits, q, root_value = mcts.run(env.states, rollout_evaluator())
 
+With reuse_nodes = R > 0, BatchedMCTS and InformationSetMCTS keep the subtree of the position reached between moves
+(sb_search_advance / sb_ismcts_advance, DESIGN.md 8.10): a search of S simulations then starts from the visits the last
+search already spent below the new root, up to R + 1 nodes of it:
+
+    mcts = BatchedMCTS(env.n, num_simulations=64, reuse_nodes=64)
+    for move in range(moves):
+        visits, q, root_value = mcts.run(env.states, evaluate)   # mcts.kept: nodes carried over per tree
+        obs, masks, reward, done, info = env.step(select_actions(visits))
+
 GumbelMCTS and InformationSetGumbelMCTS run the same two trees with Gumbel MuZero's selection (sb_*_simulate_gumbel,
 DESIGN.md 8.9): Gumbel-top-k with sequential halving at the root instead of exploration noise, and an improved policy
 softmax(logits + sigma(completed q)) to train on, next to the action to play:
@@ -113,25 +122,52 @@ class BatchedMCTS:
     the value from the point of view of to_move.  A run is exactly num_simulations + 2 library launches; with an evaluator
     that only uses torch it synchronises nothing with the host and can be captured in a torch.cuda.CUDAGraph.  The returned
     tensors are buffers of this object, overwritten by the next run.
+
+    reuse_nodes = R > 0 keeps trees between runs: the trees have num_simulations + 1 + R nodes (so S simulations always
+    fit), in two workspaces that take turns.  The first run, and the first after reset_tree(), begins fresh trees; every
+    later run starts with sb_search_advance, which carries over the subtree of the lowest node whose record is the new root
+    (the child of the action played, or an opponent position the search expanded), at most R + 1 nodes of it.  Still
+    num_simulations + 2 launches.  self.kept i32[n] holds the nodes each tree carried over in the last run (0: a fresh root).
+    Root noise added at k = 0 applies to a carried-over root too: the prior of k = 0 replaces its stored one.  A captured
+    advancing run reads the trees the run before it finished, and an advance consumes the trees it reads (their node
+    counts become 0): replaying one captured run a second time starts every tree fresh (self.kept all 0).  To replay a
+    reusing loop, capture two consecutive runs in one graph, so that the workspaces take turns as they do eagerly.
     """
 
-    def __init__(self, n, num_simulations, c_puct=1.25, fpu=0.0, max_steps=400, engine=None, device=None):
+    def __init__(self, n, num_simulations, c_puct=1.25, fpu=0.0, max_steps=400, engine=None, device=None, reuse_nodes=0):
         if int(num_simulations) < 0:
             raise ValueError("num_simulations must be >= 0")
         if not (math.isfinite(c_puct) and c_puct >= 0) or not math.isfinite(fpu):
             raise ValueError("c_puct must be finite and >= 0, fpu finite")
+        if int(reuse_nodes) < 0:
+            raise ValueError("reuse_nodes must be >= 0")
         self.engine = engine if engine is not None else get_engine(device)
-        self.n, self.num_simulations = int(n), int(num_simulations)
+        self.n, self.num_simulations, self.reuse_nodes = int(n), int(num_simulations), int(reuse_nodes)
         self.c_puct, self.fpu, self.max_steps = float(c_puct), float(fpu), int(max_steps)
-        self.max_nodes = self.num_simulations + 1
-        self.ws = torch.empty(self.engine.search_workspace_bytes(self.n, self.max_nodes), dtype=torch.uint8, device=self.engine.device)
+        self.max_nodes = self.num_simulations + 1 + self.reuse_nodes
+        nb = self.engine.search_workspace_bytes(self.n, self.max_nodes)
+        self.ws = torch.empty(nb, dtype=torch.uint8, device=self.engine.device)
+        self.ws_next = torch.empty(nb, dtype=torch.uint8, device=self.engine.device) if self.reuse_nodes else None
+        self.kept = torch.zeros(self.n, dtype=torch.int32, device=self.engine.device)
+        self.fresh = True
         self.leaf = self.engine._search_outputs(self.n, None, LEAF_KEYS)
         self.out = self.engine._search_outputs(self.n, None, ("visits", "q", "root_value"))
+
+    def reset_tree(self):
+        """the next run begins fresh trees (kept 0), e.g. after new episodes were dealt"""
+        self.fresh = True
 
     def run(self, roots, evaluate):
         e, n, m = self.engine, self.n, self.max_nodes
         assert roots.shape[0] == n, "roots are u8[n, 512] with n = %d" % n
-        e.search_begin(self.ws, roots, m, self.max_steps, out=self.leaf)
+        if self.reuse_nodes and not self.fresh:
+            e.search_advance(self.ws, self.ws_next, roots, m, self.reuse_nodes + 1, self.max_steps, out=dict(self.leaf, kept=self.kept))
+            self.ws, self.ws_next = self.ws_next, self.ws
+        else:
+            e.search_begin(self.ws, roots, m, self.max_steps, out=self.leaf)
+            if self.reuse_nodes:
+                self.kept.zero_()
+        self.fresh = False
         prior, value = evaluate(self.leaf, 0)
         for k in range(1, self.num_simulations + 1):
             e.search_simulate(self.ws, n, m, prior, value, self.c_puct, self.fpu, out=self.leaf)
@@ -212,38 +248,87 @@ class InformationSetMCTS:
     capture-safe.  With caller keys (and a capture-safe evaluator) a run synchronises nothing with the host and can be
     captured in a torch.cuda.CUDAGraph.  A run is exactly 2 * num_simulations + 3 library launches (S + 1 sb_determinize,
     begin, S simulate, end).  The returned tensors are buffers of this object, overwritten by the next run.
+
+    reuse_nodes = R > 0 keeps trees between runs, as BatchedMCTS's (num_simulations + 1 + R nodes, two workspaces,
+    reset_tree(), self.kept): a later run passes played, the id played at the previous run's roots (e.g.
+    select_actions(visits)), and starts with sb_ismcts_advance, which carries over the subtree of that root action's child
+    (at most R + 1 nodes) where the new root is exactly the record sb_step(previous root, played) gives.  The run checks
+    that on the device: it keeps a copy of the previous roots, steps it with played (one sb_step) and compares it byte for
+    byte with the new roots; where they differ (an episode that ended and was redealt, a rejected action, an opponent turn
+    in between) the tree starts fresh.  Such a run is 2 * num_simulations + 4 library launches (2S + 3 with played None,
+    which starts every tree fresh), and with caller keys still capturable, with BatchedMCTS's caveat on replaying one
+    captured advancing run.  With R = 0, played is ignored.
     """
 
-    def __init__(self, n, num_simulations, c_puct=1.25, fpu=0.0, max_steps=400, seed=0, engine=None, device=None):
+    def __init__(self, n, num_simulations, c_puct=1.25, fpu=0.0, max_steps=400, seed=0, engine=None, device=None, reuse_nodes=0):
         if int(num_simulations) < 0:
             raise ValueError("num_simulations must be >= 0")
         if not (math.isfinite(c_puct) and c_puct >= 0) or not math.isfinite(fpu):
             raise ValueError("c_puct must be finite and >= 0, fpu finite")
+        if int(reuse_nodes) < 0:
+            raise ValueError("reuse_nodes must be >= 0")
         self.engine = e = engine if engine is not None else get_engine(device)
-        self.n, self.num_simulations = int(n), int(num_simulations)
+        self.n, self.num_simulations, self.reuse_nodes = int(n), int(num_simulations), int(reuse_nodes)
         self.c_puct, self.fpu, self.max_steps = float(c_puct), float(fpu), int(max_steps)
-        self.max_nodes = self.num_simulations + 1
+        self.max_nodes = self.num_simulations + 1 + self.reuse_nodes
         self.seed, self.calls = int(seed), 0
-        self.ws = torch.empty(e.ismcts_workspace_bytes(self.n, self.max_nodes), dtype=torch.uint8, device=e.device)
+        nb = e.ismcts_workspace_bytes(self.n, self.max_nodes)
+        self.ws = torch.empty(nb, dtype=torch.uint8, device=e.device)
         self.world = torch.empty((self.n, STATE_BYTES), dtype=torch.uint8, device=e.device)
+        self.kept = torch.zeros(self.n, dtype=torch.int32, device=e.device)
+        self.fresh = True
+        if self.reuse_nodes:
+            self.ws_next = torch.empty(nb, dtype=torch.uint8, device=e.device)
+            self.prev = torch.empty((self.n, STATE_BYTES), dtype=torch.uint8, device=e.device)
+            self.stepped = torch.empty((self.n, STATE_BYTES), dtype=torch.uint8, device=e.device)
+            self.played = torch.empty(self.n, dtype=torch.int32, device=e.device)
+            self.step_out = [torch.empty(self.n, dtype=d, device=e.device) for d in (torch.uint8, torch.int8, torch.uint8, torch.uint8)]
         self.leaf = e._search_outputs(self.n, None, LEAF_KEYS)
         self.out = e._search_outputs(self.n, None, ("visits", "q", "root_value"))
 
     def default_keys(self):
         """the keys of the next run without caller keys: next_seed(base + t) for t < (S+1)*n, base = next_seed(next_seed(seed)
-        + call index)"""
+        + call index).  The count is (num_simulations + 1) * n whatever reuse_nodes is."""
         base = next_seed(next_seed(self.seed) + self.calls)
         self.calls += 1
-        return next_seed_array(np.arange(self.max_nodes * self.n, dtype=np.uint64) + np.uint64(base))
+        return next_seed_array(np.arange((self.num_simulations + 1) * self.n, dtype=np.uint64) + np.uint64(base))
 
-    def run(self, roots, evaluate, keys=None):
-        e, n, m = self.engine, self.n, self.max_nodes
+    def reset_tree(self):
+        """the next run begins fresh trees (kept 0), e.g. after new episodes were dealt"""
+        self.fresh = True
+
+    def _played(self, roots, played):
+        """played i32[n] where sb_step(previous root, played) is the new root byte for byte, else -1"""
+        if played is None:
+            return self.played.fill_(-1)
+        played = torch.as_tensor(played).to(self.engine.device, torch.int64)
+        assert tuple(played.shape) == (self.n,), "played is one action id per root, [n]"
+        act, reward, done, err = self.step_out
+        ok = (played >= 0) & (played < N_ACTIONS)
+        act.copy_(torch.where(ok, played, N_ACTIONS - 1))
+        self.stepped.copy_(self.prev)
+        self.engine.step(self.stepped, act, reward=reward, done=done, err=err)
+        ok &= (self.stepped == roots).all(1)
+        return self.played.copy_(torch.where(ok, played, -1))
+
+    def run(self, roots, evaluate, keys=None, played=None):
+        e, n, m, S = self.engine, self.n, self.max_nodes, self.num_simulations
         assert roots.shape == (n, STATE_BYTES), "roots are u8[n, 512] with n = %d" % n
         if keys is None:
             keys = torch.from_numpy(self.default_keys()).to(e.device)
-        assert keys.shape == (m * n,), "keys are i64[(S + 1) * n] with (S + 1) * n = %d" % (m * n)
+        assert keys.shape == ((S + 1) * n,), "keys are i64[(S + 1) * n] with (S + 1) * n = %d" % ((S + 1) * n)
         e.determinize(roots, keys[:n], out=self.world)
-        e.ismcts_begin(self.ws, self.world, m, self.max_steps, out=self.leaf)
+        if self.reuse_nodes and not self.fresh:
+            e.ismcts_advance(self.ws, self.ws_next, self.world, self._played(roots, played), m, self.reuse_nodes + 1, self.max_steps,
+                             out=dict(self.leaf, kept=self.kept))
+            self.ws, self.ws_next = self.ws_next, self.ws
+        else:
+            e.ismcts_begin(self.ws, self.world, m, self.max_steps, out=self.leaf)
+            if self.reuse_nodes:
+                self.kept.zero_()
+        if self.reuse_nodes:
+            self.prev.copy_(roots)
+        self.fresh = False
         prior, value = evaluate(self.leaf, 0)
         for k in range(1, self.num_simulations + 1):
             e.determinize(roots, keys[k * n:(k + 1) * n], out=self.world)
