@@ -317,6 +317,46 @@ int sb_ismcts_advance(SbHandle *h, int n, int max_nodes, void *ws_src_d, void *w
                       uint8_t *leaf_states_d, int32_t *obs_d, uint32_t *masks_d, uint8_t *obs_err_d, uint8_t *to_move_d,
                       uint8_t *leaf_kind_d, void *stream);
 
+/* Several leaves per tree per call for the perfect-information search, under virtual loss, ABI 5's additive entry points
+ * (DESIGN.md 8.11):
+ *   sb_search_begin or sb_search_advance -> evaluate (n rows) -> (sb_search_simulate_batch -> evaluate (n * L rows)) x C
+ *   -> sb_search_end_batch
+ * The workspace is sb_search_batch_workspace_bytes(n, max_nodes, L) bytes: 8.6's workspace of sb_search_workspace_bytes(n,
+ * max_nodes) bytes, unchanged (so begin and advance write it, and advance reads a finished batched tree, as for 8.6), then
+ * per tree a tail holding the call's L pending slots and one int of virtual visits per node.  0 for bad arguments (n < 0,
+ * max_nodes outside 1..2^24, leaves outside 1..256, an overflow).  Every call of one search uses the same n, max_nodes and L.
+ * Slot l of tree g is row g * L + l of prior_d f32[n * L,156], value_d f32[n * L] and of every leaf output (sb_search_begin's
+ * outputs with n * L rows).  On a tree that begin, advance or a plain simulate left (one pending leaf), a batch call or
+ * the batch end backs up that leaf from row g * L (slot 0); afterwards the L slots are pending.  Mixing plain and batch
+ * calls within one search is otherwise unsupported (it computes wrong numbers, never outside the tree).  One batch call:
+ *   1. backs up the L pending slots in ascending slot order: EVAL stores the prior and adds sgn(leaf) * value along the path,
+ *      N += 1; TERMINAL adds the node's game value; FULL and COLLISION add nothing;
+ *   2. selects L leaves one after another: V(x) = the number of earlier slots of this call whose path (root to stop node
+ *      inclusive) contains x; at a non-terminal node s, for each legal a with child c (n_a = 0 without one) and sgn the sign
+ *      of s's seat: n_a = N(c) + V(c), q = ((sgn * W(c)) - (vl * V(c))) / n_a (fpu when n_a = 0),
+ *      u = ((c_puct * P(s,a)) * sqrt(N(s) + V(s))) / (1 + n_a), score = q + u, the highest wins, ties to the lowest id;
+ *      correctly rounded FP64 in this order (with V = 0 exactly sb_search_simulate's scores).  A walk stops at a new edge
+ *      (it takes the next free node at once: the slot is EVAL, or TERMINAL when the new record is over), at an existing
+ *      terminal node (TERMINAL, backed up again), at a node allocated earlier in the same call (COLLISION = 3: the root is
+ *      emitted, nothing is backed up) or, when no free node is left, with this and every later slot FULL (the root is
+ *      emitted; later calls stop the tree, as sb_search_simulate does);
+ *   3. expands the new nodes (the records sb_step(parent, a) gives) and emits every slot's leaf outputs, in parallel over
+ *      the n * L slots.  Virtual visits are zero again when the call returns.
+ * sb_search_end_batch backs up what is pending and writes sb_search_end's read-out (visits, q NaN where unvisited, root
+ * value); root visits then add up to the slots that were neither COLLISION nor FULL (plus the root's own evaluation).
+ * Bad arguments return -1 (sb_last_error) and launch nothing: those sb_search_simulate / sb_search_end reject (ws_bytes
+ * against the batch size), leaves outside 1..256, a negative or non-finite virtual_loss, n * leaves >= 2^31; n = 0 is a
+ * no-op.  sb_search_simulate_batch is two kernel launches (selection, one thread per tree; expansion, one thread per slot),
+ * sb_search_end_batch one, without handle scratch, atomics or host synchronisation (capturable in a CUDA graph).  Every
+ * index read from the workspace is checked; a bad one stops the tree (FULL) and is never dereferenced. */
+size_t sb_search_batch_workspace_bytes(int n, int max_nodes, int leaves);
+int sb_search_simulate_batch(SbHandle *h, int n, int max_nodes, int leaves, void *ws_d, size_t ws_bytes,
+                             const float *prior_d, const float *value_d, double c_puct, double fpu, double virtual_loss,
+                             uint8_t *leaf_states_d, int32_t *obs_d, uint32_t *masks_d, uint8_t *obs_err_d,
+                             uint8_t *to_move_d, uint8_t *leaf_kind_d, void *stream);
+int sb_search_end_batch(SbHandle *h, int n, int max_nodes, int leaves, void *ws_d, size_t ws_bytes, const float *prior_d,
+                        const float *value_d, int32_t *visits_d, double *q_d, double *root_value_d, void *stream);
+
 /* Determinization for sampled (PIMC) search:out_d[g] = states_d[g] with everything observer o cannot see resampled and
  * everything o sees kept byte for byte (sb_observe / sb_legal_mask / sb_features of o's view are unchanged).
  * observer_d u8[n] is nullable: NULL = each record's own local_order (the seat sb_observe and sb_legal_mask show); a

@@ -19,6 +19,8 @@
 //   k_ismcts_*         information-set tree search over caller-supplied worlds, one tree per thread (sb_ismcts.cuh)
 //   k_*_gumbel         Gumbel selection and read-out for both tree searches (sb_gumbel.cuh)
 //   k_*_advance        tree reuse between moves for both PUCT searches, one warp per tree for the copy (sb_reuse.cuh)
+//   k_search_batch_*   several leaves per tree per call under virtual loss: selection per tree, expansion per leaf
+//                      (sb_search_batch.cuh)
 //   k_determinize      one record per warp: resample what the observer cannot see (sb_determinize.cuh)
 //   k_accumulate_fitness win/draw/loss counts per individual (evo/fitness.py:95,160-166)
 //   k_es_*             evolution-strategy operators on the resident population (sb_es.cuh; evo/weights.py, evo/population.py)
@@ -1036,6 +1038,9 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32) k_env_step_heur(const EnvA
 // ---------------------------------------------------------------- tree reuse between moves (sb_*_advance)
 #include "sb_reuse.cuh"
 
+// ---------------------------------------------------------------- several leaves per tree per call (sb_search_*_batch)
+#include "sb_search_batch.cuh"
+
 // ---------------------------------------------------------------- determinization for sampled search (sb_determinize)
 #include "sb_determinize.cuh"
 
@@ -1843,6 +1848,66 @@ int sb_ismcts_advance(SbHandle* h, int n, int max_nodes, void* ws_src_d, void* w
   k_ismcts_advance<<<grid_for(n, TPB_GAME), RS_THREADS, 0, (cudaStream_t)stream>>>(a, r, h->d_cards, h->d_wt);
   LAUNCH_CHECK();
   return 0;
+}
+// The batch entries: the checks of sb_search_simulate / sb_search_end plus leaves and virtual_loss, against the batch
+// workspace size.  sb_search_simulate_batch launches two kernels (selection per tree, expansion per slot),
+// sb_search_end_batch one; no handle scratch, atomics or host synchronisation.
+static size_t batch_tail_bytes(int max_nodes, int leaves) { return ((size_t)8 * leaves + (size_t)4 * max_nodes + 15) & ~(size_t)15; }
+size_t sb_search_batch_workspace_bytes(int n, int max_nodes, int leaves) {
+  const size_t pre = sb_search_workspace_bytes(n, max_nodes);
+  if (n < 0 || leaves < 1 || leaves > SEARCH_MAX_LEAVES || (n > 0 && pre == 0)) return 0;
+  const size_t tail = batch_tail_bytes(max_nodes, leaves);
+  return (size_t)n > (SIZE_MAX - pre) / tail ? 0 : pre + (size_t)n * tail;
+}
+static int batch_launch(SbHandle* h, const SearchArgs& a, double vl, int leaves, size_t ws_bytes, const char* bad, bool end,
+                        void* stream) {
+  DEV_GUARD(h);
+  const size_t need = sb_search_batch_workspace_bytes(a.n, a.max_nodes, leaves);
+  if (!bad) bad = leaves < 1 || leaves > SEARCH_MAX_LEAVES ? "leaves must be 1..256"
+                  : end ? nullptr
+                  : !(vl >= 0.0 && vl <= 1.7976931348623157e308) ? "virtual_loss must be finite and >= 0"
+                  : nullptr;
+  if (!bad) bad = search_bad(a, SIZE_MAX);  // its size check is the 8.6 prefix's; the batch size is checked below
+  if (!bad) bad = (long long)a.n * leaves > 0x7FFFFFFFll ? "n * leaves must be below 2^31"
+                  : a.n > 0 && need == 0 ? "workspace size overflows size_t"
+                  : ws_bytes < need ? "workspace too small (sb_search_batch_workspace_bytes)"
+                  : nullptr;
+  if (bad) { snprintf(h->err, sizeof h->err, "%s: %s", end ? "sb_search_end_batch" : "sb_search_simulate_batch", bad); return -1; }
+  if (a.n == 0) return 0;
+  const BatchArgs b = {leaves, vl, a.ws + (size_t)a.n * a.tree_bytes, batch_tail_bytes(a.max_nodes, leaves)};
+  cudaStream_t st = (cudaStream_t)stream;
+  if (end) {
+    k_search_end_batch<<<grid_for(a.n, TPB_GAME), TPB_GAME, 0, st>>>(a, b);
+    LAUNCH_CHECK();
+    return 0;
+  }
+  k_search_batch_select<<<grid_for(a.n, SB_SELECT_THREADS), SB_SELECT_THREADS, 0, st>>>(a, b);
+  LAUNCH_CHECK();
+  k_search_batch_expand<<<grid_for(a.n * leaves, TPB_GAME), TPB_GAME, 0, st>>>(a, b, h->d_cards, h->d_wt);
+  LAUNCH_CHECK();
+  return 0;
+}
+int sb_search_simulate_batch(SbHandle* h, int n, int max_nodes, int leaves, void* ws_d, size_t ws_bytes, const float* prior_d,
+                             const float* value_d, double c_puct, double fpu, double virtual_loss, uint8_t* leaf_states_d,
+                             int32_t* obs_d, uint32_t* masks_d, uint8_t* obs_err_d, uint8_t* to_move_d, uint8_t* leaf_kind_d,
+                             void* stream) {
+  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, sizeof(STree) + (size_t)(max_nodes > 0 ? max_nodes : 0) * sizeof(SNode), nullptr,
+                  0, prior_d, value_d, c_puct, fpu, leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d,
+                  nullptr, nullptr, nullptr};
+  const char* bad = !(c_puct >= 0.0 && c_puct <= 1.7976931348623157e308) ? "c_puct must be finite and >= 0"
+                    : !(fpu >= -1.7976931348623157e308 && fpu <= 1.7976931348623157e308) ? "fpu must be finite"
+                    : n > 0 && (!prior_d || !value_d) ? "prior and value are required"
+                    : nullptr;
+  return batch_launch(h, a, virtual_loss, leaves, ws_bytes, bad, false, stream);
+}
+int sb_search_end_batch(SbHandle* h, int n, int max_nodes, int leaves, void* ws_d, size_t ws_bytes, const float* prior_d,
+                        const float* value_d, int32_t* visits_d, double* q_d, double* root_value_d, void* stream) {
+  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, sizeof(STree) + (size_t)(max_nodes > 0 ? max_nodes : 0) * sizeof(SNode), nullptr,
+                  0, prior_d, value_d, 0.0, 0.0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, visits_d, q_d, root_value_d};
+  const char* bad = n > 0 && (!prior_d || !value_d) ? "prior and value are required"
+                    : n > 0 && (!visits_d || !q_d || !root_value_d) ? "visits, q and root_value are required"
+                    : nullptr;
+  return batch_launch(h, a, 0.0, leaves, ws_bytes, bad, true, stream);
 }
 // One launch, no handle scratch, atomics or host synchronisation (capturable in a CUDA graph).
 int sb_determinize(SbHandle* h, int n, const uint8_t* states_d, const uint8_t* observer_d, const uint64_t* keys_d, uint8_t* out_d,

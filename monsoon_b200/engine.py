@@ -363,6 +363,36 @@ class Engine:
                                            self._p(o["visits"]), self._p(o["q"]), self._p(o["root_value"]), self._stream()), "sb_search_end")
         return o
 
+    # ---- several leaves per tree per call (sb_search_simulate_batch / sb_search_end_batch)
+    def search_batch_workspace_bytes(self, n, max_nodes, leaves):
+        return search_batch_workspace_bytes(n, max_nodes, leaves)
+
+    def search_simulate_batch(self, ws, n, max_nodes, leaves, prior, value, c_puct=1.25, fpu=0.0, virtual_loss=1.0, out=None):
+        """sb_search_simulate_batch: back up the pending leaves with prior f32[n*L,156] / value f32[n*L] (row g*L + l is slot
+        l of tree g; a tree that begin or advance left reads only slot 0), then select L leaves per tree under virtual loss,
+        expand and emit them into out (search_begin's buffers with n*L rows; kind 3 = collision, the root emitted).  ws holds
+        at least search_batch_workspace_bytes(n, max_nodes, L) bytes.  Returns that dict."""
+        self._dev(ws, torch.uint8)
+        rows = int(n) * int(leaves)
+        self._search_eval(rows, prior, value)
+        o = self._search_outputs(rows, out, ("states", "obs", "masks", "obs_err", "to_move", "kind"))
+        self._check(self.lib.sb_search_simulate_batch(self.h, n, int(max_nodes), int(leaves), self._p(ws), ws.numel(), self._p(prior),
+                                                      self._p(value), float(c_puct), float(fpu), float(virtual_loss), self._p(o["states"]),
+                                                      self._p(o["obs"]), self._p(o["masks"]), self._p(o["obs_err"]), self._p(o["to_move"]),
+                                                      self._p(o["kind"]), self._stream()), "sb_search_simulate_batch")
+        return o
+
+    def search_end_batch(self, ws, n, max_nodes, leaves, prior, value, out=None):
+        """sb_search_end_batch: back up the pending leaves (prior f32[n*L,156], value f32[n*L]), then search_end's read-out
+        into out: visits i32[n,156], q f64[n,156] and root_value f64[n].  Returns that dict."""
+        self._dev(ws, torch.uint8)
+        self._search_eval(int(n) * int(leaves), prior, value)
+        o = self._search_outputs(n, out, ("visits", "q", "root_value"))
+        self._check(self.lib.sb_search_end_batch(self.h, n, int(max_nodes), int(leaves), self._p(ws), ws.numel(), self._p(prior),
+                                                 self._p(value), self._p(o["visits"]), self._p(o["q"]), self._p(o["root_value"]),
+                                                 self._stream()), "sb_search_end_batch")
+        return o
+
     # ---- information-set tree search (sb_ismcts_begin / sb_ismcts_simulate / sb_ismcts_end)
     def ismcts_workspace_bytes(self, n, max_nodes):
         return ismcts_workspace_bytes(n, max_nodes)
@@ -615,6 +645,16 @@ def search_workspace_bytes(n, max_nodes):
     b = int(_lib.load().sb_search_workspace_bytes(int(n), int(max_nodes)))
     if n < 0 or max_nodes < 1 or (n > 0 and b == 0):
         raise ValueError("no search workspace for n=%d, max_nodes=%d (n >= 0, max_nodes 1..2^24)" % (n, max_nodes))
+    return b
+
+
+def search_batch_workspace_bytes(n, max_nodes, leaves):
+    """sb_search_batch_workspace_bytes: bytes of the batched search workspace of n trees of max_nodes nodes, L = leaves per
+    tree per call (host only, no GPU needed)."""
+    b = int(_lib.load().sb_search_batch_workspace_bytes(int(n), int(max_nodes), int(leaves)))
+    if n < 0 or max_nodes < 1 or not 1 <= leaves <= 256 or (n > 0 and b == 0):
+        raise ValueError("no batched search workspace for n=%d, max_nodes=%d, leaves=%d (n >= 0, max_nodes 1..2^24, leaves 1..256)"
+                         % (n, max_nodes, leaves))
     return b
 
 

@@ -39,6 +39,12 @@ softmax(logits + sigma(completed q)) to train on, next to the action to play:
     mcts = GumbelMCTS(env.n, num_simulations=16)
     action, policy, visits, q, root_value = mcts.run(env.states, evaluate)
     obs, masks, reward, done, info = env.step(action)
+
+With leaves_per_call = L > 1, BatchedMCTS selects L leaves per tree per call under virtual loss (sb_search_simulate_batch,
+DESIGN.md 8.11), so the evaluator sees n * L rows per call and is called S / L times instead of S:
+
+    mcts = BatchedMCTS(env.n, num_simulations=64, leaves_per_call=16)
+    visits, q, root_value = mcts.run(env.states, evaluate)   # evaluate(leaf, k): n rows at k = 0, n * 16 rows at k = 1..4
 """
 import math
 
@@ -73,15 +79,15 @@ def rollout_evaluator(engine=None, max_steps=400):
     rollout (sb_rollout_random, at most max_steps steps) run in place on leaf["states"]: +1 / -1 when the seat to move at the
     leaf wins / loses by the bases, 0 for a draw, an engine status or a rollout that hit max_steps."""
     engine = engine if engine is not None else get_engine()
-    bufs = {}
+    bufs = {}  # row count -> (prior, value): a batched search asks for n rows at k = 0 and n * L rows after
 
     def evaluate(leaf, k):
         states = leaf["states"]
         n = states.shape[0]
-        if bufs.get("n") != n:
-            bufs.update(n=n, prior=torch.empty((n, N_ACTIONS), dtype=torch.float32, device=states.device),
-                        value=torch.empty(n, dtype=torch.float32, device=states.device))
-        prior, value = bufs["prior"], bufs["value"]
+        if n not in bufs:
+            bufs[n] = (torch.empty((n, N_ACTIONS), dtype=torch.float32, device=states.device),
+                       torch.empty(n, dtype=torch.float32, device=states.device))
+        prior, value = bufs[n]
         legal = legal_actions(leaf["masks"])
         inv = torch.reciprocal(legal.sum(1, keepdim=True, dtype=torch.int32).to(torch.float32))
         torch.where(legal, inv, torch.zeros((), dtype=torch.float32, device=states.device), out=prior)
@@ -132,26 +138,46 @@ class BatchedMCTS:
     advancing run reads the trees the run before it finished, and an advance consumes the trees it reads (their node
     counts become 0): replaying one captured run a second time starts every tree fresh (self.kept all 0).  To replay a
     reusing loop, capture two consecutive runs in one graph, so that the workspaces take turns as they do eagerly.
+
+    leaves_per_call = L > 1 selects L leaves per tree per call under virtual loss (sb_search_simulate_batch, DESIGN.md
+    8.11): each selection counts the earlier paths of the same call as extra visits, each carrying virtual_loss, so the
+    leaves spread out, and all n * L are expanded in parallel and evaluated as one batch.  num_simulations = S must be a
+    multiple of L.  A run is the begin (or advance), C = S / L batch calls and the batch end: 2C + 2 library launches.
+    evaluate(leaf, k) gets the n roots at k = 0 and n * L rows at k = 1..C, tree-major (row g * L + l is leaf l of tree g),
+    with kind 3 for a collision (the walk reached a leaf another selection of the same call had just taken; the root is
+    emitted and its evaluation is not used).  The read-out is the same triple; a root's child visits then add up to its
+    slots that were neither a collision nor full, so they can sum to less than S.  L = 1 is the plain search exactly.
     """
 
-    def __init__(self, n, num_simulations, c_puct=1.25, fpu=0.0, max_steps=400, engine=None, device=None, reuse_nodes=0):
+    def __init__(self, n, num_simulations, c_puct=1.25, fpu=0.0, max_steps=400, engine=None, device=None, reuse_nodes=0,
+                 leaves_per_call=1, virtual_loss=1.0):
         if int(num_simulations) < 0:
             raise ValueError("num_simulations must be >= 0")
         if not (math.isfinite(c_puct) and c_puct >= 0) or not math.isfinite(fpu):
             raise ValueError("c_puct must be finite and >= 0, fpu finite")
         if int(reuse_nodes) < 0:
             raise ValueError("reuse_nodes must be >= 0")
-        self.engine = engine if engine is not None else get_engine(device)
+        if not 1 <= int(leaves_per_call) <= 256 or int(num_simulations) % int(leaves_per_call):
+            raise ValueError("leaves_per_call must be 1..256 and divide num_simulations")
+        if not (math.isfinite(virtual_loss) and virtual_loss >= 0):
+            raise ValueError("virtual_loss must be finite and >= 0")
+        self.engine = e = engine if engine is not None else get_engine(device)
         self.n, self.num_simulations, self.reuse_nodes = int(n), int(num_simulations), int(reuse_nodes)
         self.c_puct, self.fpu, self.max_steps = float(c_puct), float(fpu), int(max_steps)
+        self.leaves, self.virtual_loss = int(leaves_per_call), float(virtual_loss)
         self.max_nodes = self.num_simulations + 1 + self.reuse_nodes
-        nb = self.engine.search_workspace_bytes(self.n, self.max_nodes)
-        self.ws = torch.empty(nb, dtype=torch.uint8, device=self.engine.device)
-        self.ws_next = torch.empty(nb, dtype=torch.uint8, device=self.engine.device) if self.reuse_nodes else None
-        self.kept = torch.zeros(self.n, dtype=torch.int32, device=self.engine.device)
+        L = self.leaves
+        nb = e.search_workspace_bytes(self.n, self.max_nodes) if L == 1 else e.search_batch_workspace_bytes(self.n, self.max_nodes, L)
+        self.ws = torch.empty(nb, dtype=torch.uint8, device=e.device)
+        self.ws_next = torch.empty(nb, dtype=torch.uint8, device=e.device) if self.reuse_nodes else None
+        self.kept = torch.zeros(self.n, dtype=torch.int32, device=e.device)
         self.fresh = True
-        self.leaf = self.engine._search_outputs(self.n, None, LEAF_KEYS)
-        self.out = self.engine._search_outputs(self.n, None, ("visits", "q", "root_value"))
+        self.leaf = e._search_outputs(self.n, None, LEAF_KEYS)
+        self.out = e._search_outputs(self.n, None, ("visits", "q", "root_value"))
+        if L > 1:
+            self.batch_leaf = e._search_outputs(self.n * L, None, LEAF_KEYS)
+            self.batch_prior = torch.empty((self.n * L, N_ACTIONS), dtype=torch.float32, device=e.device)
+            self.batch_value = torch.empty(self.n * L, dtype=torch.float32, device=e.device)
 
     def reset_tree(self):
         """the next run begins fresh trees (kept 0), e.g. after new episodes were dealt"""
@@ -169,10 +195,21 @@ class BatchedMCTS:
                 self.kept.zero_()
         self.fresh = False
         prior, value = evaluate(self.leaf, 0)
-        for k in range(1, self.num_simulations + 1):
-            e.search_simulate(self.ws, n, m, prior, value, self.c_puct, self.fpu, out=self.leaf)
-            prior, value = evaluate(self.leaf, k)
-        e.search_end(self.ws, n, m, prior, value, out=self.out)
+        L = self.leaves
+        if L == 1:
+            for k in range(1, self.num_simulations + 1):
+                e.search_simulate(self.ws, n, m, prior, value, self.c_puct, self.fpu, out=self.leaf)
+                prior, value = evaluate(self.leaf, k)
+            e.search_end(self.ws, n, m, prior, value, out=self.out)
+            return self.out["visits"], self.out["q"], self.out["root_value"]
+        # the first batch call backs up the roots from slot 0 of each tree's rows; the other slots are not read
+        self.batch_prior.view(n, L, N_ACTIONS)[:, 0].copy_(prior)
+        self.batch_value.view(n, L)[:, 0].copy_(value)
+        prior, value = self.batch_prior, self.batch_value
+        for k in range(1, self.num_simulations // L + 1):
+            e.search_simulate_batch(self.ws, n, m, L, prior, value, self.c_puct, self.fpu, self.virtual_loss, out=self.batch_leaf)
+            prior, value = evaluate(self.batch_leaf, k)
+        e.search_end_batch(self.ws, n, m, L, prior, value, out=self.out)
         return self.out["visits"], self.out["q"], self.out["root_value"]
 
 
