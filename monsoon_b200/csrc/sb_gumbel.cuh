@@ -34,10 +34,10 @@
 //   return out[:S]
 // The first k entries of visits are always equal, so gb_seq replays this with one counter, per tree and call, in O(log S).
 //
-// Fault safety: every node index read from the workspace by the selection and the read-out is checked against the tree's
-// node count, and the descents are bounded by max_nodes (s_walk, ism_walk); 8.6's backup is s_backup, unchanged, which like
-// the PUCT kernels trusts the parent chain of a workspace written by sb_search_begin.  The 8.8 kernels compute the per-node
-// quantities in bounded sibling-walk passes plus a pass over the ids without a child and keep no per-id table on the stack.
+// Fault safety: each search's own rule.  The 8.6 kernels share the backup, walk and read-out of the PUCT kernels
+// (s_simulate, s_read_out: sb_search.cuh's rule); the edges of node j take a child link only in j+1..count-1 (s_child);
+// the 8.8 kernels share sb_ismcts.cuh's prologues and bounds (ism_simulate, ism_end), compute the per-node quantities in
+// bounded sibling-walk passes plus a pass over the ids without a child, and keep no per-id table on the stack.
 #pragma once
 #include "sb_es.cuh"
 #include "sb_ismcts.cuh"
@@ -176,12 +176,18 @@ SBD_FI int gb_select(const GumbelArgs& gb, int i, const Edges& E, const Node& nd
   return best;
 }
 
+// the read-out of tree i when its root has no legal action: policy 0, no action
+SBD_FI void gb_no_action(const GumbelArgs& gb, int i) {
+  #pragma unroll 1
+  for (int act = 0; act < SB_N_ACTIONS; act++) gb.policy[(size_t)i * SB_N_ACTIONS + act] = 0.f;
+  gb.action[i] = GUMBEL_NO_ACTION;
+}
+
 // the read-out of tree i after the last backup: policy row and action over the root's edges E (nd the root)
 template <class Edges, class Node>
 SBD_FI void gb_read_out(const GumbelArgs& gb, int i, const Edges& E, const Node& nd) {
+  gb_no_action(gb, i);  // the policy outside A; the action is set below
   float* pol = gb.policy + (size_t)i * SB_N_ACTIONS;
-  #pragma unroll 1
-  for (int act = 0; act < SB_N_ACTIONS; act++) pol[act] = 0.f;
   GbNode s;
   gb_node(s, E, nd, gb.c_visit, gb.c_scale, -1, true);
   int best = -1, lo = GUMBEL_NO_ACTION;
@@ -199,12 +205,11 @@ SBD_FI void gb_read_out(const GumbelArgs& gb, int i, const Edges& E, const Node&
 }
 
 // ---------------------------------------------------------------- 8.6: the perfect-information trees
-// A = the node's legal ids in increasing order; a child index outside 1..lim-1 counts as none (0)
+// A = the node's legal ids in increasing order; a child index outside lo+1..lim-1 counts as none (0), lo the node's own index
 struct GbSearchEdges {
   const SNode* nodes;
   const SNode& nd;
-  int lim;
-  SBD_FI int child(int act) const { const int c = nd.child[act]; return c > 0 && c < lim ? c : 0; }
+  int lo, lim;
   template <class F> SBD_FI void each(F f) const {
     #pragma unroll 1
     for (int w = 0; w < SB_MASK_WORDS; w++) {
@@ -212,7 +217,7 @@ struct GbSearchEdges {
       while (m) {
         const int act = w * 32 + __ffs(m) - 1;
         m &= m - 1;
-        const int c = child(act);
+        const int c = s_child(nd, act, lo, lim);
         f(act, c ? nodes[c].N : 0, c ? nodes[c].W : 0.0, c);
       }
     }
@@ -225,7 +230,7 @@ struct GbSearchEdges {
     for (int w = 0; w < SB_MASK_WORDS; w++) {
       u32 m = s.mask[w];
       while (m) {
-        const int c = child(w * 32 + __ffs(m) - 1);
+        const int c = s_child(s, w * 32 + __ffs(m) - 1, lo, lim);
         m &= m - 1;
         if (c) { sn += nodes[c].N; sw = __dadd_rn(sw, nodes[c].W); }
       }
@@ -242,18 +247,8 @@ __global__ void __launch_bounds__(TPB_GAME) k_search_simulate_gumbel(const Searc
   if (i >= a.n) return;
   G g;
   init_g(g, s_cards, wt);
-  STree& t = s_tree(a, i);
-  SNode* nodes = s_nodes(a, i);
-  if (t.used < 1 || t.used > a.max_nodes || (t.kind != SEARCH_FULL && (t.leaf < 0 || t.leaf >= t.used))) t.kind = SEARCH_FULL;
-  s_backup(a, i, t, nodes);
-  if (t.kind == SEARCH_FULL || t.used >= a.max_nodes) {  // the tree stops: the root is emitted, nothing is pending
-    t.kind = SEARCH_FULL;
-    s_emit_node(a, i, g, nodes[0], SEARCH_FULL);
-    return;
-  }
-  const int lim = t.used;
-  s_walk(a, i, g, t, nodes, [&](int j, int& c) {
-    const GbSearchEdges E{nodes, nodes[j], lim};
+  s_simulate(a, i, g, [&](const SNode* nodes, int j, int used, int& c) {
+    const GbSearchEdges E{nodes, nodes[j], j, used};
     return gb_select(gb, i, E, nodes[j], j == 0, c);
   });
 }
@@ -263,27 +258,12 @@ __global__ void __launch_bounds__(TPB_GAME) k_search_end_gumbel(const SearchArgs
   if (i >= a.n) return;
   STree& t = s_tree(a, i);
   SNode* nodes = s_nodes(a, i);
-  if (t.used < 1 || t.used > a.max_nodes || (t.kind != SEARCH_FULL && (t.leaf < 0 || t.leaf >= t.used))) t.kind = SEARCH_FULL;
   s_backup(a, i, t, nodes);
   t.kind = SEARCH_FULL;
-  const int lim = t.used < 1 ? 1 : t.used > a.max_nodes ? a.max_nodes : t.used;
-  const SNode& root = nodes[0];
-  const GbSearchEdges E{nodes, root, lim};
-  #pragma unroll 1
-  for (int act = 0; act < SB_N_ACTIONS; act++) {  // sb_search_end's read-out, over the checked child indices
-    const int c = E.child(act);
-    const int na = c ? nodes[c].N : 0;
-    a.visits[(size_t)i * SB_N_ACTIONS + act] = na;
-    a.q[(size_t)i * SB_N_ACTIONS + act] = na ? __ddiv_rn(__dmul_rn(s_sign(root.seat), nodes[c].W), (double)na) : __longlong_as_double(0x7FF8000000000000ll);
-  }
-  a.root_value[i] = __ddiv_rn(__dmul_rn(s_sign(root.seat), root.W), (double)root.N);
-  if (root.terminal) {  // A is empty: a terminal root never stores a prior
-    #pragma unroll 1
-    for (int act = 0; act < SB_N_ACTIONS; act++) gb.policy[(size_t)i * SB_N_ACTIONS + act] = 0.f;
-    gb.action[i] = GUMBEL_NO_ACTION;
-    return;
-  }
-  gb_read_out(gb, i, E, root);
+  const int used = sb_count(t, a.max_nodes);
+  s_read_out(a, i, nodes, used);
+  if (nodes[0].terminal) gb_no_action(gb, i);  // A is empty: a terminal root never stores a prior
+  else gb_read_out(gb, i, GbSearchEdges{nodes, nodes[0], 0, used}, nodes[0]);
 }
 
 // ---------------------------------------------------------------- 8.8: the information-set trees
@@ -315,17 +295,7 @@ struct GbIsmEdges {
       }
     }
   }
-  SBD_FI double vhat(const INode& s, double sgn) const { return gb_ism_vhat(nodes, lim, s, sgn); }
-  // every child of s in sibling-walk order
-  static SBD_FI double gb_ism_vhat(const INode* nodes, int lim, const INode& s, double sgn) {
-    int sn = 0;
-    double sw = 0.0;
-    int c = s.child;
-    #pragma unroll 1
-    for (int k = 0; k < lim && ism_in(c, lim); k++, c = nodes[c].sibling) { sn += nodes[c].N; sw = __dadd_rn(sw, nodes[c].W); }
-    const int den = s.N - sn;
-    return den < 1 ? 0.0 : __ddiv_rn(__dmul_rn(sgn, __dadd_rn(s.W, -sw)), (double)den);
-  }
+  SBD_FI double vhat(const INode& s, double sgn) const { return ism_vhat(nodes, lim, s, sgn); }
 };
 // end: A = the root ids whose stored code is set, in increasing id order, each with the child of its code
 struct GbIsmRootEdges {
@@ -342,7 +312,7 @@ struct GbIsmRootEdges {
       f(act, c >= 0 ? nodes[c].N : 0, c >= 0 ? nodes[c].W : 0.0, c);
     }
   }
-  SBD_FI double vhat(const INode& s, double sgn) const { return GbIsmEdges::gb_ism_vhat(nodes, lim, s, sgn); }
+  SBD_FI double vhat(const INode& s, double sgn) const { return ism_vhat(nodes, lim, s, sgn); }
 };
 
 __global__ void __launch_bounds__(TPB_GAME) k_ismcts_simulate_gumbel(const SearchArgs a, const GumbelArgs gb, const DCard* cards, const double* wt) {
@@ -352,20 +322,7 @@ __global__ void __launch_bounds__(TPB_GAME) k_ismcts_simulate_gumbel(const Searc
   if (i >= a.n) return;
   G g;
   init_g(g, s_cards, wt);
-  ITree& t = ism_tree(a, i);
-  INode* nodes = ism_nodes(a, i);
-  ism_backup(a, i, t, nodes);
-  __align__(16) SbState s;
-  load_state(s, a.roots + (size_t)i * SB_STATE_BYTES);  // this call's world at the root
-  unpack(g, s);
-  u32 m[SB_MASK_WORDS];
-  legal_mask(g, m);
-  if (t.kind == SEARCH_FULL || t.used < 1 || t.used >= a.max_nodes) {  // the tree stops: the world's root is emitted
-    t.kind = SEARCH_FULL;
-    ism_emit(a, i, g, s, m, SEARCH_FULL);
-    return;
-  }
-  ism_walk(a, i, g, t, nodes, s, m, [&](int j, int lim, int& c) {
+  ism_simulate(a, i, g, [&](const INode* nodes, int j, int lim, const u32* m, int& c) {
     const GbIsmEdges E{nodes, nodes[j], lim, g.pl[g.local_order], m};
     return gb_select(gb, i, E, nodes[j], j == 0, c);
   });
@@ -374,19 +331,8 @@ __global__ void __launch_bounds__(TPB_GAME) k_ismcts_simulate_gumbel(const Searc
 __global__ void __launch_bounds__(TPB_GAME) k_ismcts_end_gumbel(const SearchArgs a, const GumbelArgs gb) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= a.n) return;
-  ITree& t = ism_tree(a, i);
-  INode* nodes = ism_nodes(a, i);
-  ism_backup(a, i, t, nodes);
-  t.kind = SEARCH_FULL;
-  const int lim = ism_lim(t, a.max_nodes);
-  if (lim < 1) {
-    ism_read_out_empty(a, i);
-    #pragma unroll 1
-    for (int act = 0; act < SB_N_ACTIONS; act++) gb.policy[(size_t)i * SB_N_ACTIONS + act] = 0.f;
-    gb.action[i] = GUMBEL_NO_ACTION;
-    return;
-  }
-  ism_read_out(a, i, t, nodes, lim);
-  const GbIsmRootEdges E{nodes, nodes[0], lim, t};
-  gb_read_out(gb, i, E, nodes[0]);
+  const int lim = ism_end(a, i);
+  const INode* nodes = ism_nodes(a, i);
+  if (lim < 1) gb_no_action(gb, i);
+  else gb_read_out(gb, i, GbIsmRootEdges{nodes, nodes[0], lim, ism_tree(a, i)}, nodes[0]);
 }

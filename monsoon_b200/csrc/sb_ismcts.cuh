@@ -160,10 +160,7 @@ SBD_FI int ism_select(const SearchArgs& a, const INode* nodes, int lim, const IN
     const int act = ism_action(p, m, nodes[c].code);
     if (act < 0) continue;  // the move does not exist in this world
     has[act >> 5] |= 1u << (act & 31);
-    const int na = nodes[c].N;
-    const double q = na ? __ddiv_rn(__dmul_rn(sgn, nodes[c].W), (double)na) : a.fpu;
-    const double u = __ddiv_rn(__dmul_rn(__dmul_rn(a.c_puct, (double)nd.prior[act]), sq), (double)(1 + na));
-    const double score = __dadd_rn(q, u);
+    const double score = s_score(a, nodes[c].N, __dmul_rn(sgn, nodes[c].W), nd.prior[act], sq);
     if (best < 0 || score > best_score || (score == best_score && act < best)) { best = act; best_score = score; best_child = c; }
   }
   #pragma unroll 1
@@ -173,8 +170,7 @@ SBD_FI int ism_select(const SearchArgs& a, const INode* nodes, int lim, const IN
       const int act = w * 32 + __ffs(r) - 1;
       r &= r - 1;
       if (!ism_rep(p, m, act)) continue;
-      const double u = __ddiv_rn(__dmul_rn(__dmul_rn(a.c_puct, (double)nd.prior[act]), sq), 1.0);
-      const double score = __dadd_rn(a.fpu, u);
+      const double score = s_score(a, 0, 0.0, nd.prior[act], sq);
       if (best < 0 || score > best_score || (score == best_score && act < best)) { best = act; best_score = score; best_child = -1; }
     }
   }
@@ -226,11 +222,26 @@ __global__ void __launch_bounds__(TPB_GAME) k_ismcts_begin(const SearchArgs a, c
   ism_start(a, i, g, s, m, 0);
 }
 
-// one simulation's walk after the backup, in this call's world (record s, working set g, legal mask m at the root):
-// select(j, lim, c) chooses the action at node j among the world's legal representatives and sets c to the child with its
-// code (-1 = none).  Every node index is checked against lim and the descent is bounded by max_nodes.
+// one simulate call of tree i (k_ismcts_simulate, k_ismcts_simulate_gumbel): back up the pending leaf, unpack this call's
+// world at the root (record s, working set g, legal mask m), stop when the tree is full, else replay the tree's moves in
+// that world from the root and expand or emit a leaf.  select(nodes, j, lim, m, c) chooses the action at node j among the
+// world's legal representatives and sets c to the child with its code (-1 = none).  Every node index is checked against
+// lim and the descent is bounded by max_nodes.
 template <class Select>
-SBD_FI void ism_walk(const SearchArgs& a, int i, G& g, ITree& t, INode* nodes, SbState& s, u32* m, Select select) {
+SBD_FI void ism_simulate(const SearchArgs& a, int i, G& g, Select select) {
+  ITree& t = ism_tree(a, i);
+  INode* nodes = ism_nodes(a, i);
+  ism_backup(a, i, t, nodes);
+  __align__(16) SbState s;
+  load_state(s, a.roots + (size_t)i * SB_STATE_BYTES);
+  unpack(g, s);
+  u32 m[SB_MASK_WORDS];
+  legal_mask(g, m);
+  if (t.kind == SEARCH_FULL || t.used < 1 || t.used >= a.max_nodes) {  // the tree stops: the world's root is emitted
+    t.kind = SEARCH_FULL;
+    ism_emit(a, i, g, s, m, SEARCH_FULL);
+    return;
+  }
   const int lim = t.used;
   int j = 0;
   #pragma unroll 1
@@ -243,13 +254,10 @@ SBD_FI void ism_walk(const SearchArgs& a, int i, G& g, ITree& t, INode* nodes, S
       return;
     }
     int c;
-    const int act = select(j, lim, c);
+    const int act = select(nodes, j, lim, m, c);
     if (act < 0) break;
     const u32 code = ism_code(g.pl[g.local_order], act);
-    game_step(g, act);  // as sb_step: the working set the next sb_* call would unpack from the child's record
-    end_of_step(g);
-    pack(g, s);
-    unpack(g, s);
+    s_step(g, s, act);
     legal_mask(g, m);
     if (c < 0) {  // expand: a node for the code
       const int k = t.used++;
@@ -287,20 +295,9 @@ __global__ void __launch_bounds__(TPB_GAME) k_ismcts_simulate(const SearchArgs a
   if (i >= a.n) return;
   G g;
   init_g(g, s_cards, wt);
-  ITree& t = ism_tree(a, i);
-  INode* nodes = ism_nodes(a, i);
-  ism_backup(a, i, t, nodes);
-  __align__(16) SbState s;
-  load_state(s, a.roots + (size_t)i * SB_STATE_BYTES);  // this call's world at the root
-  unpack(g, s);
-  u32 m[SB_MASK_WORDS];
-  legal_mask(g, m);
-  if (t.kind == SEARCH_FULL || t.used < 1 || t.used >= a.max_nodes) {  // the tree stops: the world's root is emitted
-    t.kind = SEARCH_FULL;
-    ism_emit(a, i, g, s, m, SEARCH_FULL);
-    return;
-  }
-  ism_walk(a, i, g, t, nodes, s, m, [&](int j, int lim, int& c) { return ism_select(a, nodes, lim, nodes[j], g.pl[g.local_order], m, c); });
+  ism_simulate(a, i, g, [&](const INode* nodes, int j, int lim, const u32* m, int& c) {
+    return ism_select(a, nodes, lim, nodes[j], g.pl[g.local_order], m, c);
+  });
 }
 
 // the child of node nd whose code is `code` (first in the sibling walk), -1 if none
@@ -312,47 +309,47 @@ SBD_FI int ism_find(const INode* nodes, int lim, const INode& nd, u32 code) {
   return -1;
 }
 
-// visits, q and root_value of tree i by the root's action ids (sb_ismcts_end), lim >= 1
-SBD_FI void ism_read_out(const SearchArgs& a, int i, const ITree& t, const INode* nodes, int lim) {
-  const INode& root = nodes[0];
-  const double sgn = s_sign(root.seat);
-  const double nan = __longlong_as_double(0x7FF8000000000000ll);
+// the value estimate of node s from what its children do not account for, Gumbel's vhat (sb_gumbel.cuh): every child of s
+// in sibling-walk order
+SBD_FI double ism_vhat(const INode* nodes, int lim, const INode& s, double sgn) {
+  int sn = 0;
+  double sw = 0.0;
+  int c = s.child;
   #pragma unroll 1
-  for (int act = 0; act < SB_N_ACTIONS; act++) {
-    const u32 code = t.root_code[act];
-    int na = 0;
-    double w = 0.0;
-    if (code != ISM_NONE) {
-      int c = root.child;
-      #pragma unroll 1
-      for (int k = 0; k < lim && ism_in(c, lim); k++, c = nodes[c].sibling)
-        if (nodes[c].code == code) { na = nodes[c].N; w = nodes[c].W; break; }
-    }
-    a.visits[(size_t)i * SB_N_ACTIONS + act] = na;
-    a.q[(size_t)i * SB_N_ACTIONS + act] = na ? __ddiv_rn(__dmul_rn(sgn, w), (double)na) : nan;
-  }
-  a.root_value[i] = __ddiv_rn(__dmul_rn(sgn, root.W), (double)root.N);
-}
-// the read-out of a tree whose header holds no usable node count
-SBD_FI void ism_read_out_empty(const SearchArgs& a, int i) {
-  const double nan = __longlong_as_double(0x7FF8000000000000ll);
-  #pragma unroll 1
-  for (int act = 0; act < SB_N_ACTIONS; act++) { a.visits[(size_t)i * SB_N_ACTIONS + act] = 0; a.q[(size_t)i * SB_N_ACTIONS + act] = nan; }
-  a.root_value[i] = nan;
+  for (int k = 0; k < lim && ism_in(c, lim); k++, c = nodes[c].sibling) { sn += nodes[c].N; sw = __dadd_rn(sw, nodes[c].W); }
+  const int den = s.N - sn;
+  return den < 1 ? 0.0 : __ddiv_rn(__dmul_rn(sgn, __dadd_rn(s.W, -sw)), (double)den);
 }
 
-// back up the last pending leaf (the tree then holds nothing pending) and read out the root's edges by the root's action ids
-__global__ void __launch_bounds__(TPB_GAME) k_ismcts_end(const SearchArgs a) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= a.n) return;
+// back up the last pending leaf of tree i (the tree then holds nothing pending) and read out visits, q and root_value by
+// the root's action ids; returns the node count lim, 0 when the header holds none usable (the read-out is then empty)
+SBD_FI int ism_end(const SearchArgs& a, int i) {
   ITree& t = ism_tree(a, i);
   INode* nodes = ism_nodes(a, i);
   ism_backup(a, i, t, nodes);
   t.kind = SEARCH_FULL;
   const int lim = ism_lim(t, a.max_nodes);
   if (lim < 1) {
-    ism_read_out_empty(a, i);
-    return;
+    #pragma unroll 1
+    for (int act = 0; act < SB_N_ACTIONS; act++) { a.visits[(size_t)i * SB_N_ACTIONS + act] = 0; a.q[(size_t)i * SB_N_ACTIONS + act] = S_QNAN; }
+    a.root_value[i] = S_QNAN;
+    return 0;
   }
-  ism_read_out(a, i, t, nodes, lim);
+  const INode& root = nodes[0];
+  const double sgn = s_sign(root.seat);
+  #pragma unroll 1
+  for (int act = 0; act < SB_N_ACTIONS; act++) {
+    const u32 code = t.root_code[act];
+    const int c = code == ISM_NONE ? -1 : ism_find(nodes, lim, root, code);
+    const int na = c >= 0 ? nodes[c].N : 0;
+    a.visits[(size_t)i * SB_N_ACTIONS + act] = na;
+    a.q[(size_t)i * SB_N_ACTIONS + act] = na ? __ddiv_rn(__dmul_rn(sgn, nodes[c].W), (double)na) : S_QNAN;
+  }
+  a.root_value[i] = __ddiv_rn(__dmul_rn(sgn, root.W), (double)root.N);
+  return lim;
+}
+
+__global__ void __launch_bounds__(TPB_GAME) k_ismcts_end(const SearchArgs a) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < a.n) ism_end(a, i);
 }

@@ -27,6 +27,7 @@
 // State is AoS [n][512 B]; every thread (or warp) moves its record with 128-bit loads/stores; the card
 // table (130 x 24 B) is staged in shared memory once per CTA.
 #include <cuda_runtime.h>
+#include <initializer_list>
 #include <stdio.h>
 #include <string.h>
 #include <stdlib.h>
@@ -1598,130 +1599,41 @@ int sb_env_step(SbHandle* h, int n, uint8_t* states_d, const uint8_t* actions_d,
                max_steps, (i8*)result_d, length_d, final_states_d, obs_d, masks_d, obs_err_d};
   return env_launch(h, a, "sb_env_step", stream);
 }
-// The search entries launch exactly one kernel, use no handle scratch, no atomics and no host synchronisation.
-size_t sb_search_workspace_bytes(int n, int max_nodes) {
-  if (n < 0 || max_nodes < 1 || max_nodes > SEARCH_MAX_NODES) return 0;
-  const size_t tree = sizeof(STree) + (size_t)max_nodes * sizeof(SNode);
-  return (size_t)n > SIZE_MAX / tree ? 0 : (size_t)n * tree;
-}
-static const char* search_bad(const SearchArgs& a, size_t ws_bytes) {
-  const size_t need = sb_search_workspace_bytes(a.n, a.max_nodes);
-  return a.n < 0 ? "n must be >= 0"
-         : a.max_nodes < 1 || a.max_nodes > SEARCH_MAX_NODES ? "max_nodes must be 1..2^24"
-         : a.n > 0 && need == 0 ? "workspace size overflows size_t"
-         : a.n > 0 && !a.ws ? "workspace is NULL"
-         : ((uintptr_t)a.ws & 15) ? "workspace must be 16-byte aligned"
-         : ws_bytes < need ? "workspace too small (sb_search_workspace_bytes)"
-         : nullptr;
-}
-static int search_launch(SbHandle* h, const SearchArgs& a, size_t ws_bytes, const char* bad, int which, void* stream) {
-  DEV_GUARD(h);
-  if (!bad) bad = search_bad(a, ws_bytes);
-  if (bad) { snprintf(h->err, sizeof h->err, "%s: %s", which == 0 ? "sb_search_begin" : which == 1 ? "sb_search_simulate" : "sb_search_end", bad); return -1; }
-  if (a.n == 0) return 0;
-  cudaStream_t st = (cudaStream_t)stream;
-  const int grid = grid_for(a.n, TPB_GAME);
-  if (which == 0) k_search_begin<<<grid, TPB_GAME, 0, st>>>(a, h->d_cards, h->d_wt);
-  else if (which == 1) k_search_simulate<<<grid, TPB_GAME, 0, st>>>(a, h->d_cards, h->d_wt);
-  else k_search_end<<<grid, TPB_GAME, 0, st>>>(a);
-  LAUNCH_CHECK();
-  return 0;
-}
-int sb_search_begin(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const uint8_t* roots_d, int max_steps,
-                    uint8_t* leaf_states_d, int32_t* obs_d, uint32_t* masks_d, uint8_t* obs_err_d, uint8_t* to_move_d,
-                    uint8_t* leaf_kind_d, void* stream) {
-  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, sizeof(STree) + (size_t)(max_nodes > 0 ? max_nodes : 0) * sizeof(SNode), roots_d,
-                  max_steps, nullptr, nullptr, 0.0, 0.0, leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d,
-                  nullptr, nullptr, nullptr};
-  const char* bad = max_steps < 1 || max_steps > 65535 ? "max_steps must be 1..65535"
-                    : n > 0 && !roots_d ? "roots are required"
-                    : nullptr;
-  return search_launch(h, a, ws_bytes, bad, 0, stream);
-}
-int sb_search_simulate(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const float* prior_d, const float* value_d,
-                       double c_puct, double fpu, uint8_t* leaf_states_d, int32_t* obs_d, uint32_t* masks_d, uint8_t* obs_err_d,
-                       uint8_t* to_move_d, uint8_t* leaf_kind_d, void* stream) {
-  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, sizeof(STree) + (size_t)(max_nodes > 0 ? max_nodes : 0) * sizeof(SNode), nullptr,
-                  0, prior_d, value_d, c_puct, fpu, leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d,
-                  nullptr, nullptr, nullptr};
-  const char* bad = !(c_puct >= 0.0 && c_puct <= 1.7976931348623157e308) ? "c_puct must be finite and >= 0"
-                    : !(fpu >= -1.7976931348623157e308 && fpu <= 1.7976931348623157e308) ? "fpu must be finite"
-                    : n > 0 && (!prior_d || !value_d) ? "prior and value are required"
-                    : nullptr;
-  return search_launch(h, a, ws_bytes, bad, 1, stream);
-}
-int sb_search_end(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const float* prior_d, const float* value_d,
-                  int32_t* visits_d, double* q_d, double* root_value_d, void* stream) {
-  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, sizeof(STree) + (size_t)(max_nodes > 0 ? max_nodes : 0) * sizeof(SNode), nullptr,
-                  0, prior_d, value_d, 0.0, 0.0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, visits_d, q_d, root_value_d};
-  const char* bad = n > 0 && (!prior_d || !value_d) ? "prior and value are required"
-                    : n > 0 && (!visits_d || !q_d || !root_value_d) ? "visits, q and root_value are required"
-                    : nullptr;
-  return search_launch(h, a, ws_bytes, bad, 2, stream);
-}
-// The information-set search entries launch exactly one kernel, use no handle scratch, no atomics and no host synchronisation.
-size_t sb_ismcts_workspace_bytes(int n, int max_nodes) {
-  if (n < 0 || max_nodes < 1 || max_nodes > SEARCH_MAX_NODES) return 0;
-  const size_t tree = sizeof(ITree) + (size_t)max_nodes * sizeof(INode);
-  return (size_t)n > SIZE_MAX / tree ? 0 : (size_t)n * tree;
-}
-static const char* ismcts_bad(const SearchArgs& a, size_t ws_bytes) {
-  const size_t need = sb_ismcts_workspace_bytes(a.n, a.max_nodes);
-  return a.n < 0 ? "n must be >= 0"
-         : a.max_nodes < 1 || a.max_nodes > SEARCH_MAX_NODES ? "max_nodes must be 1..2^24"
-         : a.n > 0 && need == 0 ? "workspace size overflows size_t"
-         : a.n > 0 && !a.ws ? "workspace is NULL"
-         : ((uintptr_t)a.ws & 15) ? "workspace must be 16-byte aligned"
-         : ws_bytes < need ? "workspace too small (sb_ismcts_workspace_bytes)"
-         : nullptr;
-}
-static int ismcts_launch(SbHandle* h, const SearchArgs& a, size_t ws_bytes, const char* bad, int which, void* stream) {
-  DEV_GUARD(h);
-  if (!bad) bad = ismcts_bad(a, ws_bytes);
-  if (bad) { snprintf(h->err, sizeof h->err, "%s: %s", which == 0 ? "sb_ismcts_begin" : which == 1 ? "sb_ismcts_simulate" : "sb_ismcts_end", bad); return -1; }
-  if (a.n == 0) return 0;
-  cudaStream_t st = (cudaStream_t)stream;
-  const int grid = grid_for(a.n, TPB_GAME);
-  if (which == 0) k_ismcts_begin<<<grid, TPB_GAME, 0, st>>>(a, h->d_cards, h->d_wt);
-  else if (which == 1) k_ismcts_simulate<<<grid, TPB_GAME, 0, st>>>(a, h->d_cards, h->d_wt);
-  else k_ismcts_end<<<grid, TPB_GAME, 0, st>>>(a);
-  LAUNCH_CHECK();
-  return 0;
-}
+// The search entries (sb_search_*, sb_ismcts_*): every entry launches exactly one kernel, except sb_search_simulate_batch
+// (two), and uses no handle scratch, no atomics and no host synchronisation.  Each checks its arguments in a fixed order
+// and reports the first reason it finds.
+static size_t search_tree_bytes(int max_nodes) { return sizeof(STree) + (size_t)(max_nodes > 0 ? max_nodes : 0) * sizeof(SNode); }
 static size_t ismcts_tree_bytes(int max_nodes) { return sizeof(ITree) + (size_t)(max_nodes > 0 ? max_nodes : 0) * sizeof(INode); }
-int sb_ismcts_begin(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const uint8_t* det_d, int max_steps,
-                    uint8_t* leaf_states_d, int32_t* obs_d, uint32_t* masks_d, uint8_t* obs_err_d, uint8_t* to_move_d,
-                    uint8_t* leaf_kind_d, void* stream) {
-  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, ismcts_tree_bytes(max_nodes), det_d, max_steps, nullptr, nullptr, 0.0, 0.0,
-                  leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d, nullptr, nullptr, nullptr};
-  const char* bad = max_steps < 1 || max_steps > 65535 ? "max_steps must be 1..65535"
-                    : n > 0 && !det_d ? "worlds (det) are required"
-                    : nullptr;
-  return ismcts_launch(h, a, ws_bytes, bad, 0, stream);
+// n trees of tree_bytes each, 0 on a bad argument or an overflow
+static size_t trees_bytes(int n, int max_nodes, size_t tree_bytes) {
+  if (n < 0 || max_nodes < 1 || max_nodes > SEARCH_MAX_NODES) return 0;
+  return (size_t)n > SIZE_MAX / tree_bytes ? 0 : (size_t)n * tree_bytes;
 }
-int sb_ismcts_simulate(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const uint8_t* det_d, const float* prior_d,
-                       const float* value_d, double c_puct, double fpu, uint8_t* leaf_states_d, int32_t* obs_d, uint32_t* masks_d,
-                       uint8_t* obs_err_d, uint8_t* to_move_d, uint8_t* leaf_kind_d, void* stream) {
-  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, ismcts_tree_bytes(max_nodes), det_d, 0, prior_d, value_d, c_puct, fpu,
-                  leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d, nullptr, nullptr, nullptr};
-  const char* bad = !(c_puct >= 0.0 && c_puct <= 1.7976931348623157e308) ? "c_puct must be finite and >= 0"
-                    : !(fpu >= -1.7976931348623157e308 && fpu <= 1.7976931348623157e308) ? "fpu must be finite"
-                    : n > 0 && !det_d ? "worlds (det) are required"
-                    : n > 0 && (!prior_d || !value_d) ? "prior and value are required"
-                    : nullptr;
-  return ismcts_launch(h, a, ws_bytes, bad, 1, stream);
+size_t sb_search_workspace_bytes(int n, int max_nodes) { return trees_bytes(n, max_nodes, search_tree_bytes(max_nodes)); }
+size_t sb_ismcts_workspace_bytes(int n, int max_nodes) { return trees_bytes(n, max_nodes, ismcts_tree_bytes(max_nodes)); }
+// n, max_nodes and the workspace of a.tree_bytes per tree; too_small is the reason when ws_bytes is below that size
+static const char* ws_bad(const SearchArgs& a, size_t ws_bytes, const char* too_small) {
+  const size_t need = trees_bytes(a.n, a.max_nodes, a.tree_bytes);
+  return a.n < 0 ? "n must be >= 0"
+         : a.max_nodes < 1 || a.max_nodes > SEARCH_MAX_NODES ? "max_nodes must be 1..2^24"
+         : a.n > 0 && need == 0 ? "workspace size overflows size_t"
+         : a.n > 0 && !a.ws ? "workspace is NULL"
+         : ((uintptr_t)a.ws & 15) ? "workspace must be 16-byte aligned"
+         : ws_bytes < need ? too_small
+         : nullptr;
 }
-int sb_ismcts_end(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const float* prior_d, const float* value_d,
-                  int32_t* visits_d, double* q_d, double* root_value_d, void* stream) {
-  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, ismcts_tree_bytes(max_nodes), nullptr, 0, prior_d, value_d, 0.0, 0.0,
-                  nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, visits_d, q_d, root_value_d};
-  const char* bad = n > 0 && (!prior_d || !value_d) ? "prior and value are required"
-                    : n > 0 && (!visits_d || !q_d || !root_value_d) ? "visits, q and root_value are required"
-                    : nullptr;
-  return ismcts_launch(h, a, ws_bytes, bad, 2, stream);
+#define SEARCH_WS_SMALL "workspace too small (sb_search_workspace_bytes)"
+#define ISMCTS_WS_SMALL "workspace too small (sb_ismcts_workspace_bytes)"
+static const char* steps_bad(int max_steps) { return max_steps < 1 || max_steps > 65535 ? "max_steps must be 1..65535" : nullptr; }
+static const char* puct_bad(double c_puct, double fpu) {
+  return !(c_puct >= 0.0 && c_puct <= 1.7976931348623157e308) ? "c_puct must be finite and >= 0"
+         : !(fpu >= -1.7976931348623157e308 && fpu <= 1.7976931348623157e308) ? "fpu must be finite"
+         : nullptr;
 }
-// The Gumbel entries: the checks of their PUCT siblings plus the Gumbel arguments; one launch each, no handle scratch, no
-// atomics and no host synchronisation.
+static const char* eval_bad(const SearchArgs& a) { return a.n > 0 && (!a.prior || !a.value) ? "prior and value are required" : nullptr; }
+static const char* read_out_bad(const SearchArgs& a) {
+  return a.n > 0 && (!a.visits || !a.q || !a.root_value) ? "visits, q and root_value are required" : nullptr;
+}
 static const char* gumbel_bad(int n, const GumbelArgs& gb, bool end) {
   const double big = 1.7976931348623157e308;
   return !(gb.c_visit >= 0.0 && gb.c_visit <= big) ? "c_visit must be finite and >= 0"
@@ -1734,18 +1646,125 @@ static const char* gumbel_bad(int n, const GumbelArgs& gb, bool end) {
          : gb.max_considered < 1 || gb.max_considered > SB_N_ACTIONS ? "max_considered must be 1..156"
          : nullptr;
 }
+static const char* reuse_bad(const SearchArgs& a, const ReuseArgs& r) {  // after ws_bad
+  const size_t span = (size_t)(a.n > 0 ? a.n : 0) * a.tree_bytes;
+  const uintptr_t s = (uintptr_t)r.src, d = (uintptr_t)a.ws;
+  return r.keep < 1 || r.keep > a.max_nodes ? "keep must be 1..max_nodes"
+         : a.n > 0 && !r.src ? "source workspace is NULL"
+         : ((uintptr_t)r.src & 15) ? "source workspace must be 16-byte aligned"
+         : a.n > 0 && r.src == a.ws ? "ws_src and ws_dst must be two workspaces"
+         : a.n > 0 && s < d + span && d < s + span ? "ws_src and ws_dst overlap"
+         : nullptr;
+}
+// the first reason of the list (every check is a pure function of the arguments); nullptr when there is none
+static const char* first_bad(std::initializer_list<const char*> reasons) {
+  for (const char* r : reasons)
+    if (r) return r;
+  return nullptr;
+}
+static int refuse(SbHandle* h, const char* what, const char* bad) {
+  snprintf(h->err, sizeof h->err, "%s: %s", what, bad);
+  return -1;
+}
+static void set_leaves(SearchArgs& a, uint8_t* leaf_states_d, int32_t* obs_d, uint32_t* masks_d, uint8_t* obs_err_d,
+                       uint8_t* to_move_d, uint8_t* leaf_kind_d) {
+  a.leaf_states = leaf_states_d; a.obs = obs_d; a.masks = masks_d; a.obs_err = obs_err_d; a.to_move = to_move_d;
+  a.leaf_kind = leaf_kind_d;
+}
+int sb_search_begin(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const uint8_t* roots_d, int max_steps,
+                    uint8_t* leaf_states_d, int32_t* obs_d, uint32_t* masks_d, uint8_t* obs_err_d, uint8_t* to_move_d,
+                    uint8_t* leaf_kind_d, void* stream) {
+  DEV_GUARD(h);
+  SearchArgs a(n, max_nodes, ws_d, search_tree_bytes(max_nodes));
+  a.roots = roots_d; a.max_steps = max_steps;
+  set_leaves(a, leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d);
+  const char* bad = first_bad({steps_bad(max_steps), n > 0 && !roots_d ? "roots are required" : nullptr,
+                               ws_bad(a, ws_bytes, SEARCH_WS_SMALL)});
+  if (bad) return refuse(h, "sb_search_begin", bad);
+  if (n == 0) return 0;
+  k_search_begin<<<grid_for(n, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a, h->d_cards, h->d_wt);
+  LAUNCH_CHECK();
+  return 0;
+}
+int sb_search_simulate(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const float* prior_d, const float* value_d,
+                       double c_puct, double fpu, uint8_t* leaf_states_d, int32_t* obs_d, uint32_t* masks_d, uint8_t* obs_err_d,
+                       uint8_t* to_move_d, uint8_t* leaf_kind_d, void* stream) {
+  DEV_GUARD(h);
+  SearchArgs a(n, max_nodes, ws_d, search_tree_bytes(max_nodes));
+  a.prior = prior_d; a.value = value_d; a.c_puct = c_puct; a.fpu = fpu;
+  set_leaves(a, leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d);
+  const char* bad = first_bad({puct_bad(c_puct, fpu), eval_bad(a), ws_bad(a, ws_bytes, SEARCH_WS_SMALL)});
+  if (bad) return refuse(h, "sb_search_simulate", bad);
+  if (n == 0) return 0;
+  k_search_simulate<<<grid_for(n, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a, h->d_cards, h->d_wt);
+  LAUNCH_CHECK();
+  return 0;
+}
+int sb_search_end(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const float* prior_d, const float* value_d,
+                  int32_t* visits_d, double* q_d, double* root_value_d, void* stream) {
+  DEV_GUARD(h);
+  SearchArgs a(n, max_nodes, ws_d, search_tree_bytes(max_nodes));
+  a.prior = prior_d; a.value = value_d; a.visits = visits_d; a.q = q_d; a.root_value = root_value_d;
+  const char* bad = first_bad({eval_bad(a), read_out_bad(a), ws_bad(a, ws_bytes, SEARCH_WS_SMALL)});
+  if (bad) return refuse(h, "sb_search_end", bad);
+  if (n == 0) return 0;
+  k_search_end<<<grid_for(n, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a);
+  LAUNCH_CHECK();
+  return 0;
+}
+int sb_ismcts_begin(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const uint8_t* det_d, int max_steps,
+                    uint8_t* leaf_states_d, int32_t* obs_d, uint32_t* masks_d, uint8_t* obs_err_d, uint8_t* to_move_d,
+                    uint8_t* leaf_kind_d, void* stream) {
+  DEV_GUARD(h);
+  SearchArgs a(n, max_nodes, ws_d, ismcts_tree_bytes(max_nodes));
+  a.roots = det_d; a.max_steps = max_steps;
+  set_leaves(a, leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d);
+  const char* bad = first_bad({steps_bad(max_steps), n > 0 && !det_d ? "worlds (det) are required" : nullptr,
+                               ws_bad(a, ws_bytes, ISMCTS_WS_SMALL)});
+  if (bad) return refuse(h, "sb_ismcts_begin", bad);
+  if (n == 0) return 0;
+  k_ismcts_begin<<<grid_for(n, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a, h->d_cards, h->d_wt);
+  LAUNCH_CHECK();
+  return 0;
+}
+int sb_ismcts_simulate(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const uint8_t* det_d, const float* prior_d,
+                       const float* value_d, double c_puct, double fpu, uint8_t* leaf_states_d, int32_t* obs_d, uint32_t* masks_d,
+                       uint8_t* obs_err_d, uint8_t* to_move_d, uint8_t* leaf_kind_d, void* stream) {
+  DEV_GUARD(h);
+  SearchArgs a(n, max_nodes, ws_d, ismcts_tree_bytes(max_nodes));
+  a.roots = det_d; a.prior = prior_d; a.value = value_d; a.c_puct = c_puct; a.fpu = fpu;
+  set_leaves(a, leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d);
+  const char* bad = first_bad({puct_bad(c_puct, fpu), n > 0 && !det_d ? "worlds (det) are required" : nullptr, eval_bad(a),
+                               ws_bad(a, ws_bytes, ISMCTS_WS_SMALL)});
+  if (bad) return refuse(h, "sb_ismcts_simulate", bad);
+  if (n == 0) return 0;
+  k_ismcts_simulate<<<grid_for(n, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a, h->d_cards, h->d_wt);
+  LAUNCH_CHECK();
+  return 0;
+}
+int sb_ismcts_end(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const float* prior_d, const float* value_d,
+                  int32_t* visits_d, double* q_d, double* root_value_d, void* stream) {
+  DEV_GUARD(h);
+  SearchArgs a(n, max_nodes, ws_d, ismcts_tree_bytes(max_nodes));
+  a.prior = prior_d; a.value = value_d; a.visits = visits_d; a.q = q_d; a.root_value = root_value_d;
+  const char* bad = first_bad({eval_bad(a), read_out_bad(a), ws_bad(a, ws_bytes, ISMCTS_WS_SMALL)});
+  if (bad) return refuse(h, "sb_ismcts_end", bad);
+  if (n == 0) return 0;
+  k_ismcts_end<<<grid_for(n, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a);
+  LAUNCH_CHECK();
+  return 0;
+}
 int sb_search_simulate_gumbel(SbHandle* h, int n, int max_nodes, void* ws_d, size_t ws_bytes, const float* prior_d,
                               const float* value_d, const float* gumbel_d, int sim, int num_simulations, int max_considered,
                               double c_visit, double c_scale, uint8_t* leaf_states_d, int32_t* obs_d, uint32_t* masks_d,
                               uint8_t* obs_err_d, uint8_t* to_move_d, uint8_t* leaf_kind_d, void* stream) {
   DEV_GUARD(h);
-  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, sizeof(STree) + (size_t)(max_nodes > 0 ? max_nodes : 0) * sizeof(SNode), nullptr,
-                  0, prior_d, value_d, 0.0, 0.0, leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d,
-                  nullptr, nullptr, nullptr};
+  SearchArgs a(n, max_nodes, ws_d, search_tree_bytes(max_nodes));
+  a.prior = prior_d; a.value = value_d;
+  set_leaves(a, leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d);
   const GumbelArgs gb = {gumbel_d, sim, num_simulations, max_considered, c_visit, c_scale, nullptr, nullptr};
-  const char* bad = gumbel_bad(n, gb, false);
-  if (!bad) bad = n > 0 && (!prior_d || !value_d) ? "prior and value are required" : search_bad(a, ws_bytes);
-  if (bad) { snprintf(h->err, sizeof h->err, "sb_search_simulate_gumbel: %s", bad); return -1; }
+  const char* bad = first_bad({gumbel_bad(n, gb, false), eval_bad(a), ws_bad(a, ws_bytes, SEARCH_WS_SMALL)});
+  if (bad) return refuse(h, "sb_search_simulate_gumbel", bad);
   if (n == 0) return 0;
   k_search_simulate_gumbel<<<grid_for(n, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a, gb, h->d_cards, h->d_wt);
   LAUNCH_CHECK();
@@ -1755,14 +1774,11 @@ int sb_search_end_gumbel(SbHandle* h, int n, int max_nodes, void* ws_d, size_t w
                          const float* gumbel_d, double c_visit, double c_scale, int32_t* action_d, float* policy_d,
                          int32_t* visits_d, double* q_d, double* root_value_d, void* stream) {
   DEV_GUARD(h);
-  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, sizeof(STree) + (size_t)(max_nodes > 0 ? max_nodes : 0) * sizeof(SNode), nullptr,
-                  0, prior_d, value_d, 0.0, 0.0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, visits_d, q_d, root_value_d};
+  SearchArgs a(n, max_nodes, ws_d, search_tree_bytes(max_nodes));
+  a.prior = prior_d; a.value = value_d; a.visits = visits_d; a.q = q_d; a.root_value = root_value_d;
   const GumbelArgs gb = {gumbel_d, 0, 0, 0, c_visit, c_scale, action_d, policy_d};
-  const char* bad = gumbel_bad(n, gb, true);
-  if (!bad) bad = n > 0 && (!prior_d || !value_d) ? "prior and value are required"
-                  : n > 0 && (!visits_d || !q_d || !root_value_d) ? "visits, q and root_value are required"
-                  : search_bad(a, ws_bytes);
-  if (bad) { snprintf(h->err, sizeof h->err, "sb_search_end_gumbel: %s", bad); return -1; }
+  const char* bad = first_bad({gumbel_bad(n, gb, true), eval_bad(a), read_out_bad(a), ws_bad(a, ws_bytes, SEARCH_WS_SMALL)});
+  if (bad) return refuse(h, "sb_search_end_gumbel", bad);
   if (n == 0) return 0;
   k_search_end_gumbel<<<grid_for(n, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a, gb);
   LAUNCH_CHECK();
@@ -1773,12 +1789,13 @@ int sb_ismcts_simulate_gumbel(SbHandle* h, int n, int max_nodes, void* ws_d, siz
                               int max_considered, double c_visit, double c_scale, uint8_t* leaf_states_d, int32_t* obs_d,
                               uint32_t* masks_d, uint8_t* obs_err_d, uint8_t* to_move_d, uint8_t* leaf_kind_d, void* stream) {
   DEV_GUARD(h);
-  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, ismcts_tree_bytes(max_nodes), det_d, 0, prior_d, value_d, 0.0, 0.0,
-                  leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d, nullptr, nullptr, nullptr};
+  SearchArgs a(n, max_nodes, ws_d, ismcts_tree_bytes(max_nodes));
+  a.roots = det_d; a.prior = prior_d; a.value = value_d;
+  set_leaves(a, leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d);
   const GumbelArgs gb = {gumbel_d, sim, num_simulations, max_considered, c_visit, c_scale, nullptr, nullptr};
-  const char* bad = gumbel_bad(n, gb, false);
-  if (!bad) bad = n > 0 && !det_d ? "worlds (det) are required" : n > 0 && (!prior_d || !value_d) ? "prior and value are required" : ismcts_bad(a, ws_bytes);
-  if (bad) { snprintf(h->err, sizeof h->err, "sb_ismcts_simulate_gumbel: %s", bad); return -1; }
+  const char* bad = first_bad({gumbel_bad(n, gb, false), n > 0 && !det_d ? "worlds (det) are required" : nullptr, eval_bad(a),
+                               ws_bad(a, ws_bytes, ISMCTS_WS_SMALL)});
+  if (bad) return refuse(h, "sb_ismcts_simulate_gumbel", bad);
   if (n == 0) return 0;
   k_ismcts_simulate_gumbel<<<grid_for(n, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a, gb, h->d_cards, h->d_wt);
   LAUNCH_CHECK();
@@ -1788,44 +1805,27 @@ int sb_ismcts_end_gumbel(SbHandle* h, int n, int max_nodes, void* ws_d, size_t w
                          const float* gumbel_d, double c_visit, double c_scale, int32_t* action_d, float* policy_d,
                          int32_t* visits_d, double* q_d, double* root_value_d, void* stream) {
   DEV_GUARD(h);
-  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, ismcts_tree_bytes(max_nodes), nullptr, 0, prior_d, value_d, 0.0, 0.0,
-                  nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, visits_d, q_d, root_value_d};
+  SearchArgs a(n, max_nodes, ws_d, ismcts_tree_bytes(max_nodes));
+  a.prior = prior_d; a.value = value_d; a.visits = visits_d; a.q = q_d; a.root_value = root_value_d;
   const GumbelArgs gb = {gumbel_d, 0, 0, 0, c_visit, c_scale, action_d, policy_d};
-  const char* bad = gumbel_bad(n, gb, true);
-  if (!bad) bad = n > 0 && (!prior_d || !value_d) ? "prior and value are required"
-                  : n > 0 && (!visits_d || !q_d || !root_value_d) ? "visits, q and root_value are required"
-                  : ismcts_bad(a, ws_bytes);
-  if (bad) { snprintf(h->err, sizeof h->err, "sb_ismcts_end_gumbel: %s", bad); return -1; }
+  const char* bad = first_bad({gumbel_bad(n, gb, true), eval_bad(a), read_out_bad(a), ws_bad(a, ws_bytes, ISMCTS_WS_SMALL)});
+  if (bad) return refuse(h, "sb_ismcts_end_gumbel", bad);
   if (n == 0) return 0;
   k_ismcts_end_gumbel<<<grid_for(n, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a, gb);
   LAUNCH_CHECK();
   return 0;
 }
-// The advance entries: the checks of the matching begin plus the second workspace and keep; one launch each, no handle
-// scratch, atomics or host synchronisation.
-static const char* reuse_bad(const SearchArgs& a, const ReuseArgs& r) {  // after search_bad / ismcts_bad
-  const size_t span = (size_t)(a.n > 0 ? a.n : 0) * a.tree_bytes;
-  const uintptr_t s = (uintptr_t)r.src, d = (uintptr_t)a.ws;
-  return r.keep < 1 || r.keep > a.max_nodes ? "keep must be 1..max_nodes"
-         : a.n > 0 && !r.src ? "source workspace is NULL"
-         : ((uintptr_t)r.src & 15) ? "source workspace must be 16-byte aligned"
-         : a.n > 0 && r.src == a.ws ? "ws_src and ws_dst must be two workspaces"
-         : a.n > 0 && s < d + span && d < s + span ? "ws_src and ws_dst overlap"
-         : nullptr;
-}
 int sb_search_advance(SbHandle* h, int n, int max_nodes, void* ws_src_d, void* ws_dst_d, size_t ws_bytes, const uint8_t* roots_d,
                       int max_steps, int keep, int32_t* kept_d, uint8_t* leaf_states_d, int32_t* obs_d, uint32_t* masks_d,
                       uint8_t* obs_err_d, uint8_t* to_move_d, uint8_t* leaf_kind_d, void* stream) {
   DEV_GUARD(h);
-  SearchArgs a = {n, max_nodes, (unsigned char*)ws_dst_d, sizeof(STree) + (size_t)(max_nodes > 0 ? max_nodes : 0) * sizeof(SNode), roots_d,
-                  max_steps, nullptr, nullptr, 0.0, 0.0, leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d,
-                  nullptr, nullptr, nullptr};
+  SearchArgs a(n, max_nodes, ws_dst_d, search_tree_bytes(max_nodes));
+  a.roots = roots_d; a.max_steps = max_steps;
+  set_leaves(a, leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d);
   const ReuseArgs r = {(unsigned char*)ws_src_d, keep, kept_d, nullptr};
-  const char* bad = max_steps < 1 || max_steps > 65535 ? "max_steps must be 1..65535"
-                    : n > 0 && !roots_d ? "roots are required"
-                    : search_bad(a, ws_bytes);
-  if (!bad) bad = reuse_bad(a, r);
-  if (bad) { snprintf(h->err, sizeof h->err, "sb_search_advance: %s", bad); return -1; }
+  const char* bad = first_bad({steps_bad(max_steps), n > 0 && !roots_d ? "roots are required" : nullptr,
+                               ws_bad(a, ws_bytes, SEARCH_WS_SMALL), reuse_bad(a, r)});
+  if (bad) return refuse(h, "sb_search_advance", bad);
   if (n == 0) return 0;
   k_search_advance<<<grid_for(n, TPB_GAME), RS_THREADS, 0, (cudaStream_t)stream>>>(a, r, h->d_cards, h->d_wt);
   LAUNCH_CHECK();
@@ -1835,15 +1835,14 @@ int sb_ismcts_advance(SbHandle* h, int n, int max_nodes, void* ws_src_d, void* w
                       const int32_t* played_d, int max_steps, int keep, int32_t* kept_d, uint8_t* leaf_states_d, int32_t* obs_d,
                       uint32_t* masks_d, uint8_t* obs_err_d, uint8_t* to_move_d, uint8_t* leaf_kind_d, void* stream) {
   DEV_GUARD(h);
-  SearchArgs a = {n, max_nodes, (unsigned char*)ws_dst_d, ismcts_tree_bytes(max_nodes), det_d, max_steps, nullptr, nullptr, 0.0, 0.0,
-                  leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d, nullptr, nullptr, nullptr};
+  SearchArgs a(n, max_nodes, ws_dst_d, ismcts_tree_bytes(max_nodes));
+  a.roots = det_d; a.max_steps = max_steps;
+  set_leaves(a, leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d);
   const ReuseArgs r = {(unsigned char*)ws_src_d, keep, kept_d, played_d};
-  const char* bad = max_steps < 1 || max_steps > 65535 ? "max_steps must be 1..65535"
-                    : n > 0 && !det_d ? "worlds (det) are required"
-                    : n > 0 && !played_d ? "played is required"
-                    : ismcts_bad(a, ws_bytes);
-  if (!bad) bad = reuse_bad(a, r);
-  if (bad) { snprintf(h->err, sizeof h->err, "sb_ismcts_advance: %s", bad); return -1; }
+  const char* bad = first_bad({steps_bad(max_steps), n > 0 && !det_d ? "worlds (det) are required" : nullptr,
+                               n > 0 && !played_d ? "played is required" : nullptr, ws_bad(a, ws_bytes, ISMCTS_WS_SMALL),
+                               reuse_bad(a, r)});
+  if (bad) return refuse(h, "sb_ismcts_advance", bad);
   if (n == 0) return 0;
   k_ismcts_advance<<<grid_for(n, TPB_GAME), RS_THREADS, 0, (cudaStream_t)stream>>>(a, r, h->d_cards, h->d_wt);
   LAUNCH_CHECK();
@@ -1851,7 +1850,7 @@ int sb_ismcts_advance(SbHandle* h, int n, int max_nodes, void* ws_src_d, void* w
 }
 // The batch entries: the checks of sb_search_simulate / sb_search_end plus leaves and virtual_loss, against the batch
 // workspace size.  sb_search_simulate_batch launches two kernels (selection per tree, expansion per slot),
-// sb_search_end_batch one; no handle scratch, atomics or host synchronisation.
+// sb_search_end_batch one.
 static size_t batch_tail_bytes(int max_nodes, int leaves) { return ((size_t)8 * leaves + (size_t)4 * max_nodes + 15) & ~(size_t)15; }
 size_t sb_search_batch_workspace_bytes(int n, int max_nodes, int leaves) {
   const size_t pre = sb_search_workspace_bytes(n, max_nodes);
@@ -1859,55 +1858,46 @@ size_t sb_search_batch_workspace_bytes(int n, int max_nodes, int leaves) {
   const size_t tail = batch_tail_bytes(max_nodes, leaves);
   return (size_t)n > (SIZE_MAX - pre) / tail ? 0 : pre + (size_t)n * tail;
 }
-static int batch_launch(SbHandle* h, const SearchArgs& a, double vl, int leaves, size_t ws_bytes, const char* bad, bool end,
-                        void* stream) {
-  DEV_GUARD(h);
+// leaves, then 8.6's checks without its size check (SIZE_MAX), then the batch workspace size; vl_bad between the two first
+static const char* batch_bad(const SearchArgs& a, int leaves, const char* vl_bad, size_t ws_bytes) {
   const size_t need = sb_search_batch_workspace_bytes(a.n, a.max_nodes, leaves);
-  if (!bad) bad = leaves < 1 || leaves > SEARCH_MAX_LEAVES ? "leaves must be 1..256"
-                  : end ? nullptr
-                  : !(vl >= 0.0 && vl <= 1.7976931348623157e308) ? "virtual_loss must be finite and >= 0"
-                  : nullptr;
-  if (!bad) bad = search_bad(a, SIZE_MAX);  // its size check is the 8.6 prefix's; the batch size is checked below
-  if (!bad) bad = (long long)a.n * leaves > 0x7FFFFFFFll ? "n * leaves must be below 2^31"
-                  : a.n > 0 && need == 0 ? "workspace size overflows size_t"
-                  : ws_bytes < need ? "workspace too small (sb_search_batch_workspace_bytes)"
-                  : nullptr;
-  if (bad) { snprintf(h->err, sizeof h->err, "%s: %s", end ? "sb_search_end_batch" : "sb_search_simulate_batch", bad); return -1; }
-  if (a.n == 0) return 0;
-  const BatchArgs b = {leaves, vl, a.ws + (size_t)a.n * a.tree_bytes, batch_tail_bytes(a.max_nodes, leaves)};
-  cudaStream_t st = (cudaStream_t)stream;
-  if (end) {
-    k_search_end_batch<<<grid_for(a.n, TPB_GAME), TPB_GAME, 0, st>>>(a, b);
-    LAUNCH_CHECK();
-    return 0;
-  }
-  k_search_batch_select<<<grid_for(a.n, SB_SELECT_THREADS), SB_SELECT_THREADS, 0, st>>>(a, b);
-  LAUNCH_CHECK();
-  k_search_batch_expand<<<grid_for(a.n * leaves, TPB_GAME), TPB_GAME, 0, st>>>(a, b, h->d_cards, h->d_wt);
-  LAUNCH_CHECK();
-  return 0;
+  return first_bad({leaves < 1 || leaves > SEARCH_MAX_LEAVES ? "leaves must be 1..256" : nullptr, vl_bad, ws_bad(a, SIZE_MAX, nullptr),
+                    (long long)a.n * leaves > 0x7FFFFFFFll ? "n * leaves must be below 2^31"
+                    : a.n > 0 && need == 0 ? "workspace size overflows size_t"
+                    : ws_bytes < need ? "workspace too small (sb_search_batch_workspace_bytes)"
+                    : nullptr});
 }
 int sb_search_simulate_batch(SbHandle* h, int n, int max_nodes, int leaves, void* ws_d, size_t ws_bytes, const float* prior_d,
                              const float* value_d, double c_puct, double fpu, double virtual_loss, uint8_t* leaf_states_d,
                              int32_t* obs_d, uint32_t* masks_d, uint8_t* obs_err_d, uint8_t* to_move_d, uint8_t* leaf_kind_d,
                              void* stream) {
-  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, sizeof(STree) + (size_t)(max_nodes > 0 ? max_nodes : 0) * sizeof(SNode), nullptr,
-                  0, prior_d, value_d, c_puct, fpu, leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d,
-                  nullptr, nullptr, nullptr};
-  const char* bad = !(c_puct >= 0.0 && c_puct <= 1.7976931348623157e308) ? "c_puct must be finite and >= 0"
-                    : !(fpu >= -1.7976931348623157e308 && fpu <= 1.7976931348623157e308) ? "fpu must be finite"
-                    : n > 0 && (!prior_d || !value_d) ? "prior and value are required"
-                    : nullptr;
-  return batch_launch(h, a, virtual_loss, leaves, ws_bytes, bad, false, stream);
+  DEV_GUARD(h);
+  SearchArgs a(n, max_nodes, ws_d, search_tree_bytes(max_nodes));
+  a.prior = prior_d; a.value = value_d; a.c_puct = c_puct; a.fpu = fpu;
+  set_leaves(a, leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d);
+  const char* vl_bad = !(virtual_loss >= 0.0 && virtual_loss <= 1.7976931348623157e308) ? "virtual_loss must be finite and >= 0" : nullptr;
+  const char* bad = first_bad({puct_bad(c_puct, fpu), eval_bad(a), batch_bad(a, leaves, vl_bad, ws_bytes)});
+  if (bad) return refuse(h, "sb_search_simulate_batch", bad);
+  if (n == 0) return 0;
+  const BatchArgs b = {leaves, virtual_loss, a.ws + (size_t)n * a.tree_bytes, batch_tail_bytes(max_nodes, leaves)};
+  k_search_batch_select<<<grid_for(n, SB_SELECT_THREADS), SB_SELECT_THREADS, 0, (cudaStream_t)stream>>>(a, b);
+  LAUNCH_CHECK();
+  k_search_batch_expand<<<grid_for(n * leaves, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a, b, h->d_cards, h->d_wt);
+  LAUNCH_CHECK();
+  return 0;
 }
 int sb_search_end_batch(SbHandle* h, int n, int max_nodes, int leaves, void* ws_d, size_t ws_bytes, const float* prior_d,
                         const float* value_d, int32_t* visits_d, double* q_d, double* root_value_d, void* stream) {
-  SearchArgs a = {n, max_nodes, (unsigned char*)ws_d, sizeof(STree) + (size_t)(max_nodes > 0 ? max_nodes : 0) * sizeof(SNode), nullptr,
-                  0, prior_d, value_d, 0.0, 0.0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, visits_d, q_d, root_value_d};
-  const char* bad = n > 0 && (!prior_d || !value_d) ? "prior and value are required"
-                    : n > 0 && (!visits_d || !q_d || !root_value_d) ? "visits, q and root_value are required"
-                    : nullptr;
-  return batch_launch(h, a, 0.0, leaves, ws_bytes, bad, true, stream);
+  DEV_GUARD(h);
+  SearchArgs a(n, max_nodes, ws_d, search_tree_bytes(max_nodes));
+  a.prior = prior_d; a.value = value_d; a.visits = visits_d; a.q = q_d; a.root_value = root_value_d;
+  const char* bad = first_bad({eval_bad(a), read_out_bad(a), batch_bad(a, leaves, nullptr, ws_bytes)});
+  if (bad) return refuse(h, "sb_search_end_batch", bad);
+  if (n == 0) return 0;
+  const BatchArgs b = {leaves, 0.0, a.ws + (size_t)n * a.tree_bytes, batch_tail_bytes(max_nodes, leaves)};
+  k_search_end_batch<<<grid_for(n, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a, b);
+  LAUNCH_CHECK();
+  return 0;
 }
 // One launch, no handle scratch, atomics or host synchronisation (capturable in a CUDA graph).
 int sb_determinize(SbHandle* h, int n, const uint8_t* states_d, const uint8_t* observer_d, const uint64_t* keys_d, uint8_t* out_d,

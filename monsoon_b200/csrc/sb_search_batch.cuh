@@ -23,11 +23,10 @@
 // atomics, no host synchronisation: the expansion writes only its own new node and reads records of nodes that existed
 // before the call (a walk never continues below a pending node).
 //
-// Fault safety: every index read from the workspace is checked before it is dereferenced.  The node count must lie in
-// 1..max_nodes; a pending slot's node below the node count; a child link in 0..count-1 (0 = none); a parent below its child
-// (so a walk up ends at the root); a new node's action below 156.  Every walk down stops after max_nodes levels.  A failed
-// check stops the tree: kind SEARCH_FULL, every slot FULL, the root emitted (a stopped tree's V is never read again, the
-// next header-form call zeroes it).
+// Fault safety: 8.6's rule (sb_search.cuh), with the same checks (sb_count, sb_backup_node, s_select, s_read_out); in
+// addition a pending slot's node must lie below the node count and a new node's action below 156.  A failed check stops the
+// tree: kind SEARCH_FULL, every slot FULL, the root emitted (a stopped tree's V is never read again, the next header-form
+// call zeroes it).
 #pragma once
 #include "sb_search.cuh"
 
@@ -45,22 +44,6 @@ struct BatchArgs {
 
 SBD_FI int2* sb_slots(const BatchArgs& b, int i) { return reinterpret_cast<int2*>(b.tail + (size_t)i * b.tail_bytes); }
 SBD_FI int* sb_virt(const BatchArgs& b, int i) { return reinterpret_cast<int*>(b.tail + (size_t)i * b.tail_bytes + 8 * (size_t)b.leaves); }
-// the node count of tree t, 0 when it is not in 1..max_nodes
-SBD_FI int sb_count(const STree& t, int max_nodes) { return t.used >= 1 && t.used <= max_nodes ? t.used : 0; }
-
-// add v to W and 1 to N of node j and every node above it; false on a parent link that is not below its child
-SBD_FI bool sb_add_path(SNode* nodes, int j, double v) {
-  #pragma unroll 1
-  while (true) {
-    nodes[j].N += 1;
-    nodes[j].W = __dadd_rn(nodes[j].W, v);
-    if (j == 0) return true;
-    const int p = nodes[j].parent;
-    if (p < 0 || p >= j) return false;
-    j = p;
-  }
-}
-
 // set (d = 0) or add d to (d = 1) V of node j and every node above it; false on a bad parent link
 SBD_FI bool sb_mark_path(const SNode* nodes, int* virt, int j, int d) {
   #pragma unroll 1
@@ -71,21 +54,6 @@ SBD_FI bool sb_mark_path(const SNode* nodes, int* virt, int j, int d) {
     if (p < 0 || p >= j) return false;
     j = p;
   }
-}
-
-// back up node k (slot kind EVAL or TERMINAL) with row r's prior / value, as s_backup; false on a bad index
-SBD_FI bool sb_backup_node(const SearchArgs& a, SNode* nodes, int used, size_t r, int k, int kind) {
-  if (k < 0 || k >= used) return false;
-  SNode& leaf = nodes[k];
-  double v;
-  if (kind == SEARCH_TERMINAL) v = (double)leaf.tval;
-  else {
-    const float* p = a.prior + r * SB_N_ACTIONS;
-    #pragma unroll 1
-    for (int x = 0; x < SB_N_ACTIONS; x++) leaf.prior[x] = p[x];
-    v = __dmul_rn(s_sign(leaf.seat), (double)a.value[r]);
-  }
-  return sb_add_path(nodes, k, v);
 }
 
 // what the previous call left pending in tree i: the header-form leaf (slot 0's row) or the L slots in ascending order.
@@ -114,34 +82,6 @@ SBD_FI int sb_backup(const SearchArgs& a, const BatchArgs& b, int i, STree& t, S
   return used;
 }
 
-// PUCT with virtual visits at node j (s_select's order of operations): n_a = N(c) + V(c),
-// q = ((sgn * W(c)) - (vl * V(c))) / n_a (fpu when n_a = 0), u = ((c_puct * P) * sqrt(N(j) + V(j))) / (1 + n_a).
-// Returns the action (-1: none legal), c its child link; -2 on a child link outside 0..used-1.
-SBD_FI int sb_select(const SearchArgs& a, const BatchArgs& b, const SNode* nodes, const int* virt, int j, int used, int& child) {
-  const SNode& nd = nodes[j];
-  const double sgn = s_sign(nd.seat), sq = __dsqrt_rn((double)(nd.N + virt[j]));
-  int best = -1, best_c = 0;
-  double best_score = 0.0;
-  #pragma unroll 1
-  for (int w = 0; w < SB_MASK_WORDS; w++) {
-    u32 m = nd.mask[w];
-    while (m) {
-      const int act = w * 32 + __ffs(m) - 1;
-      m &= m - 1;
-      const int c = nd.child[act];
-      if (c < 0 || c >= used) return -2;
-      const int vc = c ? virt[c] : 0;
-      const int na = c ? nodes[c].N + vc : 0;
-      const double q = na ? __ddiv_rn(__dsub_rn(__dmul_rn(sgn, nodes[c].W), __dmul_rn(b.vl, (double)vc)), (double)na) : a.fpu;
-      const double u = __ddiv_rn(__dmul_rn(__dmul_rn(a.c_puct, (double)nd.prior[act]), sq), (double)(1 + na));
-      const double score = __dadd_rn(q, u);
-      if (best < 0 || score > best_score) { best = act; best_c = c; best_score = score; }
-    }
-  }
-  child = best_c;
-  return best;
-}
-
 __global__ void __launch_bounds__(SB_SELECT_THREADS) k_search_batch_select(const SearchArgs a, const BatchArgs b) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= a.n) return;
@@ -163,7 +103,7 @@ __global__ void __launch_bounds__(SB_SELECT_THREADS) k_search_batch_select(const
       else if (nodes[j].terminal) kind = SEARCH_TERMINAL;
       else {
         int c;
-        const int act = d < a.max_nodes ? sb_select(a, b, nodes, virt, j, used, c) : -1;
+        const int act = d < a.max_nodes ? s_select<true>(a, nodes, virt, b.vl, j, used, c) : -1;
         if (act < 0) { ok = false; break; }
         if (!c) {
           if (used >= a.max_nodes) break;  // no free node: this and every later slot are FULL
@@ -205,18 +145,7 @@ __global__ void __launch_bounds__(TPB_GAME) k_search_batch_expand(const SearchAr
   int2& slot = sb_slots(b, i)[l];
   const int used = sb_count(t, a.max_nodes), k = slot.x, kind = slot.y;
   if (kind == SEARCH_EVAL && k > 0 && k < used && nodes[k].parent >= 0 && nodes[k].parent < k && nodes[k].action < SB_N_ACTIONS) {
-    const int p = nodes[k].parent, act = nodes[k].action;
-    __align__(16) SbState s;
-    load_state(s, &nodes[p].rec);
-    unpack(g, s);
-    game_step(g, act);
-    end_of_step(g);
-    pack(g, s);
-    unpack(g, s);  // the working set as the next sb_* call would unpack it from the child's record
-    s_write_node(nodes[k], g, s, p, act, t.max_steps);
-    const int kk = nodes[k].terminal ? SEARCH_TERMINAL : SEARCH_EVAL;
-    slot.y = kk;
-    s_emit(a, r, g, nodes[k], kk);
+    slot.y = s_expand(a, r, g, t, nodes, k, nodes[k].parent, nodes[k].action);
   } else if (kind == SEARCH_TERMINAL && k >= 0 && k < used) {
     s_emit_node(a, r, g, nodes[k], SEARCH_TERMINAL);
   } else if (kind == SEARCH_COLLISION || kind == SEARCH_FULL) {
@@ -228,8 +157,7 @@ __global__ void __launch_bounds__(TPB_GAME) k_search_batch_expand(const SearchAr
   }
 }
 
-// back up what is pending, mark the tree finished and read out the root's edges (a root child link outside the node count
-// is dropped, never followed)
+// back up what is pending, mark the tree finished and read out the root's edges
 __global__ void __launch_bounds__(TPB_GAME) k_search_end_batch(const SearchArgs a, const BatchArgs b) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= a.n) return;
@@ -237,11 +165,5 @@ __global__ void __launch_bounds__(TPB_GAME) k_search_end_batch(const SearchArgs 
   SNode* nodes = s_nodes(a, i);
   sb_backup(a, b, i, t, nodes);
   t.kind = SEARCH_FULL;
-  const int used = sb_count(t, a.max_nodes);
-  #pragma unroll 1
-  for (int act = 0; act < SB_N_ACTIONS; act++) {
-    const int c = nodes[0].child[act];
-    if (c < 0 || c >= used) nodes[0].child[act] = 0;
-  }
-  s_read_out(a, i, nodes);
+  s_read_out(a, i, nodes, sb_count(t, a.max_nodes));
 }
