@@ -357,6 +357,42 @@ int sb_search_simulate_batch(SbHandle *h, int n, int max_nodes, int leaves, void
 int sb_search_end_batch(SbHandle *h, int n, int max_nodes, int leaves, void *ws_d, size_t ws_bytes, const float *prior_d,
                         const float *value_d, int32_t *visits_d, double *q_d, double *root_value_d, void *stream);
 
+/* Several leaves per tree per call for the information-set search, under virtual loss, ABI 5's additive entry points
+ * (DESIGN.md 8.12): sb_search_simulate_batch's contract over sb_ismcts_*'s tree, with one world per slot.
+ *   sb_ismcts_begin (world 0) or sb_ismcts_advance -> evaluate (n rows) -> (sb_ismcts_simulate_batch (the worlds of call c)
+ *   -> evaluate (n * L rows)) x C -> sb_ismcts_end_batch
+ * The workspace is sb_ismcts_batch_workspace_bytes(n, max_nodes, L) bytes: sb_ismcts_workspace_bytes(n, max_nodes) bytes of
+ * 8.8's layout, unchanged (so begin and advance write it, and advance reads a finished batched tree), then per tree a tail
+ * of the L pending slots (node, kind and the game value a TERMINAL slot was reached with in its world) and one int of
+ * virtual visits per node.  0 for bad arguments, as sb_search_batch_workspace_bytes.  det_d u8[n * L,512]: row g * L + l is
+ * the world of slot l of tree g, a determinization of root g for root g's own local_order.  prior_d, value_d and every leaf
+ * output have n * L rows in the same layout.  A tree that begin, advance or a plain simulate left is backed up from row
+ * g * L (slot 0).  One batch call is what running these steps slot by slot gives:
+ *   1. back up the pending slots in ascending slot order: EVAL stores the prior and adds sgn(leaf) * value along the path,
+ *      N += 1; TERMINAL adds the slot's stored game value; FULL and COLLISION add nothing;
+ *   2. for l = 0 .. L-1, walk from the root through world l as sb_ismcts_simulate does: where world l is over (env_over)
+ *      the walk ends as TERMINAL with world l's value; else select among world l's legal representatives with
+ *      sb_search_simulate_batch's score (children matched by move code; V(x) = the earlier slots of this call whose path
+ *      contains x; with V = 0 exactly sb_ismcts_simulate's scores), ties to the lowest id, and step the world.  Then descend
+ *      into an existing child; stop at a node created earlier in this call (COLLISION = 3: world l's root is emitted,
+ *      nothing is backed up); or, for a code without a child, take the next free node at once (inserted at the head of the
+ *      sibling list; the slot is EVAL, or TERMINAL with a zero prior when world l is over there).  When no node is free,
+ *      this and every later slot are FULL (world l's root emitted).  V is zero again when the call returns;
+ *   3. every slot emits world l's record at its leaf (leaf record, observation, obs_err, mask, seat to move, kind).
+ * sb_ismcts_end_batch backs up what is pending and writes sb_ismcts_end's read-out by the root codes stored at begin.
+ * Bad arguments return -1 (sb_last_error) and launch nothing: those sb_ismcts_simulate / sb_ismcts_end reject (ws_bytes
+ * against the batch size), leaves outside 1..256, a negative or non-finite virtual_loss, n * leaves >= 2^31; n = 0 is a
+ * no-op.  Each call is one kernel launch, without handle scratch, atomics or host synchronisation (capturable in a CUDA
+ * graph).  Mixing plain and batch calls within one search is unsupported (wrong numbers, never outside the tree).  Every
+ * index read from the workspace is checked; a bad one stops the tree (FULL) and is never dereferenced. */
+size_t sb_ismcts_batch_workspace_bytes(int n, int max_nodes, int leaves);
+int sb_ismcts_simulate_batch(SbHandle *h, int n, int max_nodes, int leaves, void *ws_d, size_t ws_bytes,
+                             const uint8_t *det_d, const float *prior_d, const float *value_d, double c_puct, double fpu,
+                             double virtual_loss, uint8_t *leaf_states_d, int32_t *obs_d, uint32_t *masks_d,
+                             uint8_t *obs_err_d, uint8_t *to_move_d, uint8_t *leaf_kind_d, void *stream);
+int sb_ismcts_end_batch(SbHandle *h, int n, int max_nodes, int leaves, void *ws_d, size_t ws_bytes, const float *prior_d,
+                        const float *value_d, int32_t *visits_d, double *q_d, double *root_value_d, void *stream);
+
 /* Determinization for sampled (PIMC) search:out_d[g] = states_d[g] with everything observer o cannot see resampled and
  * everything o sees kept byte for byte (sb_observe / sb_legal_mask / sb_features of o's view are unchanged).
  * observer_d u8[n] is nullable: NULL = each record's own local_order (the seat sb_observe and sb_legal_mask show); a

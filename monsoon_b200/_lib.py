@@ -69,6 +69,10 @@ SIGNATURES = {
     "sb_search_simulate_batch": (_int, [_vp, _int, _int, _int, _vp, ctypes.c_size_t, _vp, _vp, ctypes.c_double, ctypes.c_double,
                                         ctypes.c_double, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "sb_search_end_batch": (_int, [_vp, _int, _int, _int, _vp, ctypes.c_size_t, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "sb_ismcts_batch_workspace_bytes": (ctypes.c_size_t, [_int, _int, _int]),
+    "sb_ismcts_simulate_batch": (_int, [_vp, _int, _int, _int, _vp, ctypes.c_size_t, _vp, _vp, _vp, ctypes.c_double, ctypes.c_double,
+                                        ctypes.c_double, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "sb_ismcts_end_batch": (_int, [_vp, _int, _int, _int, _vp, ctypes.c_size_t, _vp, _vp, _vp, _vp, _vp, _vp]),
     "sb_accumulate_fitness": (_int, [_vp, _int, _vp, _vp, _vp, _vp]),
     "sb_count_aborted": (_int, [_vp, _int, _vp, _vp, _vp, _vp]),
     "sb_eval_schedule": (_int, [_vp, _int, _int, _int, _int, ctypes.c_uint64, ctypes.c_uint32, ctypes.c_int64, _int, _vp, _vp, _vp, _vp]),

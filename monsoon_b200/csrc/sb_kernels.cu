@@ -21,6 +21,8 @@
 //   k_*_advance        tree reuse between moves for both PUCT searches, one warp per tree for the copy (sb_reuse.cuh)
 //   k_search_batch_*   several leaves per tree per call under virtual loss: selection per tree, expansion per leaf
 //                      (sb_search_batch.cuh)
+//   k_ismcts_*_batch   the same for the information-set tree: a wavefront of one lane per leaf, the lanes of a tree in
+//                      one CTA (sb_ismcts_batch.cuh)
 //   k_determinize      one record per warp: resample what the observer cannot see (sb_determinize.cuh)
 //   k_accumulate_fitness win/draw/loss counts per individual (evo/fitness.py:95,160-166)
 //   k_es_*             evolution-strategy operators on the resident population (sb_es.cuh; evo/weights.py, evo/population.py)
@@ -1041,6 +1043,7 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32) k_env_step_heur(const EnvA
 
 // ---------------------------------------------------------------- several leaves per tree per call (sb_search_*_batch)
 #include "sb_search_batch.cuh"
+#include "sb_ismcts_batch.cuh"
 
 // ---------------------------------------------------------------- determinization for sampled search (sb_determinize)
 #include "sb_determinize.cuh"
@@ -1848,25 +1851,40 @@ int sb_ismcts_advance(SbHandle* h, int n, int max_nodes, void* ws_src_d, void* w
   LAUNCH_CHECK();
   return 0;
 }
-// The batch entries: the checks of sb_search_simulate / sb_search_end plus leaves and virtual_loss, against the batch
-// workspace size.  sb_search_simulate_batch launches two kernels (selection per tree, expansion per slot),
-// sb_search_end_batch one.
-static size_t batch_tail_bytes(int max_nodes, int leaves) { return ((size_t)8 * leaves + (size_t)4 * max_nodes + 15) & ~(size_t)15; }
-size_t sb_search_batch_workspace_bytes(int n, int max_nodes, int leaves) {
-  const size_t pre = sb_search_workspace_bytes(n, max_nodes);
+// The batch entries: the checks of sb_search_simulate / sb_search_end (sb_ismcts_simulate / sb_ismcts_end) plus leaves and
+// virtual_loss, against the batch workspace size.  sb_search_simulate_batch launches two kernels (selection per tree,
+// expansion per slot), sb_ismcts_simulate_batch one (the wavefront), each end one.
+// the tail of a tree: slot_bytes per pending slot, then V, i32 per node
+static size_t batch_tail_bytes(int max_nodes, int leaves, size_t slot_bytes) {
+  return (slot_bytes * leaves + (size_t)4 * max_nodes + 15) & ~(size_t)15;
+}
+static size_t batch_bytes(size_t pre, int n, int max_nodes, int leaves, size_t slot_bytes) {
   if (n < 0 || leaves < 1 || leaves > SEARCH_MAX_LEAVES || (n > 0 && pre == 0)) return 0;
-  const size_t tail = batch_tail_bytes(max_nodes, leaves);
+  const size_t tail = batch_tail_bytes(max_nodes, leaves, slot_bytes);
   return (size_t)n > (SIZE_MAX - pre) / tail ? 0 : pre + (size_t)n * tail;
 }
-// leaves, then 8.6's checks without its size check (SIZE_MAX), then the batch workspace size; vl_bad between the two first
-static const char* batch_bad(const SearchArgs& a, int leaves, const char* vl_bad, size_t ws_bytes) {
-  const size_t need = sb_search_batch_workspace_bytes(a.n, a.max_nodes, leaves);
-  return first_bad({leaves < 1 || leaves > SEARCH_MAX_LEAVES ? "leaves must be 1..256" : nullptr, vl_bad, ws_bad(a, SIZE_MAX, nullptr),
+#define SEARCH_SLOT_BYTES 8   // int2 {node, kind}
+#define ISMCTS_SLOT_BYTES 16  // int4 {node, kind, terminal value, 0}
+size_t sb_search_batch_workspace_bytes(int n, int max_nodes, int leaves) {
+  return batch_bytes(sb_search_workspace_bytes(n, max_nodes), n, max_nodes, leaves, SEARCH_SLOT_BYTES);
+}
+size_t sb_ismcts_batch_workspace_bytes(int n, int max_nodes, int leaves) {
+  return batch_bytes(sb_ismcts_workspace_bytes(n, max_nodes), n, max_nodes, leaves, ISMCTS_SLOT_BYTES);
+}
+static const char* vl_bad(double virtual_loss) {
+  return !(virtual_loss >= 0.0 && virtual_loss <= 1.7976931348623157e308) ? "virtual_loss must be finite and >= 0" : nullptr;
+}
+// leaves, then the plain entry's checks without its size check (SIZE_MAX), then the batch workspace size `need` (too_small
+// the reason when ws_bytes is below it); vl between the two first
+static const char* batch_bad(const SearchArgs& a, int leaves, const char* vl, size_t ws_bytes, size_t need, const char* too_small) {
+  return first_bad({leaves < 1 || leaves > SEARCH_MAX_LEAVES ? "leaves must be 1..256" : nullptr, vl, ws_bad(a, SIZE_MAX, nullptr),
                     (long long)a.n * leaves > 0x7FFFFFFFll ? "n * leaves must be below 2^31"
                     : a.n > 0 && need == 0 ? "workspace size overflows size_t"
-                    : ws_bytes < need ? "workspace too small (sb_search_batch_workspace_bytes)"
+                    : ws_bytes < need ? too_small
                     : nullptr});
 }
+#define SEARCH_BATCH_WS_SMALL "workspace too small (sb_search_batch_workspace_bytes)"
+#define ISMCTS_BATCH_WS_SMALL "workspace too small (sb_ismcts_batch_workspace_bytes)"
 int sb_search_simulate_batch(SbHandle* h, int n, int max_nodes, int leaves, void* ws_d, size_t ws_bytes, const float* prior_d,
                              const float* value_d, double c_puct, double fpu, double virtual_loss, uint8_t* leaf_states_d,
                              int32_t* obs_d, uint32_t* masks_d, uint8_t* obs_err_d, uint8_t* to_move_d, uint8_t* leaf_kind_d,
@@ -1875,11 +1893,12 @@ int sb_search_simulate_batch(SbHandle* h, int n, int max_nodes, int leaves, void
   SearchArgs a(n, max_nodes, ws_d, search_tree_bytes(max_nodes));
   a.prior = prior_d; a.value = value_d; a.c_puct = c_puct; a.fpu = fpu;
   set_leaves(a, leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d);
-  const char* vl_bad = !(virtual_loss >= 0.0 && virtual_loss <= 1.7976931348623157e308) ? "virtual_loss must be finite and >= 0" : nullptr;
-  const char* bad = first_bad({puct_bad(c_puct, fpu), eval_bad(a), batch_bad(a, leaves, vl_bad, ws_bytes)});
+  const char* bad = first_bad({puct_bad(c_puct, fpu), eval_bad(a),
+                               batch_bad(a, leaves, vl_bad(virtual_loss), ws_bytes, sb_search_batch_workspace_bytes(n, max_nodes, leaves),
+                                         SEARCH_BATCH_WS_SMALL)});
   if (bad) return refuse(h, "sb_search_simulate_batch", bad);
   if (n == 0) return 0;
-  const BatchArgs b = {leaves, virtual_loss, a.ws + (size_t)n * a.tree_bytes, batch_tail_bytes(max_nodes, leaves)};
+  const BatchArgs b = {leaves, virtual_loss, a.ws + (size_t)n * a.tree_bytes, batch_tail_bytes(max_nodes, leaves, SEARCH_SLOT_BYTES)};
   k_search_batch_select<<<grid_for(n, SB_SELECT_THREADS), SB_SELECT_THREADS, 0, (cudaStream_t)stream>>>(a, b);
   LAUNCH_CHECK();
   k_search_batch_expand<<<grid_for(n * leaves, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a, b, h->d_cards, h->d_wt);
@@ -1891,11 +1910,52 @@ int sb_search_end_batch(SbHandle* h, int n, int max_nodes, int leaves, void* ws_
   DEV_GUARD(h);
   SearchArgs a(n, max_nodes, ws_d, search_tree_bytes(max_nodes));
   a.prior = prior_d; a.value = value_d; a.visits = visits_d; a.q = q_d; a.root_value = root_value_d;
-  const char* bad = first_bad({eval_bad(a), read_out_bad(a), batch_bad(a, leaves, nullptr, ws_bytes)});
+  const char* bad = first_bad({eval_bad(a), read_out_bad(a),
+                               batch_bad(a, leaves, nullptr, ws_bytes, sb_search_batch_workspace_bytes(n, max_nodes, leaves),
+                                         SEARCH_BATCH_WS_SMALL)});
   if (bad) return refuse(h, "sb_search_end_batch", bad);
   if (n == 0) return 0;
-  const BatchArgs b = {leaves, 0.0, a.ws + (size_t)n * a.tree_bytes, batch_tail_bytes(max_nodes, leaves)};
+  const BatchArgs b = {leaves, 0.0, a.ws + (size_t)n * a.tree_bytes, batch_tail_bytes(max_nodes, leaves, SEARCH_SLOT_BYTES)};
   k_search_end_batch<<<grid_for(n, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a, b);
+  LAUNCH_CHECK();
+  return 0;
+}
+// the lanes of a tree (L rounded up to a power of two) and its tail
+static IsmBatchArgs ismcts_batch_args(const SearchArgs& a, int leaves, double virtual_loss) {
+  int lanes = 1;
+  while (lanes < leaves) lanes *= 2;
+  return {leaves, lanes, virtual_loss, a.ws + (size_t)a.n * a.tree_bytes, batch_tail_bytes(a.max_nodes, leaves, ISMCTS_SLOT_BYTES)};
+}
+int sb_ismcts_simulate_batch(SbHandle* h, int n, int max_nodes, int leaves, void* ws_d, size_t ws_bytes, const uint8_t* det_d,
+                             const float* prior_d, const float* value_d, double c_puct, double fpu, double virtual_loss,
+                             uint8_t* leaf_states_d, int32_t* obs_d, uint32_t* masks_d, uint8_t* obs_err_d, uint8_t* to_move_d,
+                             uint8_t* leaf_kind_d, void* stream) {
+  DEV_GUARD(h);
+  SearchArgs a(n, max_nodes, ws_d, ismcts_tree_bytes(max_nodes));
+  a.roots = det_d; a.prior = prior_d; a.value = value_d; a.c_puct = c_puct; a.fpu = fpu;
+  set_leaves(a, leaf_states_d, obs_d, masks_d, obs_err_d, to_move_d, leaf_kind_d);
+  const char* bad = first_bad({puct_bad(c_puct, fpu), n > 0 && !det_d ? "worlds (det) are required" : nullptr, eval_bad(a),
+                               batch_bad(a, leaves, vl_bad(virtual_loss), ws_bytes, sb_ismcts_batch_workspace_bytes(n, max_nodes, leaves),
+                                         ISMCTS_BATCH_WS_SMALL)});
+  if (bad) return refuse(h, "sb_ismcts_simulate_batch", bad);
+  if (n == 0) return 0;
+  const IsmBatchArgs b = ismcts_batch_args(a, leaves, virtual_loss);
+  const int cta = b.lanes > ISM_BATCH_CTA ? b.lanes : ISM_BATCH_CTA;
+  k_ismcts_simulate_batch<<<grid_for(n, cta / b.lanes), cta, 0, (cudaStream_t)stream>>>(a, b, h->d_cards, h->d_wt);
+  LAUNCH_CHECK();
+  return 0;
+}
+int sb_ismcts_end_batch(SbHandle* h, int n, int max_nodes, int leaves, void* ws_d, size_t ws_bytes, const float* prior_d,
+                        const float* value_d, int32_t* visits_d, double* q_d, double* root_value_d, void* stream) {
+  DEV_GUARD(h);
+  SearchArgs a(n, max_nodes, ws_d, ismcts_tree_bytes(max_nodes));
+  a.prior = prior_d; a.value = value_d; a.visits = visits_d; a.q = q_d; a.root_value = root_value_d;
+  const char* bad = first_bad({eval_bad(a), read_out_bad(a),
+                               batch_bad(a, leaves, nullptr, ws_bytes, sb_ismcts_batch_workspace_bytes(n, max_nodes, leaves),
+                                         ISMCTS_BATCH_WS_SMALL)});
+  if (bad) return refuse(h, "sb_ismcts_end_batch", bad);
+  if (n == 0) return 0;
+  k_ismcts_end_batch<<<grid_for(n, TPB_GAME), TPB_GAME, 0, (cudaStream_t)stream>>>(a, ismcts_batch_args(a, leaves, 0.0));
   LAUNCH_CHECK();
   return 0;
 }

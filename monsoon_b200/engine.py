@@ -439,6 +439,39 @@ class Engine:
                                            self._p(o["visits"]), self._p(o["q"]), self._p(o["root_value"]), self._stream()), "sb_ismcts_end")
         return o
 
+    # ---- several leaves per information-set tree per call (sb_ismcts_simulate_batch / sb_ismcts_end_batch)
+    def ismcts_batch_workspace_bytes(self, n, max_nodes, leaves):
+        return ismcts_batch_workspace_bytes(n, max_nodes, leaves)
+
+    def ismcts_simulate_batch(self, ws, det, max_nodes, leaves, prior, value, c_puct=1.25, fpu=0.0, virtual_loss=1.0, out=None):
+        """sb_ismcts_simulate_batch: back up the pending leaves with prior f32[n*L,156] / value f32[n*L] (row g*L + l is slot
+        l of tree g; a tree that begin or advance left reads only slot 0), then walk slot l of tree g through its world, row
+        g*L + l of det u8[n*L,512], under virtual loss, and emit the n*L leaves into out (search_begin's buffers with n*L rows;
+        kind 3 = collision, the world's root emitted).  ws holds at least ismcts_batch_workspace_bytes(n, max_nodes, L)
+        bytes.  Returns that dict."""
+        self._dev(ws, torch.uint8)
+        det = self._worlds(det)
+        rows, L = det.shape[0], int(leaves)
+        assert L >= 1 and rows % L == 0, "worlds are u8[n * L, 512]"
+        self._search_eval(rows, prior, value)
+        o = self._search_outputs(rows, out, ("states", "obs", "masks", "obs_err", "to_move", "kind"))
+        self._check(self.lib.sb_ismcts_simulate_batch(self.h, rows // L, int(max_nodes), L, self._p(ws), ws.numel(), self._p(det),
+                                                      self._p(prior), self._p(value), float(c_puct), float(fpu), float(virtual_loss),
+                                                      self._p(o["states"]), self._p(o["obs"]), self._p(o["masks"]), self._p(o["obs_err"]),
+                                                      self._p(o["to_move"]), self._p(o["kind"]), self._stream()), "sb_ismcts_simulate_batch")
+        return o
+
+    def ismcts_end_batch(self, ws, n, max_nodes, leaves, prior, value, out=None):
+        """sb_ismcts_end_batch: back up the pending leaves (prior f32[n*L,156], value f32[n*L]), then ismcts_end's read-out
+        into out: visits i32[n,156], q f64[n,156] and root_value f64[n], by the roots' action ids.  Returns that dict."""
+        self._dev(ws, torch.uint8)
+        self._search_eval(int(n) * int(leaves), prior, value)
+        o = self._search_outputs(n, out, ("visits", "q", "root_value"))
+        self._check(self.lib.sb_ismcts_end_batch(self.h, n, int(max_nodes), int(leaves), self._p(ws), ws.numel(), self._p(prior),
+                                                 self._p(value), self._p(o["visits"]), self._p(o["q"]), self._p(o["root_value"]),
+                                                 self._stream()), "sb_ismcts_end_batch")
+        return o
+
     # ---- Gumbel search over both trees (sb_search_simulate_gumbel / sb_search_end_gumbel, sb_ismcts_*_gumbel)
     def _gumbel(self, n, gumbel):
         self._dev(gumbel, torch.float32)
@@ -665,6 +698,16 @@ def ismcts_workspace_bytes(n, max_nodes):
         raise ValueError("no ISMCTS workspace for n=%d, max_nodes=%d (n >= 0, max_nodes 1..2^24)" % (n, max_nodes))
     return b
 
+
+
+def ismcts_batch_workspace_bytes(n, max_nodes, leaves):
+    """sb_ismcts_batch_workspace_bytes: bytes of the batched information-set search workspace of n trees of max_nodes nodes,
+    L = leaves per tree per call (host only, no GPU needed)."""
+    b = int(_lib.load().sb_ismcts_batch_workspace_bytes(int(n), int(max_nodes), int(leaves)))
+    if n < 0 or max_nodes < 1 or not 1 <= leaves <= 256 or (n > 0 and b == 0):
+        raise ValueError("no batched ISMCTS workspace for n=%d, max_nodes=%d, leaves=%d (n >= 0, max_nodes 1..2^24, leaves 1..256)"
+                         % (n, max_nodes, leaves))
+    return b
 
 _engines = {}
 

@@ -45,6 +45,12 @@ DESIGN.md 8.11), so the evaluator sees n * L rows per call and is called S / L t
 
     mcts = BatchedMCTS(env.n, num_simulations=64, leaves_per_call=16)
     visits, q, root_value = mcts.run(env.states, evaluate)   # evaluate(leaf, k): n rows at k = 0, n * 16 rows at k = 1..4
+
+InformationSetMCTS takes leaves_per_call too (sb_ismcts_simulate_batch, DESIGN.md 8.12): each of the L leaves of a tree is
+walked through a world of its own, so the fair search gets the same larger evaluator batches:
+
+    mcts = InformationSetMCTS(env.n, num_simulations=64, leaves_per_call=16)
+    visits, q, root_value = mcts.run(env.states, rollout_evaluator())
 """
 import math
 
@@ -295,21 +301,39 @@ class InformationSetMCTS:
     in between) the tree starts fresh.  Such a run is 2 * num_simulations + 4 library launches (2S + 3 with played None,
     which starts every tree fresh), and with caller keys still capturable, with BatchedMCTS's caveat on replaying one
     captured advancing run.  With R = 0, played is ignored.
+
+    leaves_per_call = L > 1 selects L leaves per tree per call under virtual loss (sb_ismcts_simulate_batch, DESIGN.md
+    8.12), each walked through a world of its own: the roots are repeated once per run into a u8[n*L,512] buffer, which each
+    call determinizes with its n * L keys into a preallocated world buffer.  num_simulations = S must be a multiple of L.
+    The keys keep their shape, i64[(S+1)*n]: the first n are world 0, and call c = 1..S/L uses the n * L keys after the
+    first n + (c-1) * n * L, tree-major (key n + (c-1) * n * L + g * L + l is the world of leaf l of tree g), so
+    default_keys is unchanged.  A run is the world-0 determinization and begin (or advance), C = S / L determinizations and
+    batch calls and the batch end: 2C + 3 library launches (one more with an advance's played check).  evaluate(leaf, k) gets
+    the n roots at k = 0 and n * L rows at k = 1..C, tree-major, with kind 3 for a collision (the world's root is emitted and
+    its evaluation is not used); a root's child visits then add up to its slots that were neither a collision nor full.
+    L = 1 is the plain search exactly.  It combines with reuse_nodes (two batch-sized workspaces).
     """
 
-    def __init__(self, n, num_simulations, c_puct=1.25, fpu=0.0, max_steps=400, seed=0, engine=None, device=None, reuse_nodes=0):
+    def __init__(self, n, num_simulations, c_puct=1.25, fpu=0.0, max_steps=400, seed=0, engine=None, device=None, reuse_nodes=0,
+                 leaves_per_call=1, virtual_loss=1.0):
         if int(num_simulations) < 0:
             raise ValueError("num_simulations must be >= 0")
         if not (math.isfinite(c_puct) and c_puct >= 0) or not math.isfinite(fpu):
             raise ValueError("c_puct must be finite and >= 0, fpu finite")
         if int(reuse_nodes) < 0:
             raise ValueError("reuse_nodes must be >= 0")
+        if not 1 <= int(leaves_per_call) <= 256 or int(num_simulations) % int(leaves_per_call):
+            raise ValueError("leaves_per_call must be 1..256 and divide num_simulations")
+        if not (math.isfinite(virtual_loss) and virtual_loss >= 0):
+            raise ValueError("virtual_loss must be finite and >= 0")
         self.engine = e = engine if engine is not None else get_engine(device)
         self.n, self.num_simulations, self.reuse_nodes = int(n), int(num_simulations), int(reuse_nodes)
         self.c_puct, self.fpu, self.max_steps = float(c_puct), float(fpu), int(max_steps)
+        self.leaves, self.virtual_loss = int(leaves_per_call), float(virtual_loss)
         self.max_nodes = self.num_simulations + 1 + self.reuse_nodes
         self.seed, self.calls = int(seed), 0
-        nb = e.ismcts_workspace_bytes(self.n, self.max_nodes)
+        L = self.leaves
+        nb = e.ismcts_workspace_bytes(self.n, self.max_nodes) if L == 1 else e.ismcts_batch_workspace_bytes(self.n, self.max_nodes, L)
         self.ws = torch.empty(nb, dtype=torch.uint8, device=e.device)
         self.world = torch.empty((self.n, STATE_BYTES), dtype=torch.uint8, device=e.device)
         self.kept = torch.zeros(self.n, dtype=torch.int32, device=e.device)
@@ -322,6 +346,12 @@ class InformationSetMCTS:
             self.step_out = [torch.empty(self.n, dtype=d, device=e.device) for d in (torch.uint8, torch.int8, torch.uint8, torch.uint8)]
         self.leaf = e._search_outputs(self.n, None, LEAF_KEYS)
         self.out = e._search_outputs(self.n, None, ("visits", "q", "root_value"))
+        if L > 1:
+            self.repeated = torch.empty((self.n * L, STATE_BYTES), dtype=torch.uint8, device=e.device)
+            self.worlds = torch.empty((self.n * L, STATE_BYTES), dtype=torch.uint8, device=e.device)
+            self.batch_leaf = e._search_outputs(self.n * L, None, LEAF_KEYS)
+            self.batch_prior = torch.empty((self.n * L, N_ACTIONS), dtype=torch.float32, device=e.device)
+            self.batch_value = torch.empty(self.n * L, dtype=torch.float32, device=e.device)
 
     def default_keys(self):
         """the keys of the next run without caller keys: next_seed(base + t) for t < (S+1)*n, base = next_seed(next_seed(seed)
@@ -367,11 +397,25 @@ class InformationSetMCTS:
             self.prev.copy_(roots)
         self.fresh = False
         prior, value = evaluate(self.leaf, 0)
-        for k in range(1, self.num_simulations + 1):
-            e.determinize(roots, keys[k * n:(k + 1) * n], out=self.world)
-            e.ismcts_simulate(self.ws, self.world, m, prior, value, self.c_puct, self.fpu, out=self.leaf)
-            prior, value = evaluate(self.leaf, k)
-        e.ismcts_end(self.ws, n, m, prior, value, out=self.out)
+        L = self.leaves
+        if L == 1:
+            for k in range(1, self.num_simulations + 1):
+                e.determinize(roots, keys[k * n:(k + 1) * n], out=self.world)
+                e.ismcts_simulate(self.ws, self.world, m, prior, value, self.c_puct, self.fpu, out=self.leaf)
+                prior, value = evaluate(self.leaf, k)
+            e.ismcts_end(self.ws, n, m, prior, value, out=self.out)
+            return self.out["visits"], self.out["q"], self.out["root_value"]
+        # the first batch call backs up the roots from slot 0 of each tree's rows; the other slots are not read
+        self.repeated.view(n, L, STATE_BYTES).copy_(roots.unsqueeze(1).expand(n, L, STATE_BYTES))
+        self.batch_prior.view(n, L, N_ACTIONS)[:, 0].copy_(prior)
+        self.batch_value.view(n, L)[:, 0].copy_(value)
+        prior, value = self.batch_prior, self.batch_value
+        for k in range(1, S // L + 1):
+            lo = n + (k - 1) * n * L
+            e.determinize(self.repeated, keys[lo:lo + n * L], out=self.worlds)
+            e.ismcts_simulate_batch(self.ws, self.worlds, m, L, prior, value, self.c_puct, self.fpu, self.virtual_loss, out=self.batch_leaf)
+            prior, value = evaluate(self.batch_leaf, k)
+        e.ismcts_end_batch(self.ws, n, m, L, prior, value, out=self.out)
         return self.out["visits"], self.out["q"], self.out["root_value"]
 
 
