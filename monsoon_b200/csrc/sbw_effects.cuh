@@ -330,13 +330,14 @@ SBW_NI void w_run_op(WG* wg, u32 op, int id, const i8* p, int pos_pt) {
   else if (after == WX_DESTROY) w_destroy(wg, id, 1);
 }
 
-SBW_NI void w_effect(WG* wg, int id, int pos_pt, int has_source) {
+// The bespoke handlers of the cards that the default decks do not hold, out of line: the handlers that the bench's
+// games run (and the dispatch to them) then stay together in a few instruction-cache lines of w_effect instead of
+// being spread over the 69 KB of all handlers (tools/hot_footprint.py, DESIGN.md section 10).  Same rules either way.
+SBW_NI void w_effect_rare(WG* wg, int id, int pos_pt, int has_source) {
   W_SHARED(wg);
   const int card = wg->e_card[id];
   const DCard& cd = WCARD(wg, card);
   const i8* p = cd.p;
-  const u32 op = w_effect_op(card);
-  if (op) { w_run_op(wg, op, id, p, pos_pt); return; }
   const int me = w_owner(wg, id);
   const int ex = w_ex(wg, id), ey = w_ey(wg, id);
   int tid;
@@ -427,9 +428,6 @@ SBW_NI void w_effect(WG* wg, int id, int pos_pt, int has_source) {
         if (tid >= 0) w_destroy(wg, tid, 1);
       }
       break; }
-    case SBC_B304:  // cards/b304.py:12-13
-      w_deal_damage(wg, id, p[0], 0, 1);
-      break;
     case SBC_B305: {  // cards/b305.py:16-45: ability_amount, ability_mana, original_cost
       t = w_targets(wg, WCUR(wg), w_mkT(TK_STRUCTURE, TS_FRIENDLY), ey * 4 + ex);
 #pragma unroll 1
@@ -467,7 +465,6 @@ SBW_NI void w_effect(WG* wg, int id, int pos_pt, int has_source) {
         wg->n_obj = (u8)(wg->n_obj + 1);
       }
       break; }
-    // ------------------------------------------------------------ units
     case SBC_U017: {  // cards/u017.py:18-34
       WPly& pl = wg->pl[me];
       int nc = 0;
@@ -530,26 +527,6 @@ SBW_NI void w_effect(WG* wg, int id, int pos_pt, int has_source) {
       if (tl_n(w_bordering_t(wg, ex, ey, WCUR(wg), w_mkT(TK_UNIT, TS_ANY))) == 0) w_gain_speed(wg, id, p[0]);
       else wv_heal(wg, id, p[1]);
       break;
-    case SBC_U053:  // cards/u053.py:14-24: ability_amount=1, ability_movement=2
-      if (tl_n(w_surrounding_t(wg, ex, ey, WCUR(wg), w_mkT(TK_UNIT, TS_ANY))) == 0) w_gain_speed(wg, id, p[1]);
-      else if (tl_n(w_bordering_t(wg, ex, ey, WCUR(wg), w_mkT(TK_UNIT, TS_ANY))) == 0) w_gain_speed(wg, id, p[0]);
-      break;
-    case SBC_U061:  // cards/u061.py:12-23
-      wv_confuse(wg, id);
-      t = w_targets(wg, WCUR(wg), w_mkT(TK_UNIT, TS_FRIENDLY), ey * 4 + ex);
-      if (tl_n(t) > 0) { tid = w_need(wg, w_choice_tl(wg, t)); if (tid < 0) return; wv_confuse(wg, tid); }
-      w_gain_speed(wg, id, 2);
-      break;
-    case SBC_U071: {  // cards/u071.py:12-27
-      t = w_bordering_t(wg, ex, ey, me, tq_xstatus(w_mkT(TK_UNIT, TS_ENEMY), 1u << SB_ST_CONFUSED));
-      if (tl_n(t) > 0) {
-        tid = w_need(wg, w_choice_tl(wg, t));
-        if (tid < 0) return;
-        wv_confuse(wg, tid);
-        const int fr = w_column_first_tile(wg, ex, ey, WCUR(wg), true);
-        if (fr != PT_NONE && w_at_pt(wg, fr) < 0) wv_teleport(wg, id, wpt_x(fr), wpt_y(fr));
-      }
-      break; }
     case SBC_U076:  // cards/u076.py:14-26: ability_damage, ability_strength
       t = w_surrounding_t(wg, ex, ey, WCUR(wg), tq_xtypes(w_mkT(TK_UNIT, TS_ANY), 1u << UT_DRAGON));
       if (tl_n(t) > 0) {
@@ -563,32 +540,11 @@ SBW_NI void w_effect(WG* wg, int id, int pos_pt, int has_source) {
       if (tl_n(w_bordering_t(wg, ex, ey, WCUR(wg), w_mkT(TK_STRUCTURE, TS_FRIENDLY))) > 0 || ey == 4) wv_heal(wg, id, p[0]);
       break;
     case SBC_U117: wv_freeze(wg, id); break;          // cards/u117.py:11-12
-    case SBC_U206: w_player_damage(wg, me, p[0]); break;  // cards/u206.py:12-13
-    case SBC_U211: {  // cards/u211.py:14-19: ability_max_strength, ability_min_strength
-      const int fr = w_column_first_tile(wg, ex, ey, WCUR(wg), true);
-      if (fr != PT_NONE && w_at_pt(wg, fr) < 0) {
-        const int s = p[1] + w_rng_below(wg, p[0] + 1 - p[1]);
-        w_spawn_token_unit(wg, me, fr, s, UT_SATYR);
-      }
-      break; }
     case SBC_U216: w_player_damage(wg, me, p[0]); break;  // cards/u216.py:12-13
     case SBC_U217: {  // cards/u217.py:13-17
       const TL row = tl_tiles(0xF0000u & ~wg->occ, true);
       if (tl_n(row) > 0) w_spawn_token_unit(wg, me, w_choice_tl(wg, row), p[0], UT_SATYR);
       break; }
-    case SBC_U302:  // cards/u302.py:12-23
-      if (pos_pt < 0 || pos_pt >= 20) return;
-      tid = w_at_pt(wg, pos_pt);
-      if (tid < 0 || w_is_struct(wg, tid)) return;
-      if (wg->e_str[tid] > wg->e_str[id]) {
-        w_deal_damage(wg, tid, p[0], 0, 1);
-        if (wg->e_str[tid] > 0) wv_push(wg, tid, w_ex(wg, id), w_ey(wg, id));
-      }
-      break;
-    case SBC_U305:  // cards/u305.py:13-21: +p0 to a bordering friendly CONSTRUCT and to itself, only if there is one
-      t = w_bordering_t(wg, ex, ey, WCUR(wg), tq_types(w_mkT(TK_UNIT, TS_FRIENDLY), 1u << UT_CONSTRUCT));
-      if (tl_n(t) > 0) { tid = w_need(wg, w_choice_tl(wg, t)); if (tid < 0) return; wv_heal(wg, tid, p[0]); wv_heal(wg, id, p[0]); }
-      break;
     case SBC_U310: {  // cards/u310.py:12-41
       t = w_bordering_t(wg, ex, ey, WCUR(wg), w_mkT(TK_UNIT, TS_ENEMY));
       const u32 m = t.m;
@@ -650,15 +606,6 @@ SBW_NI void w_effect(WG* wg, int id, int pos_pt, int has_source) {
 #pragma unroll 1
       for (int k = 0; k < em.n; k++) w_spawn_token_unit(wg, me, pl_get(em, k), p[0], UT_ANCIENT);
       break; }
-    case SBC_UA07:  // cards/ua07.py:11-22
-      switch (w_rng_below(wg, 5)) {
-        case 0: wv_freeze(wg, id); break;
-        case 1: wv_poison(wg, id); break;
-        case 2: wv_vitalize(wg, id); break;
-        case 3: wv_confuse(wg, id); break;
-        case 4: wv_disable(wg, id); break;
-      }
-      break;
     case SBC_UA20:  // cards/ua20.py:21-32: ability_cost, ability_level
       if (tl_n(w_column_targets(wg, ex, ey, me, w_mkT(TK_UNIT, TS_ENEMY), true)) == 0) {
         WPly& pl = wg->pl[me];
@@ -715,6 +662,75 @@ SBW_NI void w_effect(WG* wg, int id, int pos_pt, int has_source) {
       }
       break; }
     default: break;
+  }
+}
+
+SBW_NI void w_effect(WG* wg, int id, int pos_pt, int has_source) {
+  W_SHARED(wg);
+  const int card = wg->e_card[id];
+  const DCard& cd = WCARD(wg, card);
+  const i8* p = cd.p;
+  const u32 op = w_effect_op(card);
+  if (op) { w_run_op(wg, op, id, p, pos_pt); return; }
+  const int me = w_owner(wg, id);
+  const int ex = w_ex(wg, id), ey = w_ey(wg, id);
+  int tid;
+  TL t;
+  switch (card) {
+    case SBC_B304:  // cards/b304.py:12-13
+      w_deal_damage(wg, id, p[0], 0, 1);
+      break;
+    case SBC_U053:  // cards/u053.py:14-24: ability_amount=1, ability_movement=2
+      if (tl_n(w_surrounding_t(wg, ex, ey, WCUR(wg), w_mkT(TK_UNIT, TS_ANY))) == 0) w_gain_speed(wg, id, p[1]);
+      else if (tl_n(w_bordering_t(wg, ex, ey, WCUR(wg), w_mkT(TK_UNIT, TS_ANY))) == 0) w_gain_speed(wg, id, p[0]);
+      break;
+    case SBC_U061:  // cards/u061.py:12-23
+      wv_confuse(wg, id);
+      t = w_targets(wg, WCUR(wg), w_mkT(TK_UNIT, TS_FRIENDLY), ey * 4 + ex);
+      if (tl_n(t) > 0) { tid = w_need(wg, w_choice_tl(wg, t)); if (tid < 0) return; wv_confuse(wg, tid); }
+      w_gain_speed(wg, id, 2);
+      break;
+    case SBC_U071: {  // cards/u071.py:12-27
+      t = w_bordering_t(wg, ex, ey, me, tq_xstatus(w_mkT(TK_UNIT, TS_ENEMY), 1u << SB_ST_CONFUSED));
+      if (tl_n(t) > 0) {
+        tid = w_need(wg, w_choice_tl(wg, t));
+        if (tid < 0) return;
+        wv_confuse(wg, tid);
+        const int fr = w_column_first_tile(wg, ex, ey, WCUR(wg), true);
+        if (fr != PT_NONE && w_at_pt(wg, fr) < 0) wv_teleport(wg, id, wpt_x(fr), wpt_y(fr));
+      }
+      break; }
+    case SBC_U206: w_player_damage(wg, me, p[0]); break;  // cards/u206.py:12-13
+    case SBC_U211: {  // cards/u211.py:14-19: ability_max_strength, ability_min_strength
+      const int fr = w_column_first_tile(wg, ex, ey, WCUR(wg), true);
+      if (fr != PT_NONE && w_at_pt(wg, fr) < 0) {
+        const int s = p[1] + w_rng_below(wg, p[0] + 1 - p[1]);
+        w_spawn_token_unit(wg, me, fr, s, UT_SATYR);
+      }
+      break; }
+    case SBC_U302:  // cards/u302.py:12-23
+      if (pos_pt < 0 || pos_pt >= 20) return;
+      tid = w_at_pt(wg, pos_pt);
+      if (tid < 0 || w_is_struct(wg, tid)) return;
+      if (wg->e_str[tid] > wg->e_str[id]) {
+        w_deal_damage(wg, tid, p[0], 0, 1);
+        if (wg->e_str[tid] > 0) wv_push(wg, tid, w_ex(wg, id), w_ey(wg, id));
+      }
+      break;
+    case SBC_U305:  // cards/u305.py:13-21: +p0 to a bordering friendly CONSTRUCT and to itself, only if there is one
+      t = w_bordering_t(wg, ex, ey, WCUR(wg), tq_types(w_mkT(TK_UNIT, TS_FRIENDLY), 1u << UT_CONSTRUCT));
+      if (tl_n(t) > 0) { tid = w_need(wg, w_choice_tl(wg, t)); if (tid < 0) return; wv_heal(wg, tid, p[0]); wv_heal(wg, id, p[0]); }
+      break;
+    case SBC_UA07:  // cards/ua07.py:11-22
+      switch (w_rng_below(wg, 5)) {
+        case 0: wv_freeze(wg, id); break;
+        case 1: wv_poison(wg, id); break;
+        case 2: wv_vitalize(wg, id); break;
+        case 3: wv_confuse(wg, id); break;
+        case 4: wv_disable(wg, id); break;
+      }
+      break;
+    default: w_effect_rare(wg, id, pos_pt, has_source); break;
   }
 }
 
